@@ -445,9 +445,34 @@ def ncu_evidence(precision):
     return out
 
 
-def resident_run(torch, dist, shape, args, steps, warmup, world, rank, local, device_source, x_host, lo, hi, algorithm=None):
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, mdl, trace, rank):
+    """Write what `Corex.fit` would hand its caller had it stopped after the last timed iteration -- `ws` and every `moments`
+    key after the final sort by TC (Corex._finish) -- plus the TC of each timed iteration, as float64 `<name>.npy` files
+    (moments keys with punctuation squeezed to `_`).  An array larger than an equal share of DUMP_BYTES is replaced by the
+    entries at a fixed, seeded set of flat positions, so two builds run with the same arguments compare element for element."""
+    import re
+    mdl._finish()  # collective on several ranks: every rank runs it, rank 0 writes
+    if rank != 0:
+        return
+    arrays = {"ws": mdl.ws, "TC_per_step": [t["TC"] for t in trace]}
+    for key in list(mdl.moments):
+        arrays["moments_" + re.sub(r"[^A-Za-z0-9]+", "_", key).strip("_")] = mdl.moments[key]
+    share = DUMP_BYTES // 8 // len(arrays)
+    os.makedirs(directory, exist_ok=True)
+    for name, value in arrays.items():
+        a = np.asarray(value, dtype=np.float64)
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
+def resident_run(torch, dist, shape, args, steps, warmup, world, rank, local, device_source, x_host, lo, hi, algorithm=None,
+                 dump_dir=None):
     """Exactly `steps` fit iterations with X~ (or, on the Gram route, X~^T X~ / N) resident in HBM, timed by CUDA events, max
-    over ranks."""
+    over ranks.  With `dump_dir` the fitted model is written there afterwards (dump_outputs)."""
     algorithm = algorithm or args.algorithm or "stream"
     from linearcorex_b200 import Corex, _lib
     n_total, n_vars, n_factors = shape
@@ -467,13 +492,16 @@ def resident_run(torch, dist, shape, args, steps, warmup, world, rank, local, de
     mdl._begin_stage(schedule[0], rescale=False)
     sess = mdl._sess
     def iterate(k):
-        """k iterations of the current stage, the way fit() runs them (lcx_run_stage_ns).  Returns how many ran: with
-        tol = 1e-12 the stage cannot converge inside a bench window on these workloads, but if it ever does the line reports
-        the iterations that were actually timed instead of dying."""
+        """Exactly k iterations of the current stage, the way fit() runs them (lcx_run_stage_ns).  A stage that meets its
+        stopping rule (tol = 1e-12) returns early; it is entered again until k iterations have run, so the timed window
+        always holds the requested number of steps."""
         n0 = len(mdl.trace)
-        mdl.max_iter = k
-        mdl._run_stage_native()
-        return len(mdl.trace) - n0
+        while len(mdl.trace) - n0 < k:
+            before = len(mdl.trace)
+            mdl.max_iter = k - (before - n0)
+            if not mdl._run_stage_native() or len(mdl.trace) == before:
+                raise RuntimeError("the fit stopped after %d of %d iterations" % (before - n0, k))
+        return k
 
     iterate(warmup)
     sess.lib.lcx_profile_enable(sess.h, 1)
@@ -486,7 +514,7 @@ def resident_run(torch, dist, shape, args, steps, warmup, world, rank, local, de
     with clocks:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        steps_run = max(1, iterate(steps))
+        iterate(steps)
         e1.record()
         barrier()
     ms = e0.elapsed_time(e1)
@@ -508,18 +536,20 @@ def resident_run(torch, dist, shape, args, steps, warmup, world, rank, local, de
     # per-rank phase times: shows how much of rank 0's `exchange` is waiting for the slowest rank's contractions
     per_rank = None
     if world > 1:
-        mine = torch.tensor([k1.value / np_, k2.value / np_, kx.value / np_, e0.elapsed_time(e1) / max(1, steps_run)],
+        mine = torch.tensor([k1.value / np_, k2.value / np_, kx.value / np_, e0.elapsed_time(e1) / steps],
                             dtype=torch.float64, device="cuda")
         allr = [torch.empty_like(mine) for _ in range(world)]
         dist.all_gather(allr, mine)
         per_rank = {"columns": ["k1_ms", "k2_ms", "exchange_ms", "step_ms"],
                     "ranks": [[round(float(v), 4) for v in t.tolist()] for t in allr]}
     trace = mdl.trace[n_trace0:]
-    res = {"ms": ms, "per_rank": per_rank, "it_s": steps_run / (ms / 1e3), "steps_run": steps_run, "k1_ms": k1.value / np_, "k2_ms": k2.value / np_, "exchange_ms": kx.value / np_,
+    res = {"ms": ms, "per_rank": per_rank, "it_s": steps / (ms / 1e3), "k1_ms": k1.value / np_, "k2_ms": k2.value / np_, "exchange_ms": kx.value / np_,
            "pairs": pairs.value, "launches": sess.launches() - launches0, "prep": prep,
            "trials": float(np.mean([t["trials"] for t in trace])) if trace else 0.0, "tc": float(mdl.tc),
            "clocks": clocks.summary(), "peer": sess._peer_buf is not None, "algorithm": mdl.algorithm_used, "ranks_bit_identical": identical,
            "n_local": hi - lo}
+    if dump_dir:
+        dump_outputs(dump_dir, mdl, trace, rank)
     del mdl, sess
     torch.cuda.empty_cache()
     return res
@@ -656,7 +686,8 @@ def run_ours(args, shape):
     i8_peak = measure_int8_peak(torch) if (rank == 0 and digits) else None
 
     # ---- device-resident timing: exactly K iterations ----------------------------------------------
-    res = resident_run(torch, dist, shape, args, args.steps, args.warmup, world, rank, local, device_source, x_host, lo, hi)
+    res = resident_run(torch, dist, shape, args, args.steps, args.warmup, world, rank, local, device_source, x_host, lo, hi,
+                       dump_dir=args.dump_outputs)
     ms, it_s, n_local = res["ms"], res["it_s"], res["n_local"]
     # the Gram route on the same data, as a sub-record (N >= n, split modes): the default of the public API at this shape
     gram = None
@@ -845,9 +876,6 @@ def run_ours(args, shape):
     else:
         line["config"]["algorithm"] = "stream (every pass pair reads X~: the north star's formulation); see `gram` for the route "\
                                       "the public API picks at this shape"
-    if res.get("steps_run") != args.steps:  # (never seen: the stage converged inside the timed window)
-        line["steps_run"] = res.get("steps_run")
-        line["ms_per_step"] = ms / max(1, res.get("steps_run") or 1)
     if gram is not None:
         line["gram"] = gram
     if e2e_stream is not None:
@@ -901,7 +929,12 @@ def main():
     ap.add_argument("--e2e-fit", default=None, choices=["converge", "budget"],
                     help="end-to-end fit: run to the default stopping rule (default for config3) or K iterations over the stages")
     ap.add_argument("--traffic", type=float, default=None, help="dram bytes per launch from an ncu capture, if known")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed iterations, write the fitted ws and moments of that run to DIR/<name>.npy (float64, "
+                         "at most 64 MB; larger arrays as a fixed, seeded sample of their entries)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
     shape = list(WORKLOADS[args.workload])
     for i, v in enumerate((args.rows, args.vars, args.factors)):
