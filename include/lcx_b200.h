@@ -41,6 +41,7 @@ extern "C" {
 #define LCX_ERR_CUDA (-2)
 #define LCX_ERR_STATE (-3)
 #define LCX_ERR_SINGULAR (-4) /* a pivot of the details-path solve was exactly zero: numpy raises LinAlgError there */
+#define LCX_ERR_NOT_PD (-5)   /* the covariance estimate is not (treated as) positive definite: lcx_lowrank_factor */
 
 /* precision modes */
 #define LCX_PRECISION_FP64 0   /* DMMA (mma.sync m8n8k4 f64) contractions, everything in binary64 */
@@ -249,6 +250,30 @@ int lcx_get_covariance(lcx_session* s, int synergy, double eps, const double* sd
  * synergy: left = X_i Z_j^T, right = X_i Y_j^T, scale = 1. */
 int lcx_covariance_rows(lcx_session* s, const double* left, const double* right, long long ld, int n_factors, int n_vars,
                         double scale, const double* sd, int row0, int rows, double* out, long long ldc);
+
+/* ---- scoring under the covariance estimate (ns variant; no bound problem needed) ------------------------------------
+ * The ns estimate is low rank plus diagonal:  Sigma = S (Z^T Z + Delta) S  with  Z = rhoinvrho / (1 + Si) / sqrt(1 - eps^2),
+ * Delta = diag(1 - sum_j Z_ji^2),  S = diag(sd).  With K = I + Z Delta^-1 Z^T = G G^T and B = G^-1 Z Delta^-1 (Woodbury):
+ *   Sigma^-1 = S^-1 (Delta^-1 - B^T B) S^-1,   log det Sigma = 2 sum log sd + sum log Delta + 2 sum log G_kk.
+ * lcx_lowrank_factor: rhoinvrho (m x ld), si (n), sd (n) device -> b (m x ldb), dinv (n) = 1 / Delta, logdet (1 double), all
+ *   device, enqueued on the stream; ONE mailbox read returns the status: LCX_ERR_NOT_PD when some Delta_i <= 0 or a pivot of
+ *   K is <= 0 (Delta_i <= 0 is a conservative test).  scratch >= lcx_lowrank_scratch_doubles(m, n).
+ * lcx_score_rows: raw fp32 / fp64 rows (ld ldx) -> maha[l] = (x~_l)^T C^-1 x~_l (squared Mahalanobis distance, C = S^-1 Sigma
+ *   S^-1) and logpdf[l] = log N(x_l; mean, Sigma), device, with x~ = (impute(x) - mean) / sd (lcx_standardize's 'standard'
+ *   arithmetic).  All binary64 (DMMA); rows never share a reduction, so results do not depend on how rows are blocked.
+ *   scratch >= lcx_score_scratch_doubles(n_rows, n_vars, n_factors).
+ * lcx_precision_rows: rows [row0, row0 + rows) of Sigma^-1 into out (rows x ldc, device); row0 even, ldc even. */
+long long lcx_lowrank_scratch_doubles(int n_factors, int n_vars);
+int lcx_lowrank_factor(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
+                       double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* scratch,
+                       long long scratch_doubles);
+long long lcx_score_scratch_doubles(long long n_rows, int n_vars, int n_factors);
+int lcx_score_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                   double marker, const double* impute, const double* mean, const double* sd, const double* b, long long ldb,
+                   int n_factors, const double* dinv, const double* logdet, double* maha, double* logpdf, double* scratch,
+                   long long scratch_doubles);
+int lcx_precision_rows(lcx_session* s, const double* b, long long ldb, int n_factors, int n_vars, const double* dinv,
+                       const double* sd, int row0, int rows, double* out, long long ldc);
 
 /* ---- raw FP64 tensor-core GEMM (unit tests / building block) ----------------------------------- */
 /* layout: 0 = A[M][K], B[N][K];  1 = A[K][M], B[K][N];  2 = A[M][K], B[K][N].  C = A*B (+ cadd), optionally

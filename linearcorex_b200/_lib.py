@@ -9,7 +9,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "liblcx_b200.so")
 
 OK, QUICK_FAIL = 0, 1
-ERR_SINGULAR = -4
+ERR_SINGULAR, ERR_NOT_PD = -4, -5
 PRECISION_FP64, PRECISION_FAST, PRECISION_FP64_SPLIT, PRECISION_FP64_SPLIT5, PRECISION_FP64_SPLIT7 = 0, 1, 2, 3, 4
 PRECISIONS = {"fp64": PRECISION_FP64, "fast": PRECISION_FAST, "fp64_split": PRECISION_FP64_SPLIT,
               "fp64_split5": PRECISION_FP64_SPLIT5, "fp64_split7": PRECISION_FP64_SPLIT7}
@@ -80,6 +80,11 @@ SIGNATURES = {
     "lcx_update_syn": (_i, [_p, _d, _pd, _pd]),
     "lcx_get_covariance": (_i, [_p, _i, _d, _p, _i, _i, _p, _ll]),
     "lcx_covariance_rows": (_i, [_p, _p, _p, _ll, _i, _i, _d, _p, _i, _i, _p, _ll]),
+    "lcx_lowrank_scratch_doubles": (_ll, [_i, _i]),
+    "lcx_lowrank_factor": (_i, [_p, _p, _p, _ll, _i, _i, _d, _p, _p, _ll, _p, _p, _p, _ll]),
+    "lcx_score_scratch_doubles": (_ll, [_ll, _i, _i]),
+    "lcx_score_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _p, _ll, _i, _p, _p, _p, _p, _p, _ll]),
+    "lcx_precision_rows": (_i, [_p, _p, _ll, _i, _i, _p, _p, _i, _i, _p, _ll]),
     "lcx_gemm_f64": (_i, [_p, _i, _i, _i, _i, _p, _ll, _p, _ll, _p, _ll, _i, _p, _i, _p, _ll]),
     "lcx_solve_scratch_doubles": (_ll, [_i]),
     "lcx_solve": (_i, [_p, _p, _ll, _i, _p, _ll, _p, _ll, _i, _p, _ll]),
@@ -114,6 +119,9 @@ def check(rc, what=""):
     if rc == ERR_SINGULAR:  # np.linalg.solve raises this at linearcorex.py:280 / :366
         import numpy as np
         raise np.linalg.LinAlgError("Singular matrix")
+    if rc == ERR_NOT_PD:  # what np.linalg.cholesky raises on the dense covariance
+        import numpy as np
+        raise np.linalg.LinAlgError("Matrix is not positive definite")
     if rc < 0:
         msg = load().lcx_last_error()
         raise LcxError("%s failed (%d): %s" % (what or "lcx call", rc, msg.decode() if msg else "?"))

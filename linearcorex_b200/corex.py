@@ -50,6 +50,16 @@ behaviour):
   stream_rows         split modes: prepare X in row blocks of this many rows (three streaming passes over the raw
                       input, X~ never materialised in fp64).  Default: automatic when X~ would not fit -- this is
                       what lets the 1M x 20k x 100 target run on ONE B200 (120 GB of int8 digit planes).
+
+Methods beyond the reference (sklearn's covariance-estimator interface; discourage_overlap=True models with theta):
+  score_samples(x)    log N(x_l; theta[0], get_covariance()) per row, in the units of the input (g() of 'outliers' is not
+                      applied: it is the density of the covariance estimate itself)
+  score(x)            their mean (over all ranks' rows with `comm`)
+  mahalanobis(x)      squared Mahalanobis distances under the same Gaussian
+  get_precision()     the inverse of get_covariance(), in row blocks, with get_covariance's output options
+The estimate is low rank plus diagonal, S (Z^T Z + Delta) S, so none of these forms or factors an n x n matrix: a factor
+B = G^-1 Z Delta^-1 (m x n) is built from the moments on each call and a row costs O(n m), in binary64 on the DMMA engine.
+Inputs are handled as by transform (containers, row providers, imputation of missing entries with the new data's means).
 """
 import ctypes as C
 import os
@@ -1073,15 +1083,16 @@ class Corex(object):
         free, _total = torch.cuda.mem_get_info(self._session().device)
         return int(self.stream_rows or 32768) if n_rows * self._session().lib.lcx_ld(n_vars) * 12 > 0.8 * free else 0
 
-    def _transform_streamed(self, x, rows):
-        """transform() in row blocks: preprocess (stored theta; imputation means of the new data from a first pass when a
-        missing marker is set, :389/:404) and project block by block into one (N, ldy) device tensor."""
+    def _row_blocks(self, x, rows, per_block):
+        """The row-block loop over new data (transform, scoring): imputation means of the new data from a first pass when a
+        missing marker is set (:389/:404; summed over ranks with `comm`), the stored theta, then
+        per_block(lo, hi, xd, dtype, impute, mean, sd) for every block [lo, hi) of `rows` rows uploaded as device tensor xd.
+        `x` only needs `.shape` and row slicing."""
         torch = _torch()
         sess = self._session()
         lib = sess.lib
         red = self._reducer()
         N, n = int(np.shape(x)[0]), int(np.shape(x)[1])
-        ld, ldy = lib.lcx_ld(n), lib.lcx_ldy(self.m)
         has_marker = self.missing_values is not None
         marker = float(self.missing_values) if has_marker else 0.0
         mode = _lib.GAUSS[self.gaussianize]
@@ -1107,18 +1118,32 @@ class Corex(object):
             if self._theta_dev is None:
                 self._theta_dev = tuple(torch.as_tensor(np.asarray(t, dtype=np.float64), device=sess.device) for t in self.theta)
             mean, sd = self._theta_dev
+        for lo, hi in blocks:
+            xd = self._as_input(x[lo:hi])
+            per_block(lo, hi, xd, _lib.F32 if xd.dtype == torch.float32 else _lib.F64, impute, mean, sd)
+
+    def _transform_streamed(self, x, rows):
+        """transform() in row blocks (_row_blocks): preprocess and project block by block into one (N, ldy) device tensor."""
+        torch = _torch()
+        sess = self._session()
+        lib = sess.lib
+        N, n = int(np.shape(x)[0]), int(np.shape(x)[1])
+        ld, ldy = lib.lcx_ld(n), lib.lcx_ldy(self.m)
+        has_marker = self.missing_values is not None
+        marker = float(self.missing_values) if has_marker else 0.0
+        mode = _lib.GAUSS[self.gaussianize]
         p = lambda t: t.data_ptr() if t is not None else None
         wd = torch.zeros((self.m, ld), dtype=torch.float64, device=sess.device)
         wd[:, :n].copy_(torch.from_numpy(np.ascontiguousarray(self.ws, dtype=np.float64)))
         xt = torch.empty((rows, ld), dtype=torch.float64, device=sess.device)
         y = torch.empty((N, ldy), dtype=torch.float64, device=sess.device)
-        for lo, hi in blocks:
-            xd = self._as_input(x[lo:hi])
-            dt = _lib.F32 if xd.dtype == torch.float32 else _lib.F64
+
+        def block(lo, hi, xd, dt, impute, mean, sd):
             _lib.check(lib.lcx_standardize(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker, mode,
                                            p(impute), p(mean), p(sd), xt.data_ptr(), ld), "lcx_standardize")
             _lib.check(lib.lcx_project(sess.h, xt.data_ptr(), hi - lo, n, ld, wd.data_ptr(), ld, self.m,
                                        y[lo:hi].data_ptr(), ldy, None, None, 0), "lcx_project")
+        self._row_blocks(x, rows, block)
         return y
 
     def transform(self, x, details=False, return_device=False):
@@ -1172,12 +1197,17 @@ class Corex(object):
             return self.theta[1] * (core + np.arctanh(np.clip(x - core, -1 + 1e-10, 1 - 1e-10))) + self.theta[0]
         return x
 
+    def _live_moments(self):
+        """True when the session's workspace holds this model's final moments."""
+        sess = self._session()
+        return sess.ws is not None and sess.n == self.nv and sess.m == self.m and getattr(self, "_fitted_in_session", False)
+
     def _factor_major_device(self, key, live_id):
         """(m x ld) device tensor of an n x m moments array: the live workspace view, or an upload of the host copy
         (a model restored from a pickle has only host state, which is all the reference reads at :440-455)."""
         torch = _torch()
         sess = self._session()
-        if sess.ws is not None and sess.n == self.nv and sess.m == self.m and getattr(self, "_fitted_in_session", False):
+        if self._live_moments():
             v = sess.view(live_id)
             return v, v.stride(0)
         ld = sess.lib.lcx_ld(self.nv)
@@ -1226,23 +1256,133 @@ class Corex(object):
             left, ld = self._factor_major_device("X_i Z_j", _lib.A_XZ)
             right, _ = self._factor_major_device("X_i Y_j", _lib.A_XY)
             scale = 1.
+
+        def fill(r0, rows, dst, ldd):
+            _lib.check(lib.lcx_covariance_rows(sess.h, left.data_ptr(), right.data_ptr(), ld, self.m, n, float(scale),
+                                               sd.data_ptr(), r0, rows, dst.data_ptr(), ldd), "lcx_covariance_rows")
+        return self._n_by_n_rows(fill, block_rows, out, block_callback)
+
+    def _n_by_n_rows(self, fill, block_rows, out, block_callback):
+        """Output side of get_covariance / get_precision: fill(row0, rows, dst, ld_dst) writes a row block of the n x n matrix
+        into device memory; the blocks go to a new ndarray, to `out` (ndarray / memmap, or a CUDA tensor written in place) or
+        to `block_callback`."""
+        torch = _torch()
+        sess = self._session()
+        n = self.nv
         on_device = isinstance(out, torch.Tensor) and out.is_cuda
         if on_device:
             assert tuple(out.shape) == (n, n) and out.dtype == torch.float64 and out.stride(1) == 1 and out.stride(0) % 2 == 0, \
                 "out must be an (n, n) float64 CUDA tensor with unit column stride and an even row stride"
         elif out is None and block_callback is None:
             out = np.empty((n, n), dtype=np.float64)
-        ldc = lib.lcx_ld(n)
+        ldc = sess.lib.lcx_ld(n)
         block_rows = max(2, min(block_rows, n + (n % 2)))
         block_rows -= block_rows % 2
         buf = None if on_device else torch.empty((block_rows, ldc), dtype=torch.float64, device=sess.device)
         for r0 in range(0, n, block_rows):
             rows = min(block_rows, n - r0)
             dst, ldd = (out[r0:r0 + rows], out.stride(0)) if on_device else (buf, ldc)
-            _lib.check(lib.lcx_covariance_rows(sess.h, left.data_ptr(), right.data_ptr(), ld, self.m, n, float(scale),
-                                               sd.data_ptr(), r0, rows, dst.data_ptr(), ldd), "lcx_covariance_rows")
+            fill(r0, rows, dst, ldd)
             if block_callback is not None:
                 block_callback(r0, dst[:rows, :n])
             elif not on_device:
                 out[r0:r0 + rows] = buf[:rows, :n].cpu().numpy()
         return out
+
+    # ------------------------------------------------------------------------------------------
+    # scoring under the covariance estimate (lowrank_kernels.cuh)
+    # ------------------------------------------------------------------------------------------
+    def _lowrank_factor(self):
+        """Device factor of the ns estimate Sigma = S (Z^T Z + Delta) S (lcx_lowrank_factor): returns (B, ldb, 1/Delta,
+        log det Sigma, theta[1]) as CUDA tensors.  Built from the moments on every call (about one m x m x n product): from
+        the live workspace when the session holds this model's final moments, otherwise uploaded from the host moments (an
+        unpickled model)."""
+        torch = _torch()
+        if self.theta is None:
+            raise ValueError("scoring needs theta (gaussianize='none' has none, like get_covariance)")
+        if not self.discourage_overlap:
+            raise ValueError("scoring supports discourage_overlap=True only: the synergy covariance X_i Z_j X_i Y_j^T with its "
+                             "diagonal reset has no symmetric low-rank factor to build on")
+        sess = self._session()
+        lib = sess.lib
+        n, m = self.nv, self.m
+        if self._live_moments():
+            rinv, si = sess.view(_lib.A_RHOINVRHO), sess.view(_lib.A_SI)[0]
+            ld = rinv.stride(0)
+        else:  # rhoinvrho is factor-major (m x n) in the host moments already
+            ld = lib.lcx_ld(n)
+            rinv = torch.zeros((m, ld), dtype=torch.float64, device=sess.device)
+            rinv[:, :n].copy_(torch.from_numpy(np.ascontiguousarray(self.moments["rhoinvrho"], dtype=np.float64)))
+            si = torch.as_tensor(np.asarray(self.moments["Si"], dtype=np.float64), device=sess.device)
+        sd = torch.as_tensor(np.asarray(self.theta[1], dtype=np.float64), device=sess.device)
+        ldb = lib.lcx_ld(n)
+        b = torch.zeros((m, ldb), dtype=torch.float64, device=sess.device)
+        dinv = torch.empty(n, dtype=torch.float64, device=sess.device)
+        logdet = torch.empty(1, dtype=torch.float64, device=sess.device)
+        nscr = lib.lcx_lowrank_scratch_doubles(m, n)
+        scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+        _lib.check(lib.lcx_lowrank_factor(sess.h, rinv.data_ptr(), si.data_ptr(), ld, m, n, float(self.eps), sd.data_ptr(),
+                                          b.data_ptr(), ldb, dinv.data_ptr(), logdet.data_ptr(), scratch.data_ptr(), nscr),
+                   "lcx_lowrank_factor")
+        return b, ldb, dinv, logdet, sd
+
+    def _scores(self, x):
+        """(q, log p) of the rows of x as (N,) float64 CUDA tensors: raw rows go through transform's row-block loop and
+        lcx_score_rows (standardise + sum x~^2 / Delta, Y = X~ B^T on the DMMA engine, finish)."""
+        torch = _torch()
+        sess = self._session()
+        lib = sess.lib
+        N, nv = int(np.shape(x)[0]), int(np.shape(x)[1])
+        assert self.nv == nv, "Incorrect number of variables in input, %d instead of %d" % (nv, self.nv)
+        b, ldb, dinv, logdet, _sd = self._lowrank_factor()
+        maha = torch.empty(N, dtype=torch.float64, device=sess.device)
+        logp = torch.empty(N, dtype=torch.float64, device=sess.device)
+        if N == 0:
+            return maha, logp
+        rows = min(self._transform_rows_for(x) or N, N)
+        nscr = lib.lcx_score_scratch_doubles(rows, nv, self.m)
+        scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+        has_marker = self.missing_values is not None
+        marker = float(self.missing_values) if has_marker else 0.0
+
+        def block(lo, hi, xd, dt, impute, mean, sd):
+            _lib.check(lib.lcx_score_rows(sess.h, xd.data_ptr(), dt, hi - lo, nv, xd.stride(0), int(has_marker), marker,
+                                          impute.data_ptr() if impute is not None else None, mean.data_ptr(), sd.data_ptr(),
+                                          b.data_ptr(), ldb, self.m, dinv.data_ptr(), logdet.data_ptr(), maha[lo:hi].data_ptr(),
+                                          logp[lo:hi].data_ptr(), scratch.data_ptr(), nscr), "lcx_score_rows")
+        self._row_blocks(x, rows, block)
+        return maha, logp
+
+    def score_samples(self, x):
+        """log p(x_l) under N(theta[0], get_covariance()) for every row, in the units of the input: an (N,) float64 ndarray.
+
+        For gaussianize='standard' this is multivariate_normal(theta[0], get_covariance()).logpdf(x).  For 'outliers' it is
+        the same Gaussian density of the raw x -- theta and get_covariance() as the model reports them; g() is deliberately
+        not applied, so the density is that of the covariance estimate itself.  Missing entries (missing_values) are imputed
+        with the new data's column means, as transform does.  Computed in binary64 from the low-rank-plus-diagonal structure
+        of the estimate (O(n m) per row, no n x n matrix); results do not depend on how the rows are blocked.  Raises
+        LinAlgError when the estimate is not positive definite (some Delta_i <= 0)."""
+        return self._scores(x)[1].cpu().numpy()
+
+    def mahalanobis(self, x):
+        """Squared Mahalanobis distances (x_l - theta[0])^T Sigma^-1 (x_l - theta[0]) of the rows: an (N,) float64 ndarray."""
+        return self._scores(x)[0].cpu().numpy()
+
+    def score(self, x):
+        """Mean log-likelihood of the rows of x (the mean of score_samples).  With `comm` set, x is this rank's row block and
+        the mean is over all ranks' rows; every rank returns the same value."""
+        logp = self._scores(x)[1].cpu().numpy()
+        red = self._reducer()
+        return float(red.sum_scalar(float(np.sum(logp)))) / float(red.sum_scalar(len(logp)))
+
+    def get_precision(self, block_rows=4096, out=None, block_callback=None):
+        """n x n precision matrix Sigma^-1 = S^-1 (Delta^-1 - B^T B) S^-1 of the covariance estimate, in row blocks on the
+        device; `block_rows`, `out` and `block_callback` as for get_covariance."""
+        lib = self._session().lib
+        n = self.nv
+        b, ldb, dinv, _logdet, sd = self._lowrank_factor()
+
+        def fill(r0, rows, dst, ldd):
+            _lib.check(lib.lcx_precision_rows(self._sess.h, b.data_ptr(), ldb, self.m, n, dinv.data_ptr(), sd.data_ptr(), r0,
+                                              rows, dst.data_ptr(), ldd), "lcx_precision_rows")
+        return self._n_by_n_rows(fill, block_rows, out, block_callback)

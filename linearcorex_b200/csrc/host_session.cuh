@@ -11,6 +11,7 @@
 #include "dgemm_mma.cuh"
 #include "fused_allreduce.cuh"
 #include "fused_strip_kernels.cuh"
+#include "lowrank_kernels.cuh"
 #include "lu_solve.cuh"
 #include "ozaki_i8.cuh"
 #include "preprocess_kernels.cuh"

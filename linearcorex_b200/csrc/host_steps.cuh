@@ -189,14 +189,16 @@ static bool mailbox_posted() {
     }
     return v != 0;
 }
-static int read_mailbox(lcx_session* s) {
+// scalars: 16 device doubles to post; default: the bound workspace's LCX_A_SCALARS (free-standing calls pass their own).
+static int read_mailbox(lcx_session* s, const double* scalars = nullptr) {
+    if (scalars == nullptr) scalars = s->ptr(LCX_A_SCALARS);
     if (!mailbox_posted()) {
-        LCX_CUDA(cudaMemcpyAsync(s->mailbox, s->ptr(LCX_A_SCALARS), 16 * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        LCX_CUDA(cudaMemcpyAsync(s->mailbox, scalars, 16 * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
         LCX_CUDA(cudaStreamSynchronize(s->stream));
         return 0;
     }
     const unsigned long long seq = ++s->mailbox_seq;
-    post_mailbox_kernel<<<1, 32, 0, s->stream>>>(s->ptr(LCX_A_SCALARS), s->mailbox, seq);
+    post_mailbox_kernel<<<1, 32, 0, s->stream>>>(scalars, s->mailbox, seq);
     LAUNCHED(s);
     volatile unsigned long long* flag = reinterpret_cast<volatile unsigned long long*>(s->mailbox + 16);
     unsigned polls = 0;

@@ -1050,3 +1050,173 @@ extern "C" int lcx_solve(lcx_session* s, const double* a, long long lda, int m, 
     if (status != 0) return fail(LCX_ERR_SINGULAR, "lcx_solve", "Singular matrix");
     return 0;
 }
+
+// ---- scoring under the covariance estimate (lowrank_kernels.cuh) ---------------------------------------------------------
+namespace {
+// scratch of lcx_lowrank_factor: zh | zd (m x ldz each) | K - I (m x ldk) | split-K partials | work of the cooperative factor |
+// lup (m x m) | perm (m ints) | status (2 ints) | per-column log terms (n) | log pivots (m) | mailbox scalars (16)
+struct LowrankScratch {
+    double *zh, *zd, *kmat, *part, *work, *lup, *ldiag, *lpiv, *scalars;
+    int *perm, *status;
+    long long ldz, ldk, total;
+    GemmPlan plan;
+};
+LowrankScratch lowrank_carve(double* base, int m, int n) {
+    LowrankScratch c;
+    c.ldz = round_up(n, 16);
+    c.ldk = round_up(m, 16);
+    c.plan = plan_gemm(m, m, n, kSMs, kMaxSplitsSmall, true);
+    long long cur = 0;
+    auto take = [&](long long count) {
+        double* p = base ? base + cur : nullptr;
+        cur = align16(cur + count);
+        return p;
+    };
+    c.zh = take((long long)m * c.ldz);
+    c.zd = take((long long)m * c.ldz);
+    c.kmat = take((long long)m * c.ldk);
+    c.part = take(c.plan.splits > 1 ? (long long)c.plan.splits * m * c.ldk : 16);
+    c.work = take(m <= lowrank::kCholSmemMaxM ? 16 : (long long)m * lu::factor_ld(m, false));
+    c.lup = take((long long)m * m);
+    c.perm = reinterpret_cast<int*>(take((m + 1) / 2 + 1));
+    c.status = reinterpret_cast<int*>(take(1));
+    c.ldiag = take(n);
+    c.lpiv = take(m);
+    c.scalars = take(16);
+    c.total = cur;
+    return c;
+}
+}  // namespace
+
+extern "C" long long lcx_lowrank_scratch_doubles(int n_factors, int n_vars) {
+    if (n_factors <= 0 || n_vars <= 0) return -1;
+    return lowrank_carve(nullptr, n_factors, n_vars).total;
+}
+
+extern "C" int lcx_lowrank_factor(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
+                                  double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* scratch,
+                                  long long scratch_doubles) {
+    LCX_REQUIRE(s && rhoinvrho && si && sd && b && dinv && logdet && scratch, "null argument");
+    const int m = n_factors, n = n_vars;
+    LCX_REQUIRE(m > 0 && n > 0 && ld >= n && ldb >= n && ldb % 2 == 0, "bad shape (ldb must be even and >= n_vars)");
+    LCX_REQUIRE(eps >= 0.0 && eps < 1.0, "eps must lie in [0, 1)");
+    LCX_REQUIRE(scratch_doubles >= lcx_lowrank_scratch_doubles(m, n), "scratch too small (see lcx_lowrank_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const LowrankScratch c = lowrank_carve(scratch, m, n);
+    LCX_CUDA(cudaMemsetAsync(c.status, 0, 2 * sizeof(int), s->stream));
+    lowrank::factor_prep_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(rhoinvrho, si, ld, c.ldz, m, n, 1.0 / sqrt(1.0 - eps * eps), sd,
+                                                                     c.zh, c.zd, dinv, c.ldiag, c.status);
+    LAUNCHED(s);
+    {   // K - I = (Z Delta^-1/2)(Z Delta^-1/2)^T: both operands K-contiguous, split-K over the variables, fixed-order combine;
+        // the identity is added where the factorisation loads K
+        GemmArgs a;
+        memset(&a, 0, sizeof(a));
+        a.A = c.zh; a.B = c.zh; a.C = c.kmat;
+        a.M = m; a.N = m; a.K = n;
+        a.lda = c.ldz; a.ldb = c.ldz; a.ldc = c.ldk;
+        LCX_TRY(run_gemm(s, kLayoutKK, c.plan, a, c.part, (long long)m * c.ldk));
+    }
+    static PerDeviceOnce attr_smem = {}, attr_coop = {};
+    if (m <= lowrank::kCholSmemMaxM) {
+        const size_t smem = (size_t)m * (m | 1) * sizeof(double);
+        if (attr_smem.first_time())
+            LCX_CUDA(cudaFuncSetAttribute(lowrank::chol_factor_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 216 * 1024));
+        lowrank::chol_factor_kernel<true><<<1, lowrank::kCholThreads, smem, s->stream>>>(c.kmat, c.ldk, m, nullptr, c.lup, m, c.perm,
+                                                                                        c.lpiv, c.status);
+    } else {
+        if (attr_coop.first_time())
+            LCX_CUDA(cudaFuncSetAttribute(lowrank::chol_factor_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 216 * 1024));
+        const int grid = min(64, (m + 15) / 16);
+        const double* kmat = c.kmat;
+        long long ldk = c.ldk, ldl = m;
+        int mm = m;
+        double* work = c.work;
+        double* lup = c.lup;
+        int* perm = c.perm;
+        double* lpiv = c.lpiv;
+        int* status = c.status;
+        void* args[] = {&kmat, &ldk, &mm, &work, &lup, &ldl, &perm, &lpiv, &status};
+        LCX_CUDA(cudaLaunchCooperativeKernel((void*)lowrank::chol_factor_kernel<false>, dim3(grid), dim3(lowrank::kCholThreads), args, 0,
+                                             s->stream));
+    }
+    LAUNCHED(s);
+    // B = G^-1 (Z Delta^-1) = diag(G)^-1 L^-1 (Z Delta^-1): the details path's triangular sweeps, identity permutation
+    LCX_TRY(lu::launch_solve(c.lup, m, c.perm, m, c.zd, c.ldz, b, ldb, n, c.status, nullptr, s->stream, &s->launches));
+    lowrank::logdet_kernel<<<1, 256, 0, s->stream>>>(c.ldiag, n, c.lpiv, m, c.status, logdet, c.scalars);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
+    LCX_TRY(read_mailbox(s, c.scalars));
+    if (s->mailbox[0] != 0.0) return fail(LCX_ERR_NOT_PD, "lcx_lowrank_factor", "Matrix is not positive definite");
+    return 0;
+}
+
+extern "C" long long lcx_score_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
+    if (n_rows <= 0 || n_vars <= 0 || n_factors <= 0) return -1;
+    return align16(n_rows * round_up(n_vars, 16)) + align16(n_rows) + align16(n_rows * round_up(n_factors, 8));
+}
+
+extern "C" int lcx_score_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                              double marker, const double* impute, const double* mean, const double* sd, const double* b, long long ldb,
+                              int n_factors, const double* dinv, const double* logdet, double* maha, double* logpdf, double* scratch,
+                              long long scratch_doubles) {
+    LCX_REQUIRE(s && x && mean && sd && b && dinv && logdet && maha && logpdf && scratch, "null argument");
+    LCX_REQUIRE(has_marker == 0 || impute != nullptr, "imputation means required when a missing marker is set");
+    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && n_vars > 0 && n_factors > 0 && ldx >= n_vars && ldb >= n_vars && ldb % 2 == 0,
+                "bad shape");
+    LCX_REQUIRE(scratch_doubles >= lcx_score_scratch_doubles(n_rows, n_vars, n_factors),
+                "scratch too small (see lcx_score_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const long long ld = round_up(n_vars, 16), ldy = round_up(n_factors, 8);
+    double* xt = scratch;
+    double* ssq = xt + align16(n_rows * ld);
+    double* y = ssq + align16(n_rows);
+    const int nan_marker = marker != marker;
+    if (dtype == LCX_F32 && vec4_ok((const float*)x, ldx))
+        lowrank::score_standardize_kernel<float, true><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const float*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+    else if (dtype == LCX_F32)
+        lowrank::score_standardize_kernel<float, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const float*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+    else if (dtype == LCX_F64 && vec4_ok((const double*)x, ldx))
+        lowrank::score_standardize_kernel<double, true><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const double*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+    else if (dtype == LCX_F64)
+        lowrank::score_standardize_kernel<double, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const double*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+    else
+        return fail(LCX_ERR_ARG, "lcx_score_rows", "unknown dtype");
+    LAUNCHED(s);
+    // Y = X~ B^T on the DMMA engine (transform's projection, no split-K: every row's sums run in the same order)
+    LCX_TRY(lcx_project(s, xt, n_rows, n_vars, ld, b, ldb, n_factors, y, ldy, nullptr, nullptr, 0));
+    lowrank::score_finish_kernel<<<cdiv(n_rows, 8), 256, 0, s->stream>>>(y, ldy, ssq, n_rows, n_factors, logdet,
+                                                                         (double)n_vars * log(2.0 * M_PI), maha, logpdf);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// rows [row0, row0 + rows) of Sigma^-1 = S^-1 (Delta^-1 - B^T B) S^-1: B^T B on the DMMA engine in get_covariance's layout
+// (z^T z), then the diagonal and the scales.  The twin of lcx_covariance_rows.
+extern "C" int lcx_precision_rows(lcx_session* s, const double* b, long long ldb, int n_factors, int n_vars, const double* dinv,
+                                  const double* sd, int row0, int rows, double* out, long long ldc) {
+    LCX_REQUIRE(s && b && dinv && sd && out, "null argument");
+    LCX_REQUIRE(n_factors > 0 && n_vars > 0 && ldb >= n_vars && ldb % 2 == 0, "bad shape (ldb must be even and >= n_vars)");
+    LCX_REQUIRE(row0 >= 0 && rows > 0 && row0 + rows <= n_vars && row0 % 2 == 0, "bad row block (row0 must be even)");
+    LCX_REQUIRE(ldc >= n_vars && ldc % 2 == 0, "ldc must be even and >= n_vars");
+    LCX_REQUIRE(((uintptr_t)b % 16 == 0) && ((uintptr_t)out % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    GemmPlan pl = plan_gemm(rows, n_vars, n_factors, kSMs, 1, false);
+    GemmArgs a;
+    memset(&a, 0, sizeof(a));
+    a.A = b + row0; a.B = b; a.C = out;
+    a.M = rows; a.N = n_vars; a.K = n_factors;
+    a.lda = ldb; a.ldb = ldb; a.ldc = ldc;
+    LCX_TRY(launch_gemm(kLayoutMN, pl, a, s->stream));
+    LAUNCHED(s);
+    lowrank::precision_finish_kernel<<<dim3(cdiv(n_vars, 256), rows), 256, 0, s->stream>>>(out, ldc, row0, rows, n_vars, dinv, sd);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
+    return 0;
+}

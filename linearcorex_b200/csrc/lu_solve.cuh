@@ -237,11 +237,32 @@ inline Scratch carve(double* scratch, int m) {
     return s;
 }
 
+// Enqueue the two triangular sweeps X = U^-1 L^-1 B[perm] of a factor in the lup layout (ld ldp) on `st`.
+inline int launch_solve(const double* lup, long long ldp, const int* perm, int m, const double* B, long long ldb, double* X,
+                        long long ldx, int n, const int* status, double* status_out, cudaStream_t st, long long* launches) {
+    static PerDeviceOnce attr_s = {};
+    if (m > kSolveSmemMaxM && X == B) return fail(-1, "lu::solve", "in-place solve needs m <= 832");
+    const int tiles = (n + kSolveCols - 1) / kSolveCols;
+    if (m <= kSolveSmemMaxM) {
+        const size_t smem = (size_t)m * kSolveCols * sizeof(double);
+        if (attr_s.first_time())
+            LCX_CUDA(cudaFuncSetAttribute(lu_solve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 216 * 1024));
+        lu_solve_kernel<true><<<tiles, kSolveCols * kSolveRows, smem, st>>>(lup, ldp, perm, m, B, ldb, X, ldx, n, status,
+                                                                          status_out);
+    } else {
+        lu_solve_kernel<false><<<tiles, kSolveCols * kSolveRows, 0, st>>>(lup, ldp, perm, m, B, ldb, X, ldx, n, status,
+                                                                        status_out);
+    }
+    if (launches) ++*launches;
+    LCX_CUDA(cudaGetLastError());
+    return 0;
+}
+
 // Enqueue X = A^-1 B on `st`.  Returns a negative code on a launch error.
 inline int solve(const double* A, long long lda, int m, const double* B, long long ldb, double* X, long long ldx, int n,
                  double* scratch, double* status_out, cudaStream_t st, long long* launches) {
     Scratch sc = carve(scratch, m);
-    static PerDeviceOnce attr_f_smem = {}, attr_f_coop = {}, attr_s = {};
+    static PerDeviceOnce attr_f_smem = {}, attr_f_coop = {};
     if (m <= kSmemMaxM) {
         const size_t smem = (((size_t)m * 4 + 15) & ~(size_t)15) + (size_t)m * (m | 1) * sizeof(double);
         if (attr_f_smem.first_time())
@@ -263,21 +284,7 @@ inline int solve(const double* A, long long lda, int m, const double* B, long lo
         LCX_CUDA(cudaLaunchCooperativeKernel((void*)lu_factor_kernel<false>, dim3(grid), dim3(kFactorThreads), args, smem, st));
     }
     if (launches) ++*launches;
-    if (m > kSolveSmemMaxM && X == B) return fail(-1, "lu::solve", "in-place solve needs m <= 832");
-    const int tiles = (n + kSolveCols - 1) / kSolveCols;
-    if (m <= kSolveSmemMaxM) {
-        const size_t smem = (size_t)m * kSolveCols * sizeof(double);
-        if (attr_s.first_time())
-            LCX_CUDA(cudaFuncSetAttribute(lu_solve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 216 * 1024));
-        lu_solve_kernel<true><<<tiles, kSolveCols * kSolveRows, smem, st>>>(sc.lup, m, sc.perm, m, B, ldb, X, ldx, n, sc.status,
-                                                                          status_out);
-    } else {
-        lu_solve_kernel<false><<<tiles, kSolveCols * kSolveRows, 0, st>>>(sc.lup, m, sc.perm, m, B, ldb, X, ldx, n, sc.status,
-                                                                        status_out);
-    }
-    if (launches) ++*launches;
-    LCX_CUDA(cudaGetLastError());
-    return 0;
+    return launch_solve(sc.lup, m, sc.perm, m, B, ldb, X, ldx, n, sc.status, status_out, st, launches);
 }
 
 }  // namespace lu

@@ -170,6 +170,17 @@ __device__ __forceinline__ double squash_tails(double z) {  // g(), :483-487
     return core + tanh(z - core);
 }
 
+// One element of X~ (column i): a missing entry takes impute[i] first (:404); mode 0 = 'standard' (x - mean) / std (:415),
+// 1 = 'outliers' (the same + g(), :423), 2 = 'none' (cast only).
+__device__ __forceinline__ double standardize_value(double d, int i, int has_marker, double marker, int marker_is_nan, int mode,
+                                                    const double* __restrict__ impute, const double* __restrict__ mean,
+                                                    const double* __restrict__ sd) {
+    if (is_missing_d(d, has_marker, marker, marker_is_nan)) d = impute[i];
+    if (mode == 2) return d;
+    const double o = (d - mean[i]) / sd[i];
+    return mode == 1 ? squash_tails(o) : o;
+}
+
 // X~ = (x - mean)/std  [+ g()];  missing entries take the column mean first (:404, :415, :423).
 // mode: 0 = 'standard', 1 = 'outliers', 2 = 'none' (cast only).  Output fp64, ld = ldo, columns >= n zeroed.
 template <typename T, int V>
@@ -187,17 +198,7 @@ __global__ void standardize_kernel(const T* __restrict__ x, long long N, int n, 
 #pragma unroll
     for (int j = 0; j < V; ++j) {
         const int i = i0 + j;
-        o[j] = 0.0;
-        if (i < n) {
-            double d = v[j];
-            if (is_missing_d(d, has_marker, marker, marker_is_nan)) d = impute[i];
-            if (mode == 2) {
-                o[j] = d;
-            } else {
-                o[j] = (d - mean[i]) / sd[i];
-                if (mode == 1) o[j] = squash_tails(o[j]);
-            }
-        }
+        o[j] = i < n ? standardize_value(v[j], i, has_marker, marker, marker_is_nan, mode, impute, mean, sd) : 0.0;
     }
     if constexpr (V == 1) {
         out[r * ldo + i0] = o[0];
@@ -242,14 +243,7 @@ __global__ void __launch_bounds__(128) standardize_slice_kernel(const T* __restr
         const int i = c4 + j;
         double o = 0.0;
         if (i < n) {
-            double e = v[j];
-            if (is_missing_d(e, has_marker, marker, marker_is_nan)) e = impute[i];
-            if (mode == 2) {
-                o = e;
-            } else {
-                o = (e - mean[i]) / sd[i];
-                if (mode == 1) o = squash_tails(o);
-            }
+            o = standardize_value(v[j], i, has_marker, marker, marker_is_nan, mode, impute, mean, sd);
             poison = poison || !(fabs(o) <= 1.7976931348623157e308);
         }
         oz::split_digits<S>(o, inv, radix, d[j]);
