@@ -160,10 +160,7 @@ class _HostDraw(object):
 
     def __init__(self, m, n):
         import threading
-        self.out, self.err, self._th = None, None, None
-        if os.environ.get("LCX_HOST_DRAW", "thread") != "thread":  # (A/B switch: draw inline, where the reference does)
-            self._args = (m, n)
-            return
+        self.out, self.err = None, None
         self._th = threading.Thread(target=self._run, args=(m, n), daemon=True)
         self._th.start()
 
@@ -174,10 +171,7 @@ class _HostDraw(object):
             self.err = e
 
     def result(self):
-        if self._th is None:
-            self._run(*self._args)
-        else:
-            self._th.join()
+        self._th.join()
         if self.err is not None:
             raise self.err
         return self.out

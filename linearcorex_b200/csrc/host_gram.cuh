@@ -51,11 +51,11 @@ static int gram_build_t(lcx_session* s, double* g, long long ldg, int B, double*
         p.ldc = ldg;
         p.c_split_stride = splits > 1 ? (long long)B * ldg : 0;
         p.col_scale = scale;
-        p.inv_radix = 1.0 / (double)L.radix;
+        p.inv_radix = 1.0 / (double)oz::kRadix;
         p.rows = n - c0; p.cols = nb; p.k_total = (int)s->Nl; p.k_chunk = L.oz_build_chunk;
         p.bn = bn;
         p.trans_out = 1;
-        LCX_TRY((oz::launch_oz_gemm<S, false>(map_a, map_b, p, dim3(n_tiles, cdiv(n - c0, oz::kBM), splits), s->stream, oz_cluster())));
+        LCX_TRY((oz::launch_oz_gemm<S, false>(map_a, map_b, p, dim3(n_tiles, cdiv(n - c0, oz::kBM), splits), s->stream)));
         LAUNCHED(s);
         if (splits > 1) {
             LCX_TRY(launch_reduce_splits(part, splits, (long long)B * ldg, dst, nb, n - c0, ldg, s->stream));
@@ -89,23 +89,16 @@ static int gram_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_
     const Layout& L = s->L;
     const int m = s->m, n = s->n;
     double* D = s->ptr(LCX_A_D);
-    if (s->row_parts > 0 && dot_out != nullptr) {  // grad from the fused kernel: row maxima and partial Bj are in I_FROW
-        oz::slice_rows_part_kernel<S><<<dim3(m, cdiv(L.ld8, 4 * 128)), 128, 0, s->stream>>>(
-            A, L.ld, m, n, s->ptr(I_FROW), s->ptr(I_FROW) + (long long)kSMs * L.ldm, s->row_parts, L.ldm, s->oz_xscale(),
-            s->oz_ascale(), s->oz_cscale(), dot_out, s->as(), L.ld8, (long long)m * L.ld8, (double)L.radix);
-        LAUNCHED(s);
-    } else {
     oz::row_scale_kernel<<<m, 256, 0, s->stream>>>(A, L.ld, n, s->oz_ascale(), 0, s->oz_xscale(), s->oz_cscale(), dot_b, dot_out);
     LAUNCHED(s);
     oz::slice_rows_kernel<S><<<dim3(m, cdiv(L.ld8, 4 * 128)), 128, 0, s->stream>>>(A, L.ld, m, n, s->oz_ascale(), nullptr, s->as(), L.ld8,
-                                                                              (long long)m * L.ld8, (double)L.radix);
+                                                                              (long long)m * L.ld8, (double)oz::kRadix);
     LAUNCHED(s);
-    }
     oz::GemmParams p;
     memset(&p, 0, sizeof(p));
     p.ldc = L.ld;
     p.col_scale = s->oz_cscale();
-    p.inv_radix = 1.0 / (double)L.radix;
+    p.inv_radix = 1.0 / (double)oz::kRadix;
     p.rows = n; p.cols = m; p.k_total = n;
     p.bn = s->oz_bn;
     p.trans_out = 1;
@@ -130,7 +123,7 @@ static int gram_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_
             double best = 1e300;
             for (int c = smin; c <= smax; ++c) {
                 const int rounds = cdiv((long long)mine * c, clusters);
-                const double cost = rounds * (ceil((double)kblocks / c) + oz_unit_fixed_kb()) + (c > 1 ? 1.5 * c : 0.0);
+                const double cost = rounds * (ceil((double)kblocks / c) + kOzUnitFixedKb) + (c > 1 ? 1.5 * c : 0.0);
                 if (cost < best - 1e-9) { best = cost; sp = c; }
             }
             const int chunk = (int)round_up(cdiv(n, sp), oz::kBK);
@@ -140,7 +133,7 @@ static int gram_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_
             p.k_chunk = chunk;
             p.C = splits > 1 ? s->ptr(I_PART) : D;
             p.c_split_stride = splits > 1 ? (long long)m * L.ld : 0;
-            LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(n_tiles, mine, splits), s->stream, oz_cluster())));
+            LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(n_tiles, mine, splits), s->stream)));
             LAUNCHED(s);
             if (splits > 1) {
                 LCX_TRY(launch_reduce_splits(s->ptr(I_PART) + col0, splits, (long long)m * L.ld, D + col0, m,
@@ -171,7 +164,7 @@ static int gram_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_
         p.C = D;
         p.c_split_stride = 0;
         p.k_chunk = (int)round_up(n, oz::kBK);
-        LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(n_tiles, gp.full, 1), s->stream, 2)));
+        LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(n_tiles, gp.full, 1), s->stream)));
         LAUNCHED(s);
         if (gp.rest > 0) {
             const long long col0 = (long long)gp.full * oz::kBM;
@@ -179,7 +172,7 @@ static int gram_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_
             p.k_chunk = gp.chunk;
             p.C = gp.splits > 1 ? s->ptr(I_PART) : D;
             p.c_split_stride = gp.splits > 1 ? (long long)m * L.ld : 0;
-            LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(n_tiles, gp.rest, gp.splits), s->stream, 2)));
+            LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(n_tiles, gp.rest, gp.splits), s->stream)));
             LAUNCHED(s);
             if (gp.splits > 1) {
                 LCX_TRY(launch_reduce_splits(s->ptr(I_PART) + col0, gp.splits, (long long)m * L.ld, D + col0, m, (int)(n - col0),
@@ -198,7 +191,7 @@ static int gram_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_
     p.c_split_stride = split ? (long long)m * L.ld : 0;
     p.k_chunk = L.oz1_chunk;
     LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p, dim3(cdiv(m, oz::bn_max(S)), cdiv(n, oz::kBM), L.oz1_splits),
-                                         s->stream, oz_cluster())));
+                                         s->stream)));
     LAUNCHED(s);
     if (ev) LCX_CUDA(cudaEventRecord(ev[1], s->stream));
     if (ev) LCX_CUDA(cudaEventRecord(ev[3], s->stream));

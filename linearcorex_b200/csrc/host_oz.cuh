@@ -13,7 +13,7 @@ static int oz_slice_x_t(lcx_session* s) {
     LAUNCHED(s);
     dim3 grid((unsigned)s->Nl, cdiv(L.ld8, 4 * 128));
     oz::slice_rows_kernel<S><<<grid, 128, 0, s->stream>>>(s->xt, s->ldx, (int)s->Nl, s->n, nullptr, s->oz_xscale(), s->xs(), L.ld8,
-                                                        s->Nl * L.ld8, (double)L.radix);
+                                                        s->Nl * L.ld8, (double)oz::kRadix);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     return 0;
@@ -57,11 +57,6 @@ static int oz_prepare(lcx_session* s, bool streamed) {
     return 0;
 }
 
-static int oz_cluster() {  // LCX_OZ_CLUSTER=1|2|4 overrides the cluster size of the split-integer contractions
-    const char* env = getenv("LCX_OZ_CLUSTER");
-    return env ? atoi(env) : 2;  // pairs: multicast does not lower the bytes delivered per SM, and clusters of 4 fit only 132 SMs
-}
-
 template <int S>
 static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t* ev, bool first_only, bool want_tail,
                      const double* dot_b, double* dot_out) {
@@ -70,18 +65,11 @@ static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t*
     double* Y = s->ptr(LCX_A_Y);
     double* D = s->ptr(LCX_A_D);
     // ---- Y = X~ A^T ----
-    if (s->row_parts > 0 && dot_out != nullptr) {  // grad from the fused kernel: row maxima and partial Bj are in I_FROW
-        oz::slice_rows_part_kernel<S><<<dim3(m, cdiv(L.ld8, 4 * 128)), 128, 0, s->stream>>>(
-            A, L.ld, m, n, s->ptr(I_FROW), s->ptr(I_FROW) + (long long)kSMs * L.ldm, s->row_parts, L.ldm, s->oz_xscale(),
-            s->oz_ascale(), s->oz_cscale(), dot_out, s->as(), L.ld8, (long long)m * L.ld8, (double)L.radix);
-        LAUNCHED(s);
-    } else {
     oz::row_scale_kernel<<<m, 256, 0, s->stream>>>(A, L.ld, n, s->oz_ascale(), 0, s->oz_xscale(), s->oz_cscale(), dot_b, dot_out);
     LAUNCHED(s);
     oz::slice_rows_kernel<S><<<dim3(m, cdiv(L.ld8, 4 * 128)), 128, 0, s->stream>>>(A, L.ld, m, n, s->oz_ascale(), nullptr, s->as(), L.ld8,
-                                                                              (long long)m * L.ld8, (double)L.radix);
+                                                                              (long long)m * L.ld8, (double)oz::kRadix);
     LAUNCHED(s);
-    }
     {
         oz::GemmParams p;
         memset(&p, 0, sizeof(p));
@@ -89,7 +77,7 @@ static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t*
         p.C = split1 ? s->ptr(I_PART) : Y;
         p.ldc = L.ldy; p.c_split_stride = split1 ? s->Nl * L.ldy : 0;
         p.col_scale = s->oz_cscale();
-        p.inv_radix = 1.0 / (double)L.radix;
+        p.inv_radix = 1.0 / (double)oz::kRadix;
         p.rows = (int)s->Nl; p.cols = m; p.k_total = n; p.k_chunk = L.oz1_chunk;
         p.bn = s->oz_bn;
         const int row0 = (cdiv(s->Nl, oz::kBM) - L.oz1_tail_tiles) * oz::kBM;
@@ -103,7 +91,7 @@ static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t*
             p.tail_ldc = L.ldy; p.tail_split_stride = (long long)L.oz1_tail_tiles * oz::kBM * L.ldy;
         }
         LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_x_k1, s->map_a_k1, p,
-                                             dim3(cdiv(m, oz::bn_max(S)), cdiv(s->Nl, oz::kBM), L.oz1_splits), s->stream, oz_cluster())));
+                                             dim3(cdiv(m, oz::bn_max(S)), cdiv(s->Nl, oz::kBM), L.oz1_splits), s->stream)));
         LAUNCHED(s);
         if (L.oz1_tail_tiles > 0) {
             double* dst = (split1 ? s->ptr(I_PART) + (long long)(L.oz1_splits - 1) * s->Nl * L.ldy : Y) + (long long)row0 * L.ldy;
@@ -131,7 +119,7 @@ static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t*
         return 0;
     }
     oz::slice_cols_t_kernel<S><<<dim3((unsigned)cdiv(s->Nl, 128), cdiv(m, 32)), dim3(32, 8), 0, s->stream>>>(
-        Y, L.ldy, s->Nl, m, s->oz_yscale(), s->ys(), L.ldk8, (long long)m * L.ldk8, (double)L.radix);
+        Y, L.ldy, s->Nl, m, s->oz_yscale(), s->ys(), L.ldk8, (long long)m * L.ldk8, (double)oz::kRadix);
     LAUNCHED(s);
     // ---- D = (X~^T Y)^T: tiles of 128 variables x 64 factors, stored factor-major, split over samples ----
     {
@@ -141,7 +129,7 @@ static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t*
         p.C = split ? s->ptr(I_PART) : D;
         p.ldc = L.ld; p.c_split_stride = split ? (long long)m * L.ld : 0;
         p.col_scale = s->oz_dscale();
-        p.inv_radix = 1.0 / (double)L.radix;
+        p.inv_radix = 1.0 / (double)oz::kRadix;
         p.rows = n; p.cols = m; p.k_total = (int)s->Nl; p.k_chunk = L.oz_chunk;
         p.bn = s->oz_bn;
         p.trans_out = 1;
@@ -157,7 +145,7 @@ static int oz_pair_t(lcx_session* s, const double* A, double* svec, cudaEvent_t*
             p.tail_ldc = tld; p.tail_split_stride = (long long)m * tld;
         }
         LCX_TRY((oz::launch_oz_gemm<S, false>(s->map_x_k2, s->map_y_k2, p,
-                                              dim3(cdiv(m, oz::bn_max(S)), cdiv(n, oz::kBM), L.oz_splits), s->stream, oz_cluster())));
+                                              dim3(cdiv(m, oz::bn_max(S)), cdiv(n, oz::kBM), L.oz_splits), s->stream)));
         LAUNCHED(s);
         if (L.oz_tail_tiles > 0) {
             double* dst = (split ? s->ptr(I_PART) + (long long)(L.oz_splits - 1) * m * L.ld : D) + var0;
@@ -198,12 +186,12 @@ static int oz_square_t(lcx_session* s, const double* left, const double* right, 
     oz::row_scale_kernel<<<m, 256, 0, s->stream>>>(left, L.ld, n, s->mm_scale_a());
     LAUNCHED(s);
     oz::slice_rows_kernel<S><<<gs, 128, 0, s->stream>>>(left, L.ld, m, n, s->mm_scale_a(), nullptr, s->mma(), L.ld8, st_n,
-                                                       (double)L.radix);
+                                                       (double)oz::kRadix);
     LAUNCHED(s);
     oz::row_scale_kernel<<<m, 256, 0, s->stream>>>(right, L.ld, n, s->mm_scale_b());
     LAUNCHED(s);
     oz::slice_rows_kernel<S><<<gs, 128, 0, s->stream>>>(right, L.ld, m, n, s->mm_scale_b(), nullptr, s->mmb(), L.ld8, st_n,
-                                                       (double)L.radix);
+                                                       (double)oz::kRadix);
     LAUNCHED(s);
     oz::GemmParams p;
     memset(&p, 0, sizeof(p));
@@ -212,11 +200,11 @@ static int oz_square_t(lcx_session* s, const double* left, const double* right, 
     p.ldc = L.ldm; p.c_split_stride = out_count;
     p.row_scale = s->mm_scale_a();
     p.col_scale = s->mm_scale_b();
-    p.inv_radix = 1.0 / (double)L.radix;
+    p.inv_radix = 1.0 / (double)oz::kRadix;
     p.rows = m; p.cols = m; p.k_total = n; p.k_chunk = L.mm_chunk;
     p.bn = s->oz_bn;
     LCX_TRY((oz::launch_oz_gemm<S, true>(s->map_mm_a, s->map_mm_b, p,
-                                         dim3(cdiv(m, oz::bn_max(S)), cdiv(m, oz::kBM), L.mm_splits), s->stream, oz_cluster())));
+                                         dim3(cdiv(m, oz::bn_max(S)), cdiv(m, oz::kBM), L.mm_splits), s->stream)));
     LAUNCHED(s);
     LCX_TRY(launch_reduce_splits(s->ptr(I_PART), L.mm_splits, out_count, out, m, m, L.ldm, s->stream,
                                  diag_out ? diag_out : s->ptr(I_F), diag_value));
@@ -239,17 +227,17 @@ static int oz_mn_t(lcx_session* s, const double* Q, const double* V, double* out
     oz::col_scale_finish_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(s->mm_colpart(), L.mm_slabs, L.ld, n, s->mm_colscale());
     LAUNCHED(s);
     oz::slice_colscaled_kernel<S><<<dim3(m, cdiv(L.ld8, 4 * 128)), 128, 0, s->stream>>>(V, L.ld, m, n, s->mm_colscale(), s->mmc(),
-                                                                                      L.ld8, (long long)m * L.ld8, (double)L.radix);
+                                                                                      L.ld8, (long long)m * L.ld8, (double)oz::kRadix);
     LAUNCHED(s);
     oz::row_scale_kernel<<<m, 256, 0, s->stream>>>(Q, L.ldm, m, s->mm_scale_q(), unit_diag ? 1 : 0);
     LAUNCHED(s);
     const dim3 gq(m, cdiv(L.ldm8, 4 * 128));
     if (unit_diag)
         oz::slice_rows_kernel<S, true><<<gq, 128, 0, s->stream>>>(Q, L.ldm, m, m, s->mm_scale_q(), nullptr, s->mmq(), L.ldm8,
-                                                                 (long long)m * L.ldm8, (double)L.radix);
+                                                                 (long long)m * L.ldm8, (double)oz::kRadix);
     else
         oz::slice_rows_kernel<S><<<gq, 128, 0, s->stream>>>(Q, L.ldm, m, m, s->mm_scale_q(), nullptr, s->mmq(), L.ldm8,
-                                                           (long long)m * L.ldm8, (double)L.radix);
+                                                           (long long)m * L.ldm8, (double)oz::kRadix);
     LAUNCHED(s);
     oz::GemmParams p;
     memset(&p, 0, sizeof(p));
@@ -257,13 +245,13 @@ static int oz_mn_t(lcx_session* s, const double* Q, const double* V, double* out
     p.ldc = L.ld; p.c_split_stride = 0;
     p.row_scale = s->mm_colscale();
     p.col_scale = s->mm_scale_q();
-    p.inv_radix = 1.0 / (double)L.radix;
+    p.inv_radix = 1.0 / (double)oz::kRadix;
     p.rows = n; p.cols = m; p.k_total = m; p.k_chunk = (int)round_up(m, oz::kBK);
     p.bn = s->oz_bn;
     p.trans_out = 1;
     p.c_add = c_add;
     LCX_TRY((oz::launch_oz_gemm<S, false, true>(s->map_mn_c, s->map_mn_q, p,
-                                          dim3(cdiv(m, oz::bn_max(S)), cdiv(n, oz::kBM), 1), s->stream, oz_cluster())));
+                                          dim3(cdiv(m, oz::bn_max(S)), cdiv(n, oz::kBM), 1), s->stream)));
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     return 0;
@@ -296,7 +284,7 @@ static int oz_slice_block_t(lcx_session* s, const double* xt, long long row0, lo
     const Layout& L = s->L;
     dim3 grid((unsigned)rows, cdiv(L.ld8, 4 * 128));
     oz::slice_rows_kernel<S><<<grid, 128, 0, s->stream>>>(xt, ldx, (int)rows, s->n, nullptr, s->oz_xscale(), s->xs() + row0 * L.ld8,
-                                                        L.ld8, s->Nl * L.ld8, (double)L.radix);
+                                                        L.ld8, s->Nl * L.ld8, (double)oz::kRadix);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     return 0;

@@ -10,7 +10,6 @@
 #include "corex_kernels.cuh"
 #include "dgemm_mma.cuh"
 #include "fused_allreduce.cuh"
-#include "fused_strip_kernels.cuh"
 #include "lowrank_kernels.cuh"
 #include "lu_solve.cuh"
 #include "ozaki_i8.cuh"
@@ -66,9 +65,6 @@ enum {
     I_MMC,              //              column-scaled digit slices of the operand contracted over its rows (factors)
     I_MMQ,              //              row-scaled digit slices of the m x m factor (ry or H)  [S][m][ldm8]
     I_MMV,              //              scales: col partial max (32 x ld) | col scale (ld) | row scales a, b, q (3 x ldm)
-    I_FPART,            // fused m x n phase (m <= 128, fused_strip_kernels.cuh): per-CTA partials of ry / H  [kSMs][m][ldm]
-    I_FROW,             //              per-CTA row maxima and partial Bj of grad  [2][kSMs][ldm]
-    I_TICKET,           //              arrival counters of the last-CTA reductions (self-resetting)
     I_TAIL1,            // two-level split of the first contraction: partials of the tail units  [splits][tail rows][ldy]
     I_TAIL2,            //              of the second contraction  [splits][m][tail variables]
     I_COUNT
@@ -94,20 +90,13 @@ struct Layout {
     int oz_build_splits, oz_build_chunk;                  // the uniform split over samples (what lcx_gram_build walks)
     int oz1_tail_tiles, oz1_tail_splits, oz1_tail_chunk;  // first contraction (M tiles = 128 samples)
     int ystat_slabs;
-    int radix;                   // 128: 7-bit signed digits (|d| <= 64); 254: full int8 range (|d| <= 127)
     int oz_kmax;                 // longest contraction one int32 accumulator group may see: 2^31 / ((R/2)^2 S)
     // the four m x m x n products of an iteration (ry, Qij, H, H W) on the same int8 engine (large m only)
     int mm_i8;                   // 0 = DMMA (dgemm_mma.cuh)
     long long ldm8;              // byte leading dimension of the digit slices of an m x m matrix
     int mm_splits, mm_chunk;     // split-K over the variables of the m x m outputs
     int mm_slabs, mm_slab_rows;  // row slabs of the per-column maximum
-    int fused;                   // m x n phase through fused_strip_kernels.cuh (m <= 128)
 };
-
-static int radix_for() {
-    const char* env = getenv("LCX_SPLIT_RADIX");
-    return (env && atoi(env) == 128) ? 128 : 254;  // 254: digits use the full int8 range (measured 100x tighter parity)
-}
 
 static int digits_for(int precision) {
     if (precision == LCX_PRECISION_FP64) return 0;
@@ -127,30 +116,14 @@ static int mm_i8_for(int S, int n, int m) {
     if (env) return atoi(env) != 0;
     return m >= 384 && n >= 2048;
 }
-// LCX_FUSED=1 routes the m x n phase of m <= 128 problems through fused_strip_kernels.cuh (9 launches instead of 15 per
-// iteration).  Off by default: measured on a B200 at config 3 the fused phase takes 0.26 ms against 0.23 ms for the separate
-// kernels -- with one 8-warp CTA per SM the strip kernels expose the L2 latency of their elementwise operands and DMMA.8x8x4
-// sustains only ~1 instruction per 8-9 clocks per SM in them (profiles/r02_fused_mxn_phase.md).  Kept, tested, as the
-// starting point for a version with two CTAs per SM.
-static int fused_for(int n, int m, int mm_i8) {
-    (void)n;
-    if (m > fs::kMaxM || mm_i8) return 0;
-    const char* env = getenv("LCX_FUSED");
-    return (env && atoi(env) == 1) ? 1 : 0;
-}
 constexpr int kYStatRows = 512;
 constexpr int kAmaxCtas = 592;
 
 static long long align16(long long v) { return round_up(v, 16); }
 
 // Cost of one work unit of the persistent split-integer contraction beyond its K blocks, in units of one 64-deep K block
-// (drain of the accumulators that the next unit's operand fill does not hide + the ring restart).  With one cluster per
-// unit (LCX_OZ_PERSISTENT=0) barrier set-up, TMEM allocation, the cluster handshake and the CTA launch add up to ~16.
-static double oz_unit_fixed_kb() {
-    if (const char* env = getenv("LCX_OZ_FIXED_KB")) return atof(env);
-    const char* per = getenv("LCX_OZ_PERSISTENT");
-    return (per && atoi(per) == 0) ? 16.0 : 4.0;
-}
+// (drain of the accumulators that the next unit's operand fill does not hide + the ring restart).
+constexpr double kOzUnitFixedKb = 4.0;
 
 // Two-level split of a contraction whose uniform units (M tiles x K splits, one cluster per unit and N group) do not fill whole
 // rounds of the resident clusters: R full rounds of the uniform units, and the r units left over -- the last K chunk of the
@@ -180,20 +153,16 @@ static TwoLevel plan_two_level(long long K, int m_tiles, int n_groups, int smin,
         const int tchunk = (int)round_up(cdiv(klast, t), oz::kBK);
         t = cdiv(klast, tchunk);
         if (t <= 1) continue;
-        const double cost = (double)R * (chunk / oz::kBK + oz_unit_fixed_kb()) + (tchunk / oz::kBK + oz_unit_fixed_kb()) +
+        const double cost = (double)R * (chunk / oz::kBK + kOzUnitFixedKb) + (tchunk / oz::kBK + kOzUnitFixedKb) +
                             (sp > 1 ? combine_per_split * sp : 0.0) + 4.0;  // + the fold launch
         if (cost < best.cost - 1e-9) best = TwoLevel{sp, chunk, rt, t, tchunk, cost};
     }
     return best;
 }
-// LCX_OZ_TAIL=0 switches the two-level split off; it needs the persistent unit walk and pairs of N tiles in one launch.
+// LCX_OZ_TAIL=0 switches the two-level split off; it needs pairs of N tiles in one launch.
 static bool oz_tail_allowed(int m, int S) {
     const char* env = getenv("LCX_OZ_TAIL");
     if (env && atoi(env) == 0) return false;
-    const char* per = getenv("LCX_OZ_PERSISTENT");
-    if (per && atoi(per) == 0) return false;
-    const char* cl = getenv("LCX_OZ_CLUSTER");
-    if (cl && atoi(cl) != 2) return false;
     return cdiv(m, oz::bn_max(S)) % 2 == 0;
 }
 
@@ -206,8 +175,7 @@ static GramPlan gram_plan(int n, int m, int S, int oz_kmax) {
     GramPlan g = {0, 0, 1, 0};
     const int n_tiles = cdiv(m, oz::bn_max(S)), m_tiles = cdiv(n, oz::kBM);
     const int clusters = kSMs / 2;
-    const char* env = getenv("LCX_OZ_CLUSTER");
-    if (n_tiles != 2 || (env && atoi(env) != 2) || n > oz_kmax) return g;
+    if (n_tiles != 2 || n > oz_kmax) return g;
     g.full = (m_tiles / clusters) * clusters;
     g.rest = m_tiles - g.full;
     if (g.full == 0 || g.rest == 0) return g;
@@ -224,9 +192,8 @@ static Layout make_layout(long long Nl, int n, int m, int precision, bool gram =
     Layout L;
     memset(&L, 0, sizeof(L));
     L.S = digits_for(precision);
-    L.radix = radix_for();
     if (L.S > 0) {
-        const long long half = L.radix / 2;
+        const long long half = oz::kRadix / 2;
         L.oz_kmax = (int)(((1LL << 31) / (half * half * L.S)) / 64 * 64);
         if (L.oz_kmax > 65536) L.oz_kmax = 65536;
     }
@@ -304,8 +271,8 @@ static Layout make_layout(long long Nl, int n, int m, int precision, bool gram =
         // at most oz_kmax samples per split keeps every int32 accumulator exact
         const long long tiles = (long long)cdiv(n, oz::kBM) * cdiv(m, oz::bn_max(L.S));
         const int kblocks = cdiv(Nl, oz::kBK);
-        // time model in units of one 64-deep K block: waves x (K blocks per CTA + fixed prologue/TMEM-drain/store cost
-        // of ~16 blocks) + the partial-buffer round trip; measured at 12.5k and 100k rows per GPU
+        // time model in units of one 64-deep K block: waves x (K blocks per CTA + the per-unit fixed cost kOzUnitFixedKb)
+        // + the partial-buffer round trip; measured at 12.5k and 100k rows per GPU
         int best = 1;
         double best_cost = 1e300;
         const int smin = cdiv(Nl, L.oz_kmax), smax = (int)min(64LL, (long long)max(1, kblocks / 8));
@@ -313,19 +280,15 @@ static Layout make_layout(long long Nl, int n, int m, int precision, bool gram =
             const long long ctas = tiles * sp;
             const long long waves = (ctas + kSMs - 1) / kSMs;
             const double kb = ceil((double)kblocks / sp);
-            const double cost = (double)waves * (kb + oz_unit_fixed_kb()) + (sp > 1 ? 1.5 * sp : 0.0);
+            const double cost = (double)waves * (kb + kOzUnitFixedKb) + (sp > 1 ? 1.5 * sp : 0.0);
             if (cost < best_cost - 1e-9) { best_cost = cost; best = sp; }
-        }
-        if (const char* env = getenv("LCX_OZ_SPLITS")) {  // experiment override; never below the int32-exact minimum
-            const int v = atoi(env);
-            if (v >= smin && v <= kblocks) best = v;
         }
         L.oz_chunk = (int)round_up(cdiv(Nl, best), oz::kBK);
         L.oz_splits = cdiv(Nl, L.oz_chunk);
         L.oz_build_splits = L.oz_splits;
         L.oz_build_chunk = L.oz_chunk;
         const bool tail_ok = !gram && oz_tail_allowed(m, L.S);
-        if (tail_ok && getenv("LCX_OZ_SPLITS") == nullptr) {
+        if (tail_ok) {
             const TwoLevel t2 = plan_two_level(Nl, cdiv(n, oz::kBM), cdiv(cdiv(m, oz::bn_max(L.S)), 2), smin, max(smin, smax), 1.5);
             if (t2.tail_tiles > 0 && t2.cost < best_cost) {
                 L.oz_chunk = t2.chunk; L.oz_splits = t2.splits;
@@ -340,7 +303,7 @@ static Layout make_layout(long long Nl, int n, int m, int precision, bool gram =
             const int s1min = cdiv(n, L.oz_kmax);  // int32 exactness of every accumulator group
             for (int sp = s1min; sp <= max(s1min, min(8, kblocks1 / 16)); ++sp) {
                 const long long waves = (tiles1 * sp + kSMs - 1) / kSMs;
-                const double cost = (double)waves * (ceil((double)kblocks1 / sp) + oz_unit_fixed_kb()) + (sp > 1 ? 4.0 * sp : 0.0);
+                const double cost = (double)waves * (ceil((double)kblocks1 / sp) + kOzUnitFixedKb) + (sp > 1 ? 4.0 * sp : 0.0);
                 if (cost < c1best - 1e-9) { c1best = cost; b1 = sp; }
             }
             L.oz1_chunk = (int)round_up(cdiv(n, b1), oz::kBK);
@@ -389,7 +352,7 @@ static Layout make_layout(long long Nl, int n, int m, int precision, bool gram =
                 double cbest = 1e300;
                 for (int sp = smin_mm; sp <= max(smin_mm, min(64, kblocks_mm / 8)); ++sp) {
                     const long long waves = (tiles_mm * sp + kSMs - 1) / kSMs;
-                    const double cost = (double)waves * (ceil((double)kblocks_mm / sp) + oz_unit_fixed_kb()) + 1.5 * sp;
+                    const double cost = (double)waves * (ceil((double)kblocks_mm / sp) + kOzUnitFixedKb) + 1.5 * sp;
                     if (cost < cbest - 1e-9) { cbest = cost; bmm = sp; }
                 }
                 L.mm_chunk = (int)round_up(cdiv(n, bmm), oz::kBK);
@@ -408,12 +371,6 @@ static Layout make_layout(long long Nl, int n, int m, int precision, bool gram =
             put1(I_MMV, 1, 33 * L.ld + 3 * L.ldm, 33 * L.ld + 3 * L.ldm);
         }
     }
-    L.fused = fused_for(n, m, L.mm_i8);
-    if (L.fused) {
-        put1(I_FPART, 1, (long long)kSMs * mn * L.ldm, (long long)kSMs * mn * L.ldm);
-        put1(I_FROW, 1, 2LL * kSMs * L.ldm, 2LL * kSMs * L.ldm);
-    }
-    put1(I_TICKET, 1, 16, 16);
     L.total = cur;
     if (getenv("LCX_PLAN_DEBUG") && L.S > 0)
         fprintf(stderr, "[lcx plan] Nl=%lld n=%d m=%d gram=%d | K1: splits %d chunk %d tail %d tiles x %d splits (chunk %d) | K2: splits %d "
@@ -444,8 +401,6 @@ struct lcx_session {
     double graph_eps;
     long long graph_launches[2];
     int graph_warm[2];  // iterations already run without capture on this parity (kernel attributes are configured there)
-    int tg_phys;      // physical moment set whose T / G0 (I_T, LCX_A_GRAD) the fused tail has already written, -1 = none
-    int row_parts;    // > 0: grad's row maxima / partial Bj wait in I_FROW as this many per-CTA partials (fused direction)
     int d_splits;     // > 1: the last Gram product left its split-K partials in I_PART for the consumer to add (host_gram.cuh)
     int n, m;
     double* ws;

@@ -126,10 +126,7 @@ static int xpair(lcx_session* s, const double* A, bool want_colsq, const double*
             s->prof_pending++;
         }
     } else {
-    if (dot_out && s->row_parts > 0) {  // the fused grad kernel left partial dots
-        fs::bj_finish_kernel<<<cdiv(m, 128), 128, 0, s->stream>>>(s->ptr(I_FROW) + (long long)kSMs * L.ldm, s->row_parts, L.ldm, dot_out, m);
-        LAUNCHED(s);
-    } else if (dot_out) {
+    if (dot_out) {
         row_dot_kernel<<<m, 256, 0, s->stream>>>(A, dot_b, dot_out, n, L.ld);
         LAUNCHED(s);
     }
@@ -180,23 +177,9 @@ static int xpair(lcx_session* s, const double* A, bool want_colsq, const double*
     return 0;
 }
 
-// LCX_MAILBOX=copy: cudaMemcpyAsync + cudaStreamSynchronize (the round-1 path); default: post_mailbox_kernel + polling.
-static bool mailbox_posted() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("LCX_MAILBOX");
-        v = (e && strcmp(e, "copy") == 0) ? 0 : 1;
-    }
-    return v != 0;
-}
 // scalars: 16 device doubles to post; default: the bound workspace's LCX_A_SCALARS (free-standing calls pass their own).
 static int read_mailbox(lcx_session* s, const double* scalars = nullptr) {
     if (scalars == nullptr) scalars = s->ptr(LCX_A_SCALARS);
-    if (!mailbox_posted()) {
-        LCX_CUDA(cudaMemcpyAsync(s->mailbox, scalars, 16 * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
-        LCX_CUDA(cudaStreamSynchronize(s->stream));
-        return 0;
-    }
     const unsigned long long seq = ++s->mailbox_seq;
     post_mailbox_kernel<<<1, 32, 0, s->stream>>>(scalars, s->mailbox, seq);
     LAUNCHED(s);
@@ -215,81 +198,6 @@ static int read_mailbox(lcx_session* s, const double* scalars = nullptr) {
         }
     }
     std::atomic_thread_fence(std::memory_order_acquire);
-    return 0;
-}
-
-// ---- fused m x n phase (fused_strip_kernels.cuh, m <= 128) ---------------------------------------
-struct FusedGrid {
-    int outer_grid, cols_per_cta, apply_grid;
-};
-static FusedGrid fused_grid(const lcx_session* s) {
-    FusedGrid g;
-    const int g0 = (int)min((long long)kSMs, (long long)cdiv(s->n, fs::kOuterCols));
-    g.cols_per_cta = (int)round_up(cdiv(s->n, g0), 4);
-    g.outer_grid = cdiv(s->n, g.cols_per_cta);
-    g.apply_grid = g.outer_grid;   // the same contiguous ranges of variables
-    return g;
-}
-static unsigned* ticket_ptr(lcx_session* s, int which) { return reinterpret_cast<unsigned*>(s->ptr(I_TICKET)) + 4 * which; }
-
-// Stage 1 of the moments of `set` (mode 1: rho = c1 D + e2 W; mode 2: the linear trial W + eta U, rho + eta Rdir into set 1),
-// ry, Qij, Qi-Si^2, TC, uj -- and T / G0 of the search direction that would start from this set -- in three launches.
-static int moments_fused(lcx_session* s, int set, double c1, double e2, int uj_mode, int mode, double eta) {
-    const Layout& L = s->L;
-    const int m = s->m, n = s->n;
-    const FusedGrid g = fused_grid(s);
-    fs::OuterArgs a;
-    memset(&a, 0, sizeof(a));
-    a.m = m; a.n = n; a.ld = L.ld; a.ldm = L.ldm; a.cols_per_cta = g.cols_per_cta;
-    a.part = s->ptr(I_FPART);
-    a.part_stride = (long long)m * L.ldm;
-    a.c1 = c1; a.e2 = e2; a.eta = eta;
-    a.rho = s->ptr(LCX_A_RHO, set);
-    a.invrho = s->ptr(LCX_A_INVRHO, set);
-    a.rinv = s->ptr(LCX_A_RHOINVRHO, set);
-    a.Si = s->ptr(LCX_A_SI, set);
-    if (mode == 1) {
-        a.D = s->ptr(LCX_A_D);
-        a.W = s->ptr(LCX_A_W, set);
-        LCX_TRY(fs::launch_outer<1>(a, g.outer_grid, s->stream));
-    } else {
-        a.W = s->ptr(LCX_A_W);
-        a.U = s->ptr(LCX_A_UPDATE);
-        a.rho0 = s->ptr(LCX_A_RHO);
-        a.Rdir = s->ptr(LCX_A_RDIR);
-        a.W2 = s->ptr(LCX_A_W, set);
-        LCX_TRY(fs::launch_outer<2>(a, g.outer_grid, s->stream));
-    }
-    LAUNCHED(s);
-    // ry = sum of the per-CTA partials (index order), raw diagonal -> uj by linearity, diag -> 1 (:261-263)
-    LCX_TRY(launch_reduce_splits(s->ptr(I_FPART), g.outer_grid, (long long)m * L.ldm, s->ptr(LCX_A_RY, set), m, m, L.ldm, s->stream,
-                                 s->ptr(I_UJDIAG), 1.0));
-    LAUNCHED(s);
-    fs::ApplyArgs b;
-    memset(&b, 0, sizeof(b));
-    b.m = m; b.n = n; b.ld = L.ld; b.ldm = L.ldm; b.cols_per_cta = g.cols_per_cta;
-    b.Q = s->ptr(LCX_A_RY, set);
-    b.V = s->ptr(LCX_A_RHOINVRHO, set);
-    b.rho = s->ptr(LCX_A_RHO, set);
-    b.invrho = s->ptr(LCX_A_INVRHO, set);
-    b.W = s->ptr(LCX_A_W, set);
-    b.Si = s->ptr(LCX_A_SI, set);
-    b.Qij = s->ptr(LCX_A_QIJ, set);
-    b.QiSi2 = s->ptr(LCX_A_QISI2, set);
-    b.T = s->ptr(I_T);
-    b.G0 = s->ptr(LCX_A_GRAD);
-    b.uj_mode = uj_mode;
-    b.s = s->ptr(LCX_A_D) + (long long)m * L.ld;
-    b.w2 = s->ptr(I_W2);
-    b.ujdiag = s->ptr(I_UJDIAG);
-    b.c1 = c1; b.e2 = e2;
-    b.uj = s->ptr(LCX_A_UJ, set);
-    b.part = s->ptr(I_SPART);
-    b.ticket = ticket_ptr(s, 0);
-    b.out = s->ptr(LCX_A_SCALARS);
-    LCX_TRY(fs::launch_apply<0>(b, g.apply_grid, s->stream));
-    LAUNCHED(s);
-    s->tg_phys = set ^ s->cur;
     return 0;
 }
 
@@ -343,7 +251,6 @@ static int moments_from_x(lcx_session* s, int set, double eps) {
     LCX_TRY(xpair(s, W, true));
     row_dot_kernel<<<m, 256, 0, s->stream>>>(W, W, s->ptr(I_W2), n, L.ld);
     LAUNCHED(s);
-    if (L.fused) return moments_fused(s, set, c1, e2, 0, 1, 0.0);
     moments_stage1_kernel<true><<<L.nstrips, dim3(kStripCols, kStripRows), 0, s->stream>>>(
         s->ptr(LCX_A_D), W, nullptr, nullptr, nullptr, 0.0, c1, e2, nullptr, s->ptr(LCX_A_RHO, set),
         s->ptr(LCX_A_INVRHO, set), s->ptr(LCX_A_RHOINVRHO, set), s->ptr(LCX_A_SI, set), m, n, L.ld);
@@ -361,37 +268,11 @@ static int enqueue_direction(lcx_session* s, double eps) {
     double* G = s->ptr(LCX_A_GRAD);
     double* T = s->ptr(I_T);
     double* H = s->ptr(I_RYINV);  // m x ldm scratch (the inverse buffer is idle outside the details path)
-    if (!L.fused || s->tg_phys != s->cur) {  // (the fused moments tail of the current set has already written T and G0)
-        direction_stage1_kernel<<<grid_mn(m, n), 256, 0, s->stream>>>(W, rho, s->ptr(LCX_A_INVRHO), rinv, s->ptr(LCX_A_QIJ),
-                                                                    s->ptr(LCX_A_SI), s->ptr(LCX_A_QISI2), s->ptr(LCX_A_UJ), T,
-                                                                    G, m, n, L.ld);
-        LAUNCHED(s);
-    }
-    s->tg_phys = -1;  // grad overwrites G0 below
-    s->row_parts = 0;
-    if (L.fused) {
-        const FusedGrid g = fused_grid(s);
-        fs::OuterArgs a;
-        memset(&a, 0, sizeof(a));
-        a.m = m; a.n = n; a.ld = L.ld; a.ldm = L.ldm; a.cols_per_cta = g.cols_per_cta;
-        a.part = s->ptr(I_FPART);
-        a.part_stride = (long long)m * L.ldm;
-        a.A = T; a.B = rinv;
-        LCX_TRY(fs::launch_outer<0>(a, g.outer_grid, s->stream));  // H = T rinv^T (:294), per-CTA partials
-        LAUNCHED(s);
-        LCX_TRY(launch_reduce_splits(s->ptr(I_FPART), g.outer_grid, (long long)m * L.ldm, H, m, m, L.ldm, s->stream, s->ptr(I_F),
-                                     0.0));                        // fixed-order combine, diag -> 0 (:295)
-        LAUNCHED(s);
-        fs::ApplyArgs b;
-        memset(&b, 0, sizeof(b));
-        b.m = m; b.n = n; b.ld = L.ld; b.ldm = L.ldm; b.cols_per_cta = g.cols_per_cta;
-        b.Q = H; b.V = W; b.rho = rho; b.G = G;
-        b.pmax = s->ptr(I_FROW);
-        b.pdot = s->ptr(I_FROW) + (long long)kSMs * L.ldm;
-        LCX_TRY(fs::launch_apply<1>(b, g.apply_grid, s->stream));  // grad = G0 + H W (:300) + row maxima + partial Bj
-        LAUNCHED(s);
-        s->row_parts = g.apply_grid;
-    } else if (L.mm_i8) {
+    direction_stage1_kernel<<<grid_mn(m, n), 256, 0, s->stream>>>(W, rho, s->ptr(LCX_A_INVRHO), rinv, s->ptr(LCX_A_QIJ),
+                                                                s->ptr(LCX_A_SI), s->ptr(LCX_A_QISI2), s->ptr(LCX_A_UJ), T, G,
+                                                                m, n, L.ld);
+    LAUNCHED(s);
+    if (L.mm_i8) {
         LCX_TRY(oz_square(s, T, rinv, H, 0.0, nullptr));  // H = T rinv^T, diag -> 0 (:294-295)
         LCX_TRY(oz_mn(s, H, W, G, G, false));             // grad = G0 + H W (:300)
     } else {
@@ -415,7 +296,6 @@ static int enqueue_direction(lcx_session* s, double eps) {
     // X~^T (X~ grad^T): the one pass over X of this iteration (:301); Bj = sum_i rho grad (:302) rides on its first pass over grad
     s->d_splits = 1;
     LCX_TRY(xpair(s, G, false, rho, s->ptr(I_BJ), true));
-    s->row_parts = 0;
     const dim3 g2(cdiv(n, 256), m);
     const bool parts = s->d_splits > 1;
     direction_stage2_kernel<<<g2, 256, 0, s->stream>>>(W, rho, G, parts ? s->ptr(I_PART) : s->ptr(LCX_A_D), s->ptr(LCX_A_UJ),
@@ -438,8 +318,6 @@ static int enqueue_trial(lcx_session* s, double eps, double eta, int exact) {
                                                         L.ld);
         LAUNCHED(s);
         LCX_TRY(moments_from_x(s, 1, eps));
-    } else if (L.fused) {
-        LCX_TRY(moments_fused(s, 1, c1, e2, 1, 2, eta));
     } else {
         moments_stage1_kernel<false><<<L.nstrips, dim3(kStripCols, kStripRows), 0, s->stream>>>(
             nullptr, s->ptr(LCX_A_W), s->ptr(LCX_A_UPDATE), s->ptr(LCX_A_RHO), s->ptr(LCX_A_RDIR), eta, c1, e2,

@@ -232,8 +232,6 @@ static int bind_common(lcx_session* s, const double* xt, long long n_rows_local,
     s->cur = 0;
     graphs_invalidate(s);
     s->graph_warm[0] = s->graph_warm[1] = 0;
-    s->tg_phys = -1;
-    s->row_parts = 0;
     s->d_splits = 1;
     s->bound = true;
     s->peers.world = 0;  // a new problem starts single-rank until lcx_set_peer_allreduce is called for it
@@ -343,7 +341,7 @@ extern "C" int lcx_digit_planes_info(lcx_session* s, int which, long long* offse
     if (cols) *cols = which == 2 ? s->Nl : s->n;
     if (ld_bytes) *ld_bytes = which == 2 ? L.ldk8 : L.ld8;
     if (scale_offset) *scale_offset = L.slot[I_OZV][0].off + (which == 0 ? 0 : (which == 1 ? 16 : 16 + 2 * L.ldm));
-    if (radix) *radix = L.radix;
+    if (radix) *radix = oz::kRadix;
     return 0;
 }
 
@@ -489,11 +487,11 @@ static int standardize_slice_t(lcx_session* s, const T* x, long long row0, long 
     if (vec4_ok(x, ldx))
         standardize_slice_kernel<T, S, 4><<<grid, 128, 0, s->stream>>>(x, rows, s->n, ldx, has_marker, marker, nan_marker, mode,
                                                                      impute, mean, sd, s->oz_xscale(), out, L.ld8,
-                                                                     s->Nl * L.ld8, (double)L.radix);
+                                                                     s->Nl * L.ld8, (double)oz::kRadix);
     else
         standardize_slice_kernel<T, S, 1><<<grid, 128, 0, s->stream>>>(x, rows, s->n, ldx, has_marker, marker, nan_marker, mode,
                                                                      impute, mean, sd, s->oz_xscale(), out, L.ld8,
-                                                                     s->Nl * L.ld8, (double)L.radix);
+                                                                     s->Nl * L.ld8, (double)oz::kRadix);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     return 0;
@@ -573,7 +571,6 @@ extern "C" int lcx_sig(lcx_session* s, const double* u, double eps, double* out)
 
 extern "C" int lcx_set_w(lcx_session* s, const double* host_w, long long host_ld) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     LCX_REQUIRE(host_w && host_ld >= s->n, "bad host array");
     LCX_CUDA(cudaMemcpy2DAsync(s->ptr(LCX_A_W), s->L.ld * sizeof(double), host_w, host_ld * sizeof(double),
                                (size_t)s->n * sizeof(double), s->m, cudaMemcpyHostToDevice, s->stream));
@@ -592,7 +589,6 @@ extern "C" int lcx_get_w(lcx_session* s, double* host_w, long long host_ld) {
 
 extern "C" int lcx_init_scale(lcx_session* s, double eps) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     const Layout& L = s->L;
     const int m = s->m, n = s->n;
     double* W = s->ptr(LCX_A_W);
@@ -620,7 +616,6 @@ extern "C" int lcx_init_scale(lcx_session* s, double eps) {
 
 extern "C" int lcx_stage_rescale(lcx_session* s, double eps, double eps_prev) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     const Layout& L = s->L;
     const int m = s->m, n = s->n;
     double* W = s->ptr(LCX_A_W);
@@ -636,7 +631,6 @@ extern "C" int lcx_stage_rescale(lcx_session* s, double eps, double eps_prev) {
 
 extern "C" int lcx_permute_rows(lcx_session* s, const int* host_order) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     LCX_REQUIRE(host_order != nullptr, "null order");
     const Layout& L = s->L;
     double* W = s->ptr(LCX_A_W);
@@ -694,18 +688,13 @@ extern "C" int lcx_direction_trial_ns(lcx_session* s, double eps, double eta, do
 // (README demo, big5: kernels of 2-3 us).  Measured on a B200 (tools/small_configs.py, profiles/r02_cuda_graph_ab.txt): README
 // demo 0.124 -> 0.075 ms per iteration; at config 3 a replay is 50 us SLOWER per iteration than stream launches (the host
 // waits for every iteration, so a graph's launch latency is exposed while stream launches run ahead of 5-30 us kernels), and a
-// capture costs ~1 ms, so a stage must run kGraphAfter iterations on a parity before it is captured.  LCX_GRAPH=0 / 1 forces
-// them off / on for every size.  Single-rank sessions only (the rank exchange is a cooperative kernel / a host hook).
+// capture costs ~1 ms, so a stage must run kGraphAfter iterations on a parity before it is captured.  Single-rank sessions
+// only (the rank exchange is a cooperative kernel / a host hook).
 constexpr long long kGraphMaxElems = 1 << 17;
 constexpr int kGraphAfter = 8;
 static bool graphs_enabled(const lcx_session* s) {
-    static int mode = -2;
-    if (mode == -2) {
-        const char* env = getenv("LCX_GRAPH");
-        mode = env ? (atoi(env) != 0 ? 1 : 0) : -1;
-    }
-    if (mode == 0 || s->peers.world > 1 || s->hook != nullptr || s->prof_on || s->L.fused) return false;
-    return mode == 1 || (long long)s->m * s->n <= kGraphMaxElems;
+    if (s->peers.world > 1 || s->hook != nullptr || s->prof_on) return false;
+    return (long long)s->m * s->n <= kGraphMaxElems;
 }
 
 // Direction (:292-305) + the eta = 1 trial (:320-321) + the mailbox copy of ONE iteration, replayed from a CUDA graph: ~17
@@ -879,7 +868,6 @@ extern "C" int lcx_details_ns(lcx_session* s, double* tc_no_overlap, double* add
 
 extern "C" int lcx_moments_syn(lcx_session* s, double* tc, double* additivity) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     const Layout& L = s->L;
     const int m = s->m, n = s->n;
     double* W = s->ptr(LCX_A_W);
@@ -934,7 +922,6 @@ extern "C" int lcx_moments_syn(lcx_session* s, double* tc, double* additivity) {
 
 extern "C" int lcx_update_syn(lcx_session* s, double eta, double* tc, double* additivity) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     const Layout& L = s->L;
     const int m = s->m, n = s->n;
     double* W = s->ptr(LCX_A_W);
@@ -986,7 +973,6 @@ static int covariance_rows(lcx_session* s, const double* left, const double* rig
 extern "C" int lcx_get_covariance(lcx_session* s, int synergy, double eps, const double* sd, int row0, int rows, double* out,
                                   long long ldc) {
     S_REQUIRE_BOUND(s);
-    s->tg_phys = -1;  // (T / G0 of the fused moments tail no longer match the current set)
     const Layout& L = s->L;
     const int m = s->m, n = s->n;
     LCX_REQUIRE(sd && out, "null argument");

@@ -5,7 +5,7 @@
 //
 // tcgen05.mma has no f64 kind, but kind::i8 multiplies int8 digits exactly into int32 TMEM accumulators.
 // Each fp64 operand is written as a fixed-point number with S signed int8 digits ("planes") in radix R = 254:
-//     v = 2^E * sum_{k=1..S} d_k R^-k,   |d_k| <= 127          (R = 128, |d_k| <= 64, is the power-of-two variant)
+//     v = 2^E * sum_{k=1..S} d_k R^-k,   |d_k| <= 127
 // with one exponent E for all of X~ (standardised data is bounded; chosen from max|X~|), one per factor
 // row of A and one per factor column of Y.  The product is then
 //     sum_i x_i a_i = 2^(Ex+Ea) * sum_{g=2..S+1} R^-g * P_g,   P_g = sum_{k+l=g} sum_i dx_k[i] da_l[i]
@@ -32,6 +32,7 @@
 namespace lcx {
 namespace oz {
 
+constexpr int kRadix = 254;   // R: digits use the full int8 range (measured 100x tighter parity than the power of two 128)
 constexpr int kBM = 128;      // output rows per CTA (UMMA M)
 constexpr int kBK = 64;       // contraction depth per pipeline stage (two UMMA K=32 steps)
 // Output columns per CTA (UMMA N per digit plane).  S group accumulators of bn columns must fit the 512 TMEM columns:
@@ -244,7 +245,7 @@ __device__ __forceinline__ void issue_kblock(uint32_t sa, uint32_t sb, uint32_t 
     }
 }
 
-// CL = thread-block cluster size along the N tiles (1, 2, 3 or 4).  The CL CTAs of a cluster share the M-side operand
+// CL = thread-block cluster size along the N tiles (1, 2 or 3).  The CL CTAs of a cluster share the M-side operand
 // (the X~ planes, in both contractions): each CTA fetches S/CL of its digit planes and TMA
 // multicasts them into every CTA of the cluster, which divides the L2 -> SM traffic of that operand by CL (the kernel
 // ran at the L2 throughput cap without it: 18 GB per launch at config 3).  A stage is released to the producers only
@@ -559,55 +560,6 @@ __global__ void slice_rows_kernel(const double* __restrict__ in, long long ld_in
     for (int j = 0; j < 4; ++j) {
         const int c = c4 + j;
         const double x = (c < cols && !(ZERO_DIAG && c == r)) ? in[r * ld_in + c] : 0.0;
-        split_digits<S>(x, inv, radix, d[j]);
-    }
-#pragma unroll
-    for (int k = 0; k < S; ++k) {
-        char4 v = make_char4(d[0][k], d[1][k], d[2][k], d[3][k]);
-        *reinterpret_cast<char4*>(out + (long long)k * slice_stride + r * ld_out + c4) = v;
-    }
-}
-
-// slice_rows_kernel for grad when its producer (fs::strip_apply_kernel, EPI 1) left per-CTA row maxima and partial dots:
-// the row's exponent comes from the nparts partial maxima, and the first block of each row also publishes the scales and
-// Bj = sum of the partial dots (fixed tree) -- no separate pass over grad for its maximum.
-template <int S>
-__global__ void __launch_bounds__(128) slice_rows_part_kernel(const double* __restrict__ in, long long ld_in, int rows, int cols,
-                                                              const double* __restrict__ pmax, const double* __restrict__ pdot,
-                                                              int nparts, long long ldp, const double* __restrict__ x_scale,
-                                                              double* __restrict__ a_scale, double* __restrict__ c_scale,
-                                                              double* __restrict__ bj, int8_t* __restrict__ out,
-                                                              long long ld_out, long long slice_stride, double radix) {
-    __shared__ double sh[4];
-    const long long r = blockIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double mx = 0.0;
-    for (int p = threadIdx.x; p < nparts; p += 128) mx = fmax(mx, pmax[(long long)p * ldp + r]);
-    mx = lcx::warp_max(mx);
-    if (lane == 0) sh[warp] = mx;
-    __syncthreads();
-    mx = fmax(fmax(sh[0], sh[1]), fmax(sh[2], sh[3]));
-    const double sc = pow2_above(mx);
-    if (blockIdx.y == 0 && warp == 0) {
-        double d = 0.0;
-        if (bj != nullptr) {
-            for (int p = lane; p < nparts; p += 32) d += pdot[(long long)p * ldp + r];
-            d = lcx::warp_sum(d);
-        }
-        if (lane == 0) {
-            a_scale[r] = sc;
-            c_scale[r] = x_scale[0] * sc;
-            if (bj != nullptr) bj[r] = d;
-        }
-    }
-    const int c4 = (blockIdx.y * blockDim.x + threadIdx.x) * 4;
-    if (r >= rows || c4 >= ld_out) return;
-    const double inv = 1.0 / sc;
-    int8_t d[4][S];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int c = c4 + j;
-        const double x = (c < cols) ? in[r * ld_in + c] : 0.0;
         split_digits<S>(x, inv, radix, d[j]);
     }
 #pragma unroll
@@ -967,27 +919,11 @@ inline int make_slice_map(CUtensorMap* map, const void* base, long long inner, l
     cuuint64_t strides[2] = {(cuuint64_t)ld, (cuuint64_t)slice_stride};
     cuuint32_t box[3] = {(cuuint32_t)box_inner, (cuuint32_t)box_rows, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-    if (const char* env = getenv("LCX_OZ_L2PROMO")) {  // experiment knob: 0 none, 64, 128, 256 (default)
-        const int v = atoi(env);
-        promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-              : v == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-    }
     CUresult rc = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, promo,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (rc != CUDA_SUCCESS) return fail(-2, "cuTensorMapEncodeTiled", "encode failed (check alignment / strides)");
     return 0;
-}
-
-// LCX_OZ_PERSISTENT=0 launches one cluster per work unit (the pre-persistent behaviour) for A/B measurements.
-inline bool oz_persistent() {
-    static int v = -1;
-    if (v < 0) {
-        const char* env = getenv("LCX_OZ_PERSISTENT");
-        v = (env && atoi(env) == 0) ? 0 : 1;
-    }
-    return v != 0;
 }
 
 template <int S, bool KMAJOR, int CL, bool CADD = false>
@@ -1036,25 +972,23 @@ inline int launch_oz_gemm_cl(const CUtensorMap& mapA, const CUtensorMap& mapB, G
         }
         resident[dev] = n > 0 ? n : 1;
     }
-    const long long clusters = oz_persistent() ? (units < resident[dev] ? units : resident[dev]) : units;
+    const long long clusters = units < resident[dev] ? units : resident[dev];
     LCX_REQUIRE(clusters * CL < (1LL << 31), "grid too large");
     cfg.gridDim = dim3((unsigned)(clusters * CL));
     LCX_CUDA(cudaLaunchKernelEx(&cfg, kern, mapA, mapB, p));
     return 0;
 }
 
-// cluster = how many N tiles share the M-side operand through TMA multicast (1, 2 or 4; default 2).  A padded cluster
-// slot would occupy an SM for the whole K loop and take a full copy of the X~ tile for nothing, so an odd tile count
-// under pairs runs as pairs plus one final cluster of three (m = 192: 3 tiles in 5.9 ms instead of 7.0 ms).
+// Pairs of N tiles share the M-side operand through TMA multicast (clusters of 1 and of 4 measured slower: multicast does
+// not lower the bytes delivered per SM, and clusters of 4 fit only 132 SMs).  A padded cluster slot would occupy an SM for the whole K loop and take a full copy
+// of the X~ tile for nothing, so an odd tile count runs as pairs plus one final cluster of three (m = 192: 3 tiles in
+// 5.9 ms instead of 7.0 ms), and a single tile as a cluster of one.
 template <int S, bool KMAJOR, bool CADD = false>
-inline int launch_oz_gemm(const CUtensorMap& mapA, const CUtensorMap& mapB, GemmParams p, dim3 grid, cudaStream_t st,
-                          int cluster) {
+inline int launch_oz_gemm(const CUtensorMap& mapA, const CUtensorMap& mapB, GemmParams p, dim3 grid, cudaStream_t st) {
     const int n_tiles = (int)grid.x;
     p.n_tiles = n_tiles;
     p.n_tile0 = 0;
-    if (CADD) cluster = cluster > 2 ? 2 : cluster;  // (the c_add variant is built for clusters of 1, 2 and 3 only)
-    if (!CADD && cluster >= 4 && n_tiles >= 4) return launch_oz_gemm_cl<S, KMAJOR, 4, false>(mapA, mapB, p, grid, st);
-    if (cluster >= 2 && n_tiles >= 2) {
+    if (n_tiles >= 2) {
         if (n_tiles % 2 == 0) return launch_oz_gemm_cl<S, KMAJOR, 2, CADD>(mapA, mapB, p, grid, st);
         if (n_tiles > 3) {
             grid.x = (unsigned)(n_tiles - 3);

@@ -300,16 +300,3 @@ def test_pass_pair_two_level_split(N, n, m, monkeypatch, capfd):
     test_pass_pair_over_tile_edges("fp64_split", 5e-11, N, n, m)
     monkeypatch.setenv("LCX_OZ_TAIL", "0")   # and the uniform plan still works when the tail is switched off
     test_pass_pair_over_tile_edges("fp64_split", 5e-11, N, n, m)
-
-
-@pytest.mark.parametrize("name,algorithm", [("syn_400x300x10_f64", "stream"), ("big5_l0_f64", "stream"),
-                                            ("standard_missing_f64", "gram"), ("syn_4000x2000x20_f64", "gram")])
-def test_fused_mxn_phase_matches_golden(name, algorithm, monkeypatch):
-    """LCX_FUSED=1: the m x n phase of an iteration through csrc/fused_strip_kernels.cuh (the four skinny products inside the
-    elementwise strip kernels, DMMA.8x8x4; opt-in, see host_session.cuh) -- same goldens, same 1e-9, same iteration counts."""
-    from test_gpu_parity import _check_fit, _fit, RTOL
-    monkeypatch.setenv("LCX_FUSED", "1")
-    z, mdl, x = _fit(name, precision="fp64_split", algorithm=algorithm)
-    monkeypatch.delenv("LCX_FUSED")
-    assert mdl.algorithm_used == algorithm
-    _check_fit(z, mdl, x, RTOL)

@@ -1,6 +1,6 @@
 """Device time of the two X contractions (K1: Y = X~ A^T, K2: X~^T Y) for one shape and mode, from the library's own CUDA
-events (lcx_profile_read_phases), on random data drawn on the device.  Experiment knobs are read by the library from the
-environment (LCX_OZ_CLUSTER, LCX_OZ_PERSISTENT, LCX_OZ_DEBUG, LCX_OZ_L2PROMO, LCX_OZ_SPLITS, LCX_OZ_FIXED_KB).
+events (lcx_profile_read_phases), on random data drawn on the device.  The library reads the experiment knob LCX_OZ_DEBUG
+from the environment (it switches the MMAs / the loads off).
 
     python tools/pair_probe.py [N n m [precision [repeats]]]        # one JSON line
 """
