@@ -275,6 +275,32 @@ int lcx_score_rows(lcx_session* s, const void* x, int dtype, long long n_rows, i
 int lcx_precision_rows(lcx_session* s, const double* b, long long ldb, int n_factors, int n_vars, const double* dinv,
                        const double* sd, int row0, int rows, double* out, long long ldc);
 
+/* ---- conditioning on the observed entries (ns variant) -----------------------------------------------------------------
+ * For a row with missing set M and observed set O, in standardised space (x~ = (x - mean) / sd, Lambda = Delta^-1 - B^T B):
+ *   x^_M = E[x~_M | x~_O] = Lambda_MM^-1 B_M^T B x~°  (x~° = x~ with the missing entries zeroed),
+ *   q_O = x~_O^T (Sigma~_OO)^-1 x~_O,   log p(x_O) = log N(x_O; mean_O, Sigma_OO).
+ * Each row solves one SPD system without pivoting, of order |M| (Lambda_MM) or m (E = H + sum_O Delta_i b_i b_i^T, Woodbury),
+ * whichever has the smaller flop estimate (|M|^2 m + |M|^3 / 3 against |O| m^2 + m^3 / 3).
+ * lcx_lowrank_factor_h: lcx_lowrank_factor (same b, dinv, logdet bit for bit) plus h (m x ldh, device) = H = G^-1 G^-T, under
+ *   the same single mailbox read.  ldh even, >= m.  scratch >= lcx_lowrank_h_scratch_doubles(m, n).
+ * lcx_condition_rows: raw fp32 / fp64 rows (ld ldx) as in lcx_score_rows, but a missing entry -- NaN, or the marker when
+ *   has_marker -- is conditioned on instead of imputed by a column mean; no imputation means are needed.  Optional device
+ *   outputs: imputed (n_rows x ldi): observed entries copied as binary64, missing ones mean + sd x^; maha = q_O; logpdf =
+ *   log p(x_O).  A complete row gives lcx_score_rows' maha and logpdf bit for bit; a row with nothing observed gives x^ = 0
+ *   and q = log p = 0.  Every per-row sum runs in an order fixed by n and the row's own mask, so results do not depend on how
+ *   rows are blocked.  class_counts (optional, host, 8 long longs; the call then synchronises the stream): rows with nothing
+ *   to solve, rows whose system has order <= 64, <= 160 (both in shared memory), > 160 (per-CTA global slab), rows on the
+ *   order-|M| path, on the order-m path.  scratch >= lcx_condition_scratch_doubles(n_rows, n_vars, n_factors). */
+long long lcx_lowrank_h_scratch_doubles(int n_factors, int n_vars);
+int lcx_lowrank_factor_h(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
+                         double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* h, long long ldh,
+                         double* scratch, long long scratch_doubles);
+long long lcx_condition_scratch_doubles(long long n_rows, int n_vars, int n_factors);
+int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                       double marker, const double* mean, const double* sd, const double* b, long long ldb, int n_factors,
+                       const double* h, long long ldh, const double* dinv, const double* logdet, double* imputed, long long ldi,
+                       double* maha, double* logpdf, long long* class_counts, double* scratch, long long scratch_doubles);
+
 /* ---- raw FP64 tensor-core GEMM (unit tests / building block) ----------------------------------- */
 /* layout: 0 = A[M][K], B[N][K];  1 = A[K][M], B[K][N];  2 = A[M][K], B[K][N].  C = A*B (+ cadd), optionally
  * stored transposed.  scratch holds split-K partials (may be NULL with max_splits <= 1). */

@@ -85,6 +85,11 @@ SIGNATURES = {
     "lcx_score_scratch_doubles": (_ll, [_ll, _i, _i]),
     "lcx_score_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _p, _ll, _i, _p, _p, _p, _p, _p, _ll]),
     "lcx_precision_rows": (_i, [_p, _p, _ll, _i, _i, _p, _p, _i, _i, _p, _ll]),
+    "lcx_lowrank_h_scratch_doubles": (_ll, [_i, _i]),
+    "lcx_lowrank_factor_h": (_i, [_p, _p, _p, _ll, _i, _i, _d, _p, _p, _ll, _p, _p, _p, _ll, _p, _ll]),
+    "lcx_condition_scratch_doubles": (_ll, [_ll, _i, _i]),
+    "lcx_condition_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _ll, _i, _p, _ll, _p, _p, _p, _ll, _p, _p, _pll,
+                                _p, _ll]),
     "lcx_gemm_f64": (_i, [_p, _i, _i, _i, _i, _p, _ll, _p, _ll, _p, _ll, _i, _p, _i, _p, _ll]),
     "lcx_solve_scratch_doubles": (_ll, [_i]),
     "lcx_solve": (_i, [_p, _p, _ll, _i, _p, _ll, _p, _ll, _i, _p, _ll]),

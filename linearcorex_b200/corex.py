@@ -1077,11 +1077,11 @@ class Corex(object):
         free, _total = torch.cuda.mem_get_info(self._session().device)
         return int(self.stream_rows or 32768) if n_rows * self._session().lib.lcx_ld(n_vars) * 12 > 0.8 * free else 0
 
-    def _row_blocks(self, x, rows, per_block):
+    def _row_blocks(self, x, rows, per_block, impute_pass=True):
         """The row-block loop over new data (transform, scoring): imputation means of the new data from a first pass when a
-        missing marker is set (:389/:404; summed over ranks with `comm`), the stored theta, then
-        per_block(lo, hi, xd, dtype, impute, mean, sd) for every block [lo, hi) of `rows` rows uploaded as device tensor xd.
-        `x` only needs `.shape` and row slicing."""
+        missing marker is set (:389/:404; summed over ranks with `comm`; skipped with impute_pass=False), the stored theta,
+        then per_block(lo, hi, xd, dtype, impute, mean, sd) for every block [lo, hi) of `rows` rows uploaded as device tensor
+        xd.  `x` only needs `.shape` and row slicing."""
         torch = _torch()
         sess = self._session()
         lib = sess.lib
@@ -1093,7 +1093,7 @@ class Corex(object):
         blocks = [(lo, min(N, lo + rows)) for lo in range(0, N, rows)]
         vec = lambda: torch.zeros(n, dtype=torch.float64, device=sess.device)
         impute = None
-        if has_marker:
+        if has_marker and impute_pass:
             nscr = lib.lcx_colstats_scratch_doubles(rows, n)
             scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
             ssum, cnt, t1, t2, impute = vec(), vec(), vec(), vec(), vec()
@@ -1286,11 +1286,11 @@ class Corex(object):
     # ------------------------------------------------------------------------------------------
     # scoring under the covariance estimate (lowrank_kernels.cuh)
     # ------------------------------------------------------------------------------------------
-    def _lowrank_factor(self):
+    def _lowrank_factor(self, with_h=False):
         """Device factor of the ns estimate Sigma = S (Z^T Z + Delta) S (lcx_lowrank_factor): returns (B, ldb, 1/Delta,
-        log det Sigma, theta[1]) as CUDA tensors.  Built from the moments on every call (about one m x m x n product): from
-        the live workspace when the session holds this model's final moments, otherwise uploaded from the host moments (an
-        unpickled model)."""
+        log det Sigma, theta[1]) as CUDA tensors, and with `with_h` also (H, ldh), H = G^-1 G^-T (lcx_lowrank_factor_h).  Built
+        from the moments on every call (about one m x m x n product): from the live workspace when the session holds this
+        model's final moments, otherwise uploaded from the host moments (an unpickled model)."""
         torch = _torch()
         if self.theta is None:
             raise ValueError("scoring needs theta (gaussianize='none' has none, like get_covariance)")
@@ -1313,6 +1313,15 @@ class Corex(object):
         b = torch.zeros((m, ldb), dtype=torch.float64, device=sess.device)
         dinv = torch.empty(n, dtype=torch.float64, device=sess.device)
         logdet = torch.empty(1, dtype=torch.float64, device=sess.device)
+        if with_h:
+            ldh = lib.lcx_ld(m)
+            h = torch.empty((m, ldh), dtype=torch.float64, device=sess.device)
+            nscr = lib.lcx_lowrank_h_scratch_doubles(m, n)
+            scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+            _lib.check(lib.lcx_lowrank_factor_h(sess.h, rinv.data_ptr(), si.data_ptr(), ld, m, n, float(self.eps), sd.data_ptr(),
+                                                b.data_ptr(), ldb, dinv.data_ptr(), logdet.data_ptr(), h.data_ptr(), ldh,
+                                                scratch.data_ptr(), nscr), "lcx_lowrank_factor_h")
+            return b, ldb, dinv, logdet, sd, h, ldh
         nscr = lib.lcx_lowrank_scratch_doubles(m, n)
         scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
         _lib.check(lib.lcx_lowrank_factor(sess.h, rinv.data_ptr(), si.data_ptr(), ld, m, n, float(self.eps), sd.data_ptr(),
@@ -1347,25 +1356,82 @@ class Corex(object):
         self._row_blocks(x, rows, block)
         return maha, logp
 
-    def score_samples(self, x):
+    def _conditioned(self, x, imputed=False, scores=True):
+        """lcx_condition_rows over the rows of x in transform's row blocks, without the column-mean pass: returns
+        (imputed (N, ld) or None, q (N,) or None, log p (N,) or None) as CUDA tensors.  Entries that are NaN, or equal
+        missing_values, are missing.  The per-class row counts of the call are kept in self._condition_counts."""
+        torch = _torch()
+        sess = self._session()
+        lib = sess.lib
+        N, nv = int(np.shape(x)[0]), int(np.shape(x)[1])
+        assert self.nv == nv, "Incorrect number of variables in input, %d instead of %d" % (nv, self.nv)
+        b, ldb, dinv, logdet, _sd, h, ldh = self._lowrank_factor(with_h=True)
+        ld = lib.lcx_ld(nv)
+        out = torch.empty((N, ld), dtype=torch.float64, device=sess.device) if imputed else None
+        maha = torch.empty(N, dtype=torch.float64, device=sess.device) if scores else None
+        logp = torch.empty(N, dtype=torch.float64, device=sess.device) if scores else None
+        self._condition_counts = np.zeros(8, dtype=np.int64)
+        if N == 0:
+            return out, maha, logp
+        rows = min(self._transform_rows_for(x) or N, N)
+        nscr = lib.lcx_condition_scratch_doubles(rows, nv, self.m)
+        scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+        has_marker = self.missing_values is not None
+        marker = float(self.missing_values) if has_marker else 0.0
+        counts = np.zeros(8, dtype=np.int64)
+        p = lambda t, lo: t[lo].data_ptr() if t is not None else None
+
+        def block(lo, hi, xd, dt, _impute, mean, sd):
+            _lib.check(lib.lcx_condition_rows(sess.h, xd.data_ptr(), dt, hi - lo, nv, xd.stride(0), int(has_marker), marker,
+                                              mean.data_ptr(), sd.data_ptr(), b.data_ptr(), ldb, self.m, h.data_ptr(), ldh,
+                                              dinv.data_ptr(), logdet.data_ptr(), p(out, lo), ld, p(maha, lo), p(logp, lo),
+                                              counts.ctypes.data_as(C.POINTER(C.c_longlong)), scratch.data_ptr(), nscr),
+                       "lcx_condition_rows")
+            self._condition_counts += counts
+        self._row_blocks(x, rows, block, impute_pass=False)
+        return out, maha, logp
+
+    def _scores_for(self, x, missing):
+        if missing == 'impute':
+            return self._scores(x)
+        if missing == 'marginalize':
+            return self._conditioned(x)[1:]
+        raise ValueError("missing must be 'impute' or 'marginalize', not %r" % (missing,))
+
+    def impute(self, x, return_device=False):
+        """x with every missing entry (NaN, or equal to missing_values) replaced by its conditional mean given the row's
+        observed entries, E[x_M | x_O] under N(theta[0], get_covariance()): an (N, n) float64 ndarray (an (N, n) CUDA tensor
+        view with `return_device=True`).  Observed entries come back as the binary64 value of the input, bit for bit; a row
+        with nothing observed gets theta[0].  Computed like score_samples(missing='marginalize'): one SPD system per row, of
+        order |M| or m whichever is cheaper, from the low-rank-plus-diagonal structure, never an n x n matrix.  The same preconditions and
+        errors as score_samples."""
+        out = self._conditioned(x, imputed=True, scores=False)[0][:, :self.nv]
+        return out if return_device else out.cpu().numpy()
+
+    def score_samples(self, x, missing='impute'):
         """log p(x_l) under N(theta[0], get_covariance()) for every row, in the units of the input: an (N,) float64 ndarray.
 
         For gaussianize='standard' this is multivariate_normal(theta[0], get_covariance()).logpdf(x).  For 'outliers' it is
         the same Gaussian density of the raw x -- theta and get_covariance() as the model reports them; g() is deliberately
-        not applied, so the density is that of the covariance estimate itself.  Missing entries (missing_values) are imputed
-        with the new data's column means, as transform does.  Computed in binary64 from the low-rank-plus-diagonal structure
-        of the estimate (O(n m) per row, no n x n matrix); results do not depend on how the rows are blocked.  Raises
-        LinAlgError when the estimate is not positive definite (some Delta_i <= 0)."""
-        return self._scores(x)[1].cpu().numpy()
+        not applied, so the density is that of the covariance estimate itself.  Computed in binary64 from the low-rank-plus-
+        diagonal structure of the estimate (O(n m) per row, no n x n matrix); results do not depend on how the rows are
+        blocked.  Raises LinAlgError when the estimate is not positive definite (some Delta_i <= 0).
 
-    def mahalanobis(self, x):
-        """Squared Mahalanobis distances (x_l - theta[0])^T Sigma^-1 (x_l - theta[0]) of the rows: an (N,) float64 ndarray."""
-        return self._scores(x)[0].cpu().numpy()
+        missing='impute' (default): missing entries (missing_values) are imputed with the new data's column means, as
+        transform does, and the row is scored as if complete.  missing='marginalize': the marginal density of the observed
+        entries, log N(x_O; theta[0]_O, Sigma_OO), with NaN entries missing too; a complete row scores exactly as with
+        'impute', a row with nothing observed scores 0."""
+        return self._scores_for(x, missing)[1].cpu().numpy()
 
-    def score(self, x):
-        """Mean log-likelihood of the rows of x (the mean of score_samples).  With `comm` set, x is this rank's row block and
-        the mean is over all ranks' rows; every rank returns the same value."""
-        logp = self._scores(x)[1].cpu().numpy()
+    def mahalanobis(self, x, missing='impute'):
+        """Squared Mahalanobis distances (x_l - theta[0])^T Sigma^-1 (x_l - theta[0]) of the rows: an (N,) float64 ndarray.
+        missing='marginalize' gives the distance of the observed part under Sigma_OO (see score_samples)."""
+        return self._scores_for(x, missing)[0].cpu().numpy()
+
+    def score(self, x, missing='impute'):
+        """Mean log-likelihood of the rows of x (the mean of score_samples(x, missing)).  With `comm` set, x is this rank's row
+        block and the mean is over all ranks' rows; every rank returns the same value."""
+        logp = self._scores_for(x, missing)[1].cpu().numpy()
         red = self._reducer()
         return float(red.sum_scalar(float(np.sum(logp)))) / float(red.sum_scalar(len(logp)))
 

@@ -1041,13 +1041,14 @@ extern "C" int lcx_solve(lcx_session* s, const double* a, long long lda, int m, 
 namespace {
 // scratch of lcx_lowrank_factor: zh | zd (m x ldz each) | K - I (m x ldk) | split-K partials | work of the cooperative factor |
 // lup (m x m) | perm (m ints) | status (2 ints) | per-column log terms (n) | log pivots (m) | mailbox scalars (16)
+// [| G^-1 (m x ldk), lcx_lowrank_factor_h only]
 struct LowrankScratch {
-    double *zh, *zd, *kmat, *part, *work, *lup, *ldiag, *lpiv, *scalars;
+    double *zh, *zd, *kmat, *part, *work, *lup, *ldiag, *lpiv, *scalars, *ginv;
     int *perm, *status;
     long long ldz, ldk, total;
     GemmPlan plan;
 };
-LowrankScratch lowrank_carve(double* base, int m, int n) {
+LowrankScratch lowrank_carve(double* base, int m, int n, bool with_h) {
     LowrankScratch c;
     c.ldz = round_up(n, 16);
     c.ldk = round_up(m, 16);
@@ -1069,6 +1070,7 @@ LowrankScratch lowrank_carve(double* base, int m, int n) {
     c.ldiag = take(n);
     c.lpiv = take(m);
     c.scalars = take(16);
+    c.ginv = with_h ? take((long long)m * c.ldk) : nullptr;
     c.total = cur;
     return c;
 }
@@ -1076,20 +1078,29 @@ LowrankScratch lowrank_carve(double* base, int m, int n) {
 
 extern "C" long long lcx_lowrank_scratch_doubles(int n_factors, int n_vars) {
     if (n_factors <= 0 || n_vars <= 0) return -1;
-    return lowrank_carve(nullptr, n_factors, n_vars).total;
+    return lowrank_carve(nullptr, n_factors, n_vars, false).total;
 }
 
-extern "C" int lcx_lowrank_factor(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
-                                  double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* scratch,
-                                  long long scratch_doubles) {
+extern "C" long long lcx_lowrank_h_scratch_doubles(int n_factors, int n_vars) {
+    if (n_factors <= 0 || n_vars <= 0) return -1;
+    return lowrank_carve(nullptr, n_factors, n_vars, true).total;
+}
+
+// lcx_lowrank_factor, and with h != nullptr also H = G^-1 G^-T (m x ldh) before the one mailbox read
+static int lowrank_factor(lcx_session* s, const char* who, const double* rhoinvrho, const double* si, long long ld, int n_factors,
+                          int n_vars, double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* h,
+                          long long ldh, double* scratch, long long scratch_doubles) {
     LCX_REQUIRE(s && rhoinvrho && si && sd && b && dinv && logdet && scratch, "null argument");
     const int m = n_factors, n = n_vars;
     LCX_REQUIRE(m > 0 && n > 0 && ld >= n && ldb >= n && ldb % 2 == 0, "bad shape (ldb must be even and >= n_vars)");
     LCX_REQUIRE(eps >= 0.0 && eps < 1.0, "eps must lie in [0, 1)");
-    LCX_REQUIRE(scratch_doubles >= lcx_lowrank_scratch_doubles(m, n), "scratch too small (see lcx_lowrank_scratch_doubles)");
+    const bool with_h = h != nullptr;
+    LCX_REQUIRE(scratch_doubles >= lowrank_carve(nullptr, m, n, with_h).total,
+                with_h ? "scratch too small (see lcx_lowrank_h_scratch_doubles)" : "scratch too small (see lcx_lowrank_scratch_doubles)");
     LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    LCX_REQUIRE(!with_h || (ldh >= m && ldh % 2 == 0 && (uintptr_t)h % 16 == 0), "bad h (ldh must be even and >= n_factors)");
     LCX_CUDA(cudaSetDevice(s->device));
-    const LowrankScratch c = lowrank_carve(scratch, m, n);
+    const LowrankScratch c = lowrank_carve(scratch, m, n, with_h);
     LCX_CUDA(cudaMemsetAsync(c.status, 0, 2 * sizeof(int), s->stream));
     lowrank::factor_prep_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(rhoinvrho, si, ld, c.ldz, m, n, 1.0 / sqrt(1.0 - eps * eps), sd,
                                                                      c.zh, c.zd, dinv, c.ldiag, c.status);
@@ -1129,12 +1140,38 @@ extern "C" int lcx_lowrank_factor(lcx_session* s, const double* rhoinvrho, const
     LAUNCHED(s);
     // B = G^-1 (Z Delta^-1) = diag(G)^-1 L^-1 (Z Delta^-1): the details path's triangular sweeps, identity permutation
     LCX_TRY(lu::launch_solve(c.lup, m, c.perm, m, c.zd, c.ldz, b, ldb, n, c.status, nullptr, s->stream, &s->launches));
+    if (with_h) {  // G^-1 = the same sweeps on the identity (held in h until the product overwrites it), H = G^-1 (G^-1)^T
+        lowrank::eye_kernel<<<dim3(cdiv(m, 256), m), 256, 0, s->stream>>>(h, ldh, m);
+        LAUNCHED(s);
+        LCX_TRY(lu::launch_solve(c.lup, m, c.perm, m, h, ldh, c.ginv, c.ldk, m, c.status, nullptr, s->stream, &s->launches));
+        GemmArgs a;
+        memset(&a, 0, sizeof(a));
+        a.A = c.ginv; a.B = c.ginv; a.C = h;
+        a.M = m; a.N = m; a.K = m;
+        a.lda = c.ldk; a.ldb = c.ldk; a.ldc = ldh;
+        LCX_TRY(run_gemm(s, kLayoutKK, plan_gemm(m, m, m, kSMs, 1, false), a, nullptr, (long long)m * ldh));
+    }
     lowrank::logdet_kernel<<<1, 256, 0, s->stream>>>(c.ldiag, n, c.lpiv, m, c.status, logdet, c.scalars);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     LCX_TRY(read_mailbox(s, c.scalars));
-    if (s->mailbox[0] != 0.0) return fail(LCX_ERR_NOT_PD, "lcx_lowrank_factor", "Matrix is not positive definite");
+    if (s->mailbox[0] != 0.0) return fail(LCX_ERR_NOT_PD, who, "Matrix is not positive definite");
     return 0;
+}
+
+extern "C" int lcx_lowrank_factor(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
+                                  double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* scratch,
+                                  long long scratch_doubles) {
+    return lowrank_factor(s, "lcx_lowrank_factor", rhoinvrho, si, ld, n_factors, n_vars, eps, sd, b, ldb, dinv, logdet, nullptr, 0,
+                          scratch, scratch_doubles);
+}
+
+extern "C" int lcx_lowrank_factor_h(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors,
+                                    int n_vars, double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet,
+                                    double* h, long long ldh, double* scratch, long long scratch_doubles) {
+    LCX_REQUIRE(h != nullptr, "null argument");
+    return lowrank_factor(s, "lcx_lowrank_factor_h", rhoinvrho, si, ld, n_factors, n_vars, eps, sd, b, ldb, dinv, logdet, h, ldh,
+                          scratch, scratch_doubles);
 }
 
 extern "C" long long lcx_score_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
@@ -1160,17 +1197,21 @@ extern "C" int lcx_score_rows(lcx_session* s, const void* x, int dtype, long lon
     double* y = ssq + align16(n_rows);
     const int nan_marker = marker != marker;
     if (dtype == LCX_F32 && vec4_ok((const float*)x, ldx))
-        lowrank::score_standardize_kernel<float, true><<<(unsigned)n_rows, 256, 0, s->stream>>>(
-            (const float*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+        lowrank::score_standardize_kernel<float, true, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const float*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq, nullptr, nullptr,
+            nullptr, 0);
     else if (dtype == LCX_F32)
-        lowrank::score_standardize_kernel<float, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
-            (const float*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+        lowrank::score_standardize_kernel<float, false, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const float*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq, nullptr, nullptr,
+            nullptr, 0);
     else if (dtype == LCX_F64 && vec4_ok((const double*)x, ldx))
-        lowrank::score_standardize_kernel<double, true><<<(unsigned)n_rows, 256, 0, s->stream>>>(
-            (const double*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+        lowrank::score_standardize_kernel<double, true, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const double*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq, nullptr, nullptr,
+            nullptr, 0);
     else if (dtype == LCX_F64)
-        lowrank::score_standardize_kernel<double, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
-            (const double*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq);
+        lowrank::score_standardize_kernel<double, false, false><<<(unsigned)n_rows, 256, 0, s->stream>>>(
+            (const double*)x, n_rows, n_vars, ldx, has_marker, marker, nan_marker, impute, mean, sd, dinv, xt, ld, ssq, nullptr, nullptr,
+            nullptr, 0);
     else
         return fail(LCX_ERR_ARG, "lcx_score_rows", "unknown dtype");
     LAUNCHED(s);
@@ -1204,5 +1245,129 @@ extern "C" int lcx_precision_rows(lcx_session* s, const double* b, long long ldb
     lowrank::precision_finish_kernel<<<dim3(cdiv(n_vars, 256), rows), 256, 0, s->stream>>>(out, ldc, row0, rows, n_vars, dinv, sd);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// ---- conditioning on the observed entries (lowrank_kernels.cuh: score_standardize_kernel<MASK>, condition_rows_kernel) ----
+namespace {
+// scratch of lcx_condition_rows: x~° (rows x ld) | s° (rows) | c (rows x ldy) | missing / observed lists (rows x n ints) |
+// missing counts (rows ints) | class counters (kCondCounts) | per-CTA slabs of the global class
+struct ConditionScratch {
+    double *xt, *ssq, *y, *slabs;
+    int *miss, *nmiss;
+    unsigned long long* counts;
+    long long ld, ldy, slab_doubles, total;
+    int pmax, nslabs;
+};
+ConditionScratch condition_carve(double* base, long long rows, int n, int m) {
+    ConditionScratch c;
+    c.ld = round_up(n, 16);
+    c.ldy = round_up(m, 8);
+    c.pmax = 0;
+    for (int k = 1; k < n; ++k) c.pmax = max(c.pmax, lowrank::cond_order(k, n, m));
+    c.slab_doubles = c.nslabs = 0;
+    if (c.pmax > lowrank::kCondSmemMax) {  // at most 2 CTAs per SM, and about 1 GB of slabs
+        c.slab_doubles = align16(lowrank::cond_matrix_doubles(c.pmax));
+        c.nslabs = (int)max(1LL, min(min((long long)2 * kSMs, rows), (1LL << 27) / c.slab_doubles));
+    }
+    long long cur = 0;
+    auto take = [&](long long count) {
+        double* p = base ? base + cur : nullptr;
+        cur = align16(cur + count);
+        return p;
+    };
+    c.xt = take(rows * c.ld);
+    c.ssq = take(rows);
+    c.y = take(rows * c.ldy);
+    c.miss = reinterpret_cast<int*>(take((rows * n + 1) / 2));
+    c.nmiss = reinterpret_cast<int*>(take((rows + 1) / 2));
+    c.counts = reinterpret_cast<unsigned long long*>(take(lowrank::kCondCounts));
+    c.slabs = take((long long)c.nslabs * c.slab_doubles);
+    c.total = cur;
+    return c;
+}
+
+template <bool IN_SMEM>
+int launch_condition(lcx_session* s, const ConditionScratch& c, long long n_rows, int n, int m, const double* b, long long ldb,
+                     const double* h, long long ldh, const double* dinv, const double* mean, const double* sd, const double* logdet,
+                     int pmin, int pmax, double* imputed, long long ldi, double* maha, double* logpdf,
+                     unsigned long long* counts) {
+    static PerDeviceOnce attr = {};
+    const size_t smem = IN_SMEM ? (size_t)lowrank::cond_matrix_doubles(pmax) * sizeof(double) : 0;
+    if (IN_SMEM && attr.first_time())
+        LCX_CUDA(cudaFuncSetAttribute(lowrank::condition_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)(lowrank::cond_matrix_doubles(lowrank::kCondSmemMax) * sizeof(double))));
+    int grid = c.nslabs;
+    if (IN_SMEM) {
+        int per_sm = 0;
+        LCX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lowrank::condition_rows_kernel<true>, lowrank::kCondThreads,
+                                                               smem));
+        grid = (int)min(n_rows, (long long)max(per_sm, 1) * kSMs);
+    }
+    lowrank::condition_rows_kernel<IN_SMEM><<<grid, lowrank::kCondThreads, smem, s->stream>>>(
+        c.miss, c.nmiss, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, log(2.0 * M_PI), c.ssq, c.xt, c.ld, c.y, c.ldy, pmin,
+        pmax, c.slabs, c.slab_doubles, imputed, ldi, maha, logpdf, counts);
+    LAUNCHED(s);
+    return 0;
+}
+}  // namespace
+
+extern "C" long long lcx_condition_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
+    if (n_rows <= 0 || n_vars <= 0 || n_factors <= 0) return -1;
+    return condition_carve(nullptr, n_rows, n_vars, n_factors).total;
+}
+
+extern "C" int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                                  double marker, const double* mean, const double* sd, const double* b, long long ldb, int n_factors,
+                                  const double* h, long long ldh, const double* dinv, const double* logdet, double* imputed,
+                                  long long ldi, double* maha, double* logpdf, long long* class_counts, double* scratch,
+                                  long long scratch_doubles) {
+    LCX_REQUIRE(s && x && mean && sd && b && h && dinv && logdet && scratch, "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && n_vars > 0 && n_factors > 0 && ldx >= n_vars && ldb >= n_vars && ldb % 2 == 0 &&
+                    ldh >= n_factors,
+                "bad shape");
+    LCX_REQUIRE(imputed == nullptr || ldi >= n_vars, "bad shape (ldi must be >= n_vars)");
+    LCX_REQUIRE(scratch_doubles >= lcx_condition_scratch_doubles(n_rows, n_vars, n_factors),
+                "scratch too small (see lcx_condition_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const int n = n_vars, m = n_factors;
+    const ConditionScratch c = condition_carve(scratch, n_rows, n, m);
+    const int nan_marker = marker != marker;
+    LCX_CUDA(cudaMemsetAsync(c.counts, 0, lowrank::kCondCounts * sizeof(unsigned long long), s->stream));
+#define LCX_MASK_LAUNCH(T, V)                                                                                                  \
+    lowrank::score_standardize_kernel<T, V, true><<<(unsigned)n_rows, 256, 0, s->stream>>>(                                    \
+        (const T*)x, n_rows, n, ldx, has_marker, marker, nan_marker, nullptr, mean, sd, dinv, c.xt, c.ld, c.ssq, c.miss, c.nmiss, \
+        imputed, ldi)
+    if (dtype == LCX_F32 && vec4_ok((const float*)x, ldx))
+        LCX_MASK_LAUNCH(float, true);
+    else if (dtype == LCX_F32)
+        LCX_MASK_LAUNCH(float, false);
+    else if (dtype == LCX_F64 && vec4_ok((const double*)x, ldx))
+        LCX_MASK_LAUNCH(double, true);
+    else if (dtype == LCX_F64)
+        LCX_MASK_LAUNCH(double, false);
+    else
+        return fail(LCX_ERR_ARG, "lcx_condition_rows", "unknown dtype");
+#undef LCX_MASK_LAUNCH
+    LAUNCHED(s);
+    // c = X~° B^T: lcx_score_rows' projection, so a complete row gets the same c bit for bit
+    LCX_TRY(lcx_project(s, c.xt, n_rows, n, c.ld, b, ldb, m, c.y, c.ldy, nullptr, nullptr, 0));
+    // size classes by the order p of a row's system: [0, 64] and (64, 160] in shared memory, beyond in the slabs
+    LCX_TRY(launch_condition<true>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, 0, min(c.pmax, lowrank::kCondSmallMax),
+                                   imputed, ldi, maha, logpdf, c.counts));
+    if (c.pmax > lowrank::kCondSmallMax)
+        LCX_TRY(launch_condition<true>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, lowrank::kCondSmallMax + 1,
+                                       min(c.pmax, lowrank::kCondSmemMax), imputed, ldi, maha, logpdf, c.counts));
+    if (c.pmax > lowrank::kCondSmemMax)
+        LCX_TRY(launch_condition<false>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, lowrank::kCondSmemMax + 1, c.pmax,
+                                        imputed, ldi, maha, logpdf, c.counts));
+    LCX_CUDA(cudaGetLastError());
+    if (class_counts) {
+        unsigned long long hc[lowrank::kCondCounts];
+        LCX_CUDA(cudaMemcpyAsync(hc, c.counts, sizeof(hc), cudaMemcpyDeviceToHost, s->stream));
+        LCX_CUDA(cudaStreamSynchronize(s->stream));
+        for (int i = 0; i < lowrank::kCondCounts; ++i) class_counts[i] = (long long)hc[i];
+    }
     return 0;
 }
