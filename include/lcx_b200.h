@@ -300,6 +300,45 @@ int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long long n_row
                        double marker, const double* mean, const double* sd, const double* b, long long ldb, int n_factors,
                        const double* h, long long ldh, const double* dinv, const double* logdet, double* imputed, long long ldi,
                        double* maha, double* logpdf, long long* class_counts, double* scratch, long long scratch_doubles);
+/* lcx_condition_sample_rows: lcx_condition_rows' standardisation, projection and per-row systems (imputed required and
+ *   bit-identical to lcx_condition_rows'; no maha / logpdf), plus, from the same L D L^T factor of each row's system:
+ *   std (optional, n_rows x ldo, device): theta1_i sqrt(var(x_i | x_O)) at the missing entries, exactly 0.0 at observed ones;
+ *     Path A var = diag(Lambda_MM^-1) by forward sweeps on e_a, Path B var_a = Delta_a + Delta_a^2 b_a^T E^-1 b_a.
+ *   draws (optional, device): n_draws completed rows per row, draw d of row r at draws + d draw_stride + r ldo (draw_stride >=
+ *     n_rows ldo): the observed entries as imputed holds them, the missing ones theta0 + theta1 (x^ + v) with v ~ N(0, Lambda_MM^-1):
+ *     Path A v = L^-T D^-1/2 eps, Path B v = Delta_M^1/2 eps1 + Delta_M B_M^T L^-T D^-1/2 eps2, eps from lcx_normal_fill's stream
+ *     (seed, tag 1, row0 + r, d).
+ *   A row with nothing observed solves E = H (order m): std theta1, unconditional draws.  A complete row has std 0 and draws
+ *   equal to the row.  Every per-row sum runs in a fixed order, so results do not depend on the row blocking; row0 is the global
+ *   index of the first row, so a split of the rows between calls or ranks gives the same draws.  class_counts as for
+ *   lcx_condition_rows (rows with nothing observed count as order-m, Path B).
+ *   scratch >= lcx_condition_sample_scratch_doubles(n_rows, n_vars, n_factors). */
+long long lcx_condition_sample_scratch_doubles(long long n_rows, int n_vars, int n_factors);
+int lcx_condition_sample_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                              double marker, const double* mean, const double* sd, const double* b, long long ldb, int n_factors,
+                              const double* h, long long ldh, const double* dinv, double* imputed, long long ldi, double* std_out,
+                              double* draws, long long ldo, long long draw_stride, unsigned long long seed, long long row0,
+                              int n_draws, long long* class_counts, double* scratch, long long scratch_doubles);
+
+/* ---- sampling from the fitted Gaussian (ns variant) ---------------------------------------------------------------------
+ * lcx_normal_fill: out[r][j] (n_rows x ldo, device) = standard normal j of the stream (seed, tag, row0 + r, draw), j < n_cols.
+ *   Philox4x32-10 with counter (j / 2, draw, row mod 2^32, row / 2^32 + 2^24 tag) and key (seed mod 2^32, seed / 2^32); two
+ *   53-bit uniforms in (0, 1], u1 from words 0/1 and u2 from words 2/3, ((w_hi 2^21 + w_lo / 2^11) + 1) 2^-53; Box-Muller
+ *   z_2t = sqrt(-2 ln u1) cospi(2 u2), z_2t+1 = sqrt(-2 ln u1) sinpi(2 u2).  A normal depends on nothing else.  words
+ *   (optional, n_rows x ldw uint32, ldw >= 4 ceil(n_cols / 2)) receives the Philox words of counter t at [4t, 4t + 4).
+ *   Tags: 0 = lcx_sample_rows (columns 0..m-1 are u, m..m+n-1 eps), 1 = lcx_condition_sample_rows.
+ * lcx_sample_rows: rows row0 .. row0 + n_rows - 1 of the stream of draws x = mean + sd (Z^T u + Delta^1/2 eps) from
+ *   N(mean, Sigma), Sigma = S (Z^T Z + Delta) S as for lcx_lowrank_factor (same inputs, same Delta bit for bit), into out
+ *   (n_rows x ldo, device, ldo even).  O(n m) per row: Z and sqrt(Delta) by one column kernel, U (n_rows x m) by
+ *   lcx_normal_fill, Y = U Z on the DMMA engine, and a finish pass that generates eps in registers.  Row r depends only on
+ *   (seed, row0 + r), not on n_rows.  ONE mailbox read returns LCX_ERR_NOT_PD when some Delta_i <= 0.
+ *   scratch >= lcx_sample_scratch_doubles(n_rows, n_vars, n_factors). */
+int lcx_normal_fill(lcx_session* s, unsigned long long seed, int tag, long long row0, long long n_rows, long long draw, int n_cols,
+                    double* out, long long ldo, unsigned int* words, long long ldw);
+long long lcx_sample_scratch_doubles(long long n_rows, int n_vars, int n_factors);
+int lcx_sample_rows(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars, double eps,
+                    const double* mean, const double* sd, unsigned long long seed, long long row0, long long n_rows, double* out,
+                    long long ldo, double* scratch, long long scratch_doubles);
 
 /* ---- raw FP64 tensor-core GEMM (unit tests / building block) ----------------------------------- */
 /* layout: 0 = A[M][K], B[N][K];  1 = A[K][M], B[K][N];  2 = A[M][K], B[K][N].  C = A*B (+ cadd), optionally

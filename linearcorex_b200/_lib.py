@@ -23,7 +23,7 @@ GAUSS = {"standard": 0, "outliers": 1, "none": 2}
 
 ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_longlong, C.c_longlong)
 
-_p, _i, _ll, _d = C.c_void_p, C.c_int, C.c_longlong, C.c_double
+_p, _i, _ll, _d, _ull = C.c_void_p, C.c_int, C.c_longlong, C.c_double, C.c_ulonglong
 _pd = C.POINTER(C.c_double)
 _pll = C.POINTER(C.c_longlong)
 
@@ -90,6 +90,12 @@ SIGNATURES = {
     "lcx_condition_scratch_doubles": (_ll, [_ll, _i, _i]),
     "lcx_condition_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _ll, _i, _p, _ll, _p, _p, _p, _ll, _p, _p, _pll,
                                 _p, _ll]),
+    "lcx_condition_sample_scratch_doubles": (_ll, [_ll, _i, _i]),
+    "lcx_condition_sample_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _ll, _i, _p, _ll, _p, _p, _ll, _p, _p, _ll,
+                                       _ll, _ull, _ll, _i, _pll, _p, _ll]),
+    "lcx_normal_fill": (_i, [_p, _ull, _i, _ll, _ll, _ll, _i, _p, _ll, _p, _ll]),
+    "lcx_sample_scratch_doubles": (_ll, [_ll, _i, _i]),
+    "lcx_sample_rows": (_i, [_p, _p, _p, _ll, _i, _i, _d, _p, _p, _ull, _ll, _ll, _p, _ll, _p, _ll]),
     "lcx_gemm_f64": (_i, [_p, _i, _i, _i, _i, _p, _ll, _p, _ll, _p, _ll, _i, _p, _i, _p, _ll]),
     "lcx_solve_scratch_doubles": (_ll, [_i]),
     "lcx_solve": (_i, [_p, _p, _ll, _i, _p, _ll, _p, _ll, _i, _p, _ll]),

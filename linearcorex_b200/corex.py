@@ -57,8 +57,14 @@ Methods beyond the reference (sklearn's covariance-estimator interface; discoura
   score(x)            their mean (over all ranks' rows with `comm`)
   mahalanobis(x)      squared Mahalanobis distances under the same Gaussian
   get_precision()     the inverse of get_covariance(), in row blocks, with get_covariance's output options
+  impute(x)           conditional means E[x_M | x_O] of the missing entries; return_std=True adds their conditional
+                      standard deviations
+  sample_missing(x)   multiple imputation: draws of the missing entries from their conditional distribution
+  sample(n_samples)   draws from N(theta[0], get_covariance()), reproducible per (seed, row) and splittable by `first_row`
 The estimate is low rank plus diagonal, S (Z^T Z + Delta) S, so none of these forms or factors an n x n matrix: a factor
-B = G^-1 Z Delta^-1 (m x n) is built from the moments on each call and a row costs O(n m), in binary64 on the DMMA engine.
+B = G^-1 Z Delta^-1 (m x n) is built from the moments on each call and a row costs O(n m), in binary64 on the DMMA engine
+(conditioning: one SPD system of order |M| or m per row).  Random draws come from counter-based Philox4x32-10 normals, so
+they do not depend on how rows are blocked.
 Inputs are handled as by transform (containers, row providers, imputation of missing entries with the new data's means).
 """
 import ctypes as C
@@ -1286,11 +1292,10 @@ class Corex(object):
     # ------------------------------------------------------------------------------------------
     # scoring under the covariance estimate (lowrank_kernels.cuh)
     # ------------------------------------------------------------------------------------------
-    def _lowrank_factor(self, with_h=False):
-        """Device factor of the ns estimate Sigma = S (Z^T Z + Delta) S (lcx_lowrank_factor): returns (B, ldb, 1/Delta,
-        log det Sigma, theta[1]) as CUDA tensors, and with `with_h` also (H, ldh), H = G^-1 G^-T (lcx_lowrank_factor_h).  Built
-        from the moments on every call (about one m x m x n product): from the live workspace when the session holds this
-        model's final moments, otherwise uploaded from the host moments (an unpickled model)."""
+    def _lowrank_moments(self):
+        """(rhoinvrho (m x ld), ld, Si, theta[1]) as CUDA tensors for the low-rank-plus-diagonal routines, after their
+        preconditions: from the live workspace when the session holds this model's final moments, otherwise uploaded from the
+        host moments (an unpickled model)."""
         torch = _torch()
         if self.theta is None:
             raise ValueError("scoring needs theta (gaussianize='none' has none, like get_covariance)")
@@ -1309,6 +1314,17 @@ class Corex(object):
             rinv[:, :n].copy_(torch.from_numpy(np.ascontiguousarray(self.moments["rhoinvrho"], dtype=np.float64)))
             si = torch.as_tensor(np.asarray(self.moments["Si"], dtype=np.float64), device=sess.device)
         sd = torch.as_tensor(np.asarray(self.theta[1], dtype=np.float64), device=sess.device)
+        return rinv, ld, si, sd
+
+    def _lowrank_factor(self, with_h=False):
+        """Device factor of the ns estimate Sigma = S (Z^T Z + Delta) S (lcx_lowrank_factor): returns (B, ldb, 1/Delta,
+        log det Sigma, theta[1]) as CUDA tensors, and with `with_h` also (H, ldh), H = G^-1 G^-T (lcx_lowrank_factor_h).  Built
+        from the moments (_lowrank_moments) on every call, about one m x m x n product."""
+        torch = _torch()
+        rinv, ld, si, sd = self._lowrank_moments()
+        sess = self._session()
+        lib = sess.lib
+        n, m = self.nv, self.m
         ldb = lib.lcx_ld(n)
         b = torch.zeros((m, ldb), dtype=torch.float64, device=sess.device)
         dinv = torch.empty(n, dtype=torch.float64, device=sess.device)
@@ -1356,25 +1372,31 @@ class Corex(object):
         self._row_blocks(x, rows, block)
         return maha, logp
 
-    def _conditioned(self, x, imputed=False, scores=True):
+    def _conditioned(self, x, imputed=False, scores=True, std=False, n_draws=0, seed=0, first_row=0):
         """lcx_condition_rows over the rows of x in transform's row blocks, without the column-mean pass: returns
-        (imputed (N, ld) or None, q (N,) or None, log p (N,) or None) as CUDA tensors.  Entries that are NaN, or equal
-        missing_values, are missing.  The per-class row counts of the call are kept in self._condition_counts."""
+        (imputed (N, ld) or None, q (N,) or None, log p (N,) or None, std (N, ld) or None, draws (n_draws, N, ld) or None) as
+        CUDA tensors.  With `std` or `n_draws` the rows go through lcx_condition_sample_rows instead (imputed values, no
+        scores), its draws from the stream of `seed` with x's first row at global index `first_row`.  Entries that are NaN, or
+        equal missing_values, are missing.  The per-class row counts of the call are kept in self._condition_counts."""
         torch = _torch()
         sess = self._session()
         lib = sess.lib
         N, nv = int(np.shape(x)[0]), int(np.shape(x)[1])
         assert self.nv == nv, "Incorrect number of variables in input, %d instead of %d" % (nv, self.nv)
         b, ldb, dinv, logdet, _sd, h, ldh = self._lowrank_factor(with_h=True)
+        sample = bool(std or n_draws)
         ld = lib.lcx_ld(nv)
-        out = torch.empty((N, ld), dtype=torch.float64, device=sess.device) if imputed else None
-        maha = torch.empty(N, dtype=torch.float64, device=sess.device) if scores else None
-        logp = torch.empty(N, dtype=torch.float64, device=sess.device) if scores else None
+        new = lambda *shape: torch.empty(shape, dtype=torch.float64, device=sess.device)
+        out = new(N, ld) if imputed or sample else None
+        maha = new(N) if scores and not sample else None
+        logp = new(N) if scores and not sample else None
+        sdo = new(N, ld) if std else None
+        draws = new(n_draws, N, ld) if n_draws else None
         self._condition_counts = np.zeros(8, dtype=np.int64)
         if N == 0:
-            return out, maha, logp
+            return out, maha, logp, sdo, draws
         rows = min(self._transform_rows_for(x) or N, N)
-        nscr = lib.lcx_condition_scratch_doubles(rows, nv, self.m)
+        nscr = (lib.lcx_condition_sample_scratch_doubles if sample else lib.lcx_condition_scratch_doubles)(rows, nv, self.m)
         scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
         has_marker = self.missing_values is not None
         marker = float(self.missing_values) if has_marker else 0.0
@@ -1382,31 +1404,115 @@ class Corex(object):
         p = lambda t, lo: t[lo].data_ptr() if t is not None else None
 
         def block(lo, hi, xd, dt, _impute, mean, sd):
-            _lib.check(lib.lcx_condition_rows(sess.h, xd.data_ptr(), dt, hi - lo, nv, xd.stride(0), int(has_marker), marker,
-                                              mean.data_ptr(), sd.data_ptr(), b.data_ptr(), ldb, self.m, h.data_ptr(), ldh,
-                                              dinv.data_ptr(), logdet.data_ptr(), p(out, lo), ld, p(maha, lo), p(logp, lo),
-                                              counts.ctypes.data_as(C.POINTER(C.c_longlong)), scratch.data_ptr(), nscr),
-                       "lcx_condition_rows")
+            if sample:
+                _lib.check(lib.lcx_condition_sample_rows(
+                    sess.h, xd.data_ptr(), dt, hi - lo, nv, xd.stride(0), int(has_marker), marker, mean.data_ptr(), sd.data_ptr(),
+                    b.data_ptr(), ldb, self.m, h.data_ptr(), ldh, dinv.data_ptr(), p(out, lo), ld, p(sdo, lo),
+                    draws[0, lo].data_ptr() if draws is not None else None, ld, N * ld, seed, first_row + lo, n_draws,
+                    counts.ctypes.data_as(C.POINTER(C.c_longlong)), scratch.data_ptr(), nscr), "lcx_condition_sample_rows")
+            else:
+                _lib.check(lib.lcx_condition_rows(sess.h, xd.data_ptr(), dt, hi - lo, nv, xd.stride(0), int(has_marker), marker,
+                                                  mean.data_ptr(), sd.data_ptr(), b.data_ptr(), ldb, self.m, h.data_ptr(), ldh,
+                                                  dinv.data_ptr(), logdet.data_ptr(), p(out, lo), ld, p(maha, lo), p(logp, lo),
+                                                  counts.ctypes.data_as(C.POINTER(C.c_longlong)), scratch.data_ptr(), nscr),
+                           "lcx_condition_rows")
             self._condition_counts += counts
         self._row_blocks(x, rows, block, impute_pass=False)
-        return out, maha, logp
+        return out, maha, logp, sdo, draws
 
     def _scores_for(self, x, missing):
         if missing == 'impute':
             return self._scores(x)
         if missing == 'marginalize':
-            return self._conditioned(x)[1:]
+            return self._conditioned(x)[1:3]
         raise ValueError("missing must be 'impute' or 'marginalize', not %r" % (missing,))
 
-    def impute(self, x, return_device=False):
+    def impute(self, x, return_std=False, return_device=False):
         """x with every missing entry (NaN, or equal to missing_values) replaced by its conditional mean given the row's
         observed entries, E[x_M | x_O] under N(theta[0], get_covariance()): an (N, n) float64 ndarray (an (N, n) CUDA tensor
         view with `return_device=True`).  Observed entries come back as the binary64 value of the input, bit for bit; a row
         with nothing observed gets theta[0].  Computed like score_samples(missing='marginalize'): one SPD system per row, of
         order |M| or m whichever is cheaper, from the low-rank-plus-diagonal structure, never an n x n matrix.  The same preconditions and
-        errors as score_samples."""
-        out = self._conditioned(x, imputed=True, scores=False)[0][:, :self.nv]
-        return out if return_device else out.cpu().numpy()
+        errors as score_samples.
+
+        return_std=True returns (imputed, std): std is the conditional standard deviation sqrt(var(x_i | x_O)) of each missing
+        entry, in the units of the input, and exactly 0.0 at observed entries (theta[1] for a row with nothing observed).  It
+        comes from more triangular sweeps on the factor of the same per-row system; `imputed` is the same bit for bit."""
+        res = self._conditioned(x, imputed=True, scores=False, std=return_std)
+        out = res[0][:, :self.nv]
+        if not return_std:
+            return out if return_device else out.cpu().numpy()
+        sd = res[3][:, :self.nv]
+        return (out, sd) if return_device else (out.cpu().numpy(), sd.cpu().numpy())
+
+    def sample_missing(self, x, n_draws=1, seed=None, first_row=0, return_device=False):
+        """Multiple imputation: n_draws completed copies of x, an (n_draws, N, n) float64 ndarray (a CUDA tensor view with
+        `return_device=True`).  Each missing entry set x_M of each row is drawn from its conditional distribution
+        N(E[x_M | x_O], Cov[x_M | x_O]) under N(theta[0], get_covariance()); observed entries are the binary64 of the input, bit
+        for bit.  A row with nothing observed gets unconditional draws, a complete row n_draws copies of itself.  Draw d of
+        row l depends only on (seed, first_row + l, d): `first_row` is the global index of x's first row, so a caller that
+        splits the rows between calls or ranks gets the same draws as one call.  seed=None takes a seed from numpy's global
+        legacy RNG (seeded by Corex(seed=...)).  The same preconditions and errors as impute."""
+        n_draws = int(n_draws)
+        if n_draws < 1:
+            raise ValueError("n_draws must be >= 1")
+        seed = self._sample_seed(seed)
+        first_row = int(first_row)
+        if first_row < 0:
+            raise ValueError("first_row must be >= 0")
+        draws = self._conditioned(x, scores=False, n_draws=n_draws, seed=seed, first_row=first_row)[4][:, :, :self.nv]
+        return draws if return_device else draws.cpu().numpy()
+
+    @staticmethod
+    def _sample_seed(seed):
+        if seed is None:  # numpy's global legacy RNG, like the reference's seeding at :89
+            return int(np.random.randint(np.iinfo(np.int64).max, dtype=np.int64))
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must lie in [0, 2**64)")
+        return seed
+
+    def sample(self, n_samples, seed=None, first_row=0, return_device=False):
+        """Draws from the fitted Gaussian N(theta[0], get_covariance()): rows first_row .. first_row + n_samples - 1 of one
+        stream per (model, seed), an (n_samples, n) float64 ndarray (a CUDA tensor view with `return_device=True`).  Row l
+        depends only on (seed, l), so sample(10, s)[3:] equals sample(7, s, first_row=3) bit for bit: a sample larger than
+        memory, or one piece per rank, comes in pieces.  seed=None takes a seed from numpy's global legacy RNG (seeded by
+        Corex(seed=...)).
+
+        x = theta[0] + theta[1] (Z^T u + Delta^1/2 eps), u ~ N(0, I_m), eps ~ N(0, I_n), from the low-rank-plus-diagonal
+        structure of the estimate: O(n m) per row, no n x n matrix (a dense Cholesky would need n^3 / 3 flops and n^2 doubles).
+        For 'outliers' the draws are of the estimate's Gaussian itself (no g^-1), as score_samples defines its density.  The
+        same preconditions and errors as score_samples; host moments are enough (an unpickled model)."""
+        torch = _torch()
+        n_samples, first_row = int(n_samples), int(first_row)
+        if n_samples < 0 or first_row < 0:
+            raise ValueError("n_samples and first_row must be >= 0")
+        seed = self._sample_seed(seed)
+        rinv, ld, si, sd = self._lowrank_moments()
+        sess = self._session()
+        lib = sess.lib
+        n, m = self.nv, self.m
+        if self._theta_dev is None:
+            self._theta_dev = tuple(torch.as_tensor(np.asarray(t, dtype=np.float64), device=sess.device) for t in self.theta)
+        mean = self._theta_dev[0]
+        ldo = lib.lcx_ld(n)
+        free, _total = torch.cuda.mem_get_info(sess.device)
+        rows = int(self.stream_rows or 32768) if n_samples * ldo * 12 > 0.8 * free else n_samples
+        rows = max(1, min(rows, n_samples))
+        out = torch.empty((n_samples, ldo), dtype=torch.float64, device=sess.device) if return_device else \
+            np.empty((n_samples, n), dtype=np.float64)
+        buf = None if return_device else torch.empty((rows, ldo), dtype=torch.float64, device=sess.device)
+        nscr = lib.lcx_sample_scratch_doubles(rows, n, m)
+        scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+        for lo in range(0, n_samples, rows):
+            hi = min(n_samples, lo + rows)
+            dst = out[lo:hi] if return_device else buf
+            _lib.check(lib.lcx_sample_rows(sess.h, rinv.data_ptr(), si.data_ptr(), ld, m, n, float(self.eps), mean.data_ptr(),
+                                           sd.data_ptr(), seed, first_row + lo, hi - lo, dst.data_ptr(), ldo, scratch.data_ptr(),
+                                           nscr), "lcx_sample_rows")
+            if not return_device:
+                out[lo:hi] = buf[:hi - lo, :n].cpu().numpy()
+        return out[:, :n] if return_device else out
 
     def score_samples(self, x, missing='impute'):
         """log p(x_l) under N(theta[0], get_covariance()) for every row, in the units of the input: an (N,) float64 ndarray.

@@ -1259,12 +1259,12 @@ struct ConditionScratch {
     long long ld, ldy, slab_doubles, total;
     int pmax, nslabs;
 };
-ConditionScratch condition_carve(double* base, long long rows, int n, int m) {
+ConditionScratch condition_carve(double* base, long long rows, int n, int m, bool sample = false) {
     ConditionScratch c;
     c.ld = round_up(n, 16);
     c.ldy = round_up(m, 8);
     c.pmax = 0;
-    for (int k = 1; k < n; ++k) c.pmax = max(c.pmax, lowrank::cond_order(k, n, m));
+    for (int k = 1; k <= n; ++k) c.pmax = max(c.pmax, lowrank::cond_order(k, n, m, sample));
     c.slab_doubles = c.nslabs = 0;
     if (c.pmax > lowrank::kCondSmemMax) {  // at most 2 CTAs per SM, and about 1 GB of slabs
         c.slab_doubles = align16(lowrank::cond_matrix_doubles(c.pmax));
@@ -1287,52 +1287,49 @@ ConditionScratch condition_carve(double* base, long long rows, int n, int m) {
     return c;
 }
 
-template <bool IN_SMEM>
+// the kCondSample outputs of condition_rows_kernel (all zero in kCondMean mode)
+struct CondSampleOut {
+    double *sdo, *draws;
+    long long ldo, draw_stride;
+    unsigned long long seed;
+    long long row0;
+    int n_draws;
+};
+
+template <bool IN_SMEM, int MODE>
 int launch_condition(lcx_session* s, const ConditionScratch& c, long long n_rows, int n, int m, const double* b, long long ldb,
                      const double* h, long long ldh, const double* dinv, const double* mean, const double* sd, const double* logdet,
                      int pmin, int pmax, double* imputed, long long ldi, double* maha, double* logpdf,
-                     unsigned long long* counts) {
+                     unsigned long long* counts, const CondSampleOut& so) {
     static PerDeviceOnce attr = {};
+    auto kern = lowrank::condition_rows_kernel<IN_SMEM, MODE>;
     const size_t smem = IN_SMEM ? (size_t)lowrank::cond_matrix_doubles(pmax) * sizeof(double) : 0;
     if (IN_SMEM && attr.first_time())
-        LCX_CUDA(cudaFuncSetAttribute(lowrank::condition_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        LCX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)(lowrank::cond_matrix_doubles(lowrank::kCondSmemMax) * sizeof(double))));
     int grid = c.nslabs;
     if (IN_SMEM) {
         int per_sm = 0;
-        LCX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lowrank::condition_rows_kernel<true>, lowrank::kCondThreads,
-                                                               smem));
+        LCX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, lowrank::kCondThreads, smem));
         grid = (int)min(n_rows, (long long)max(per_sm, 1) * kSMs);
     }
-    lowrank::condition_rows_kernel<IN_SMEM><<<grid, lowrank::kCondThreads, smem, s->stream>>>(
+    kern<<<grid, lowrank::kCondThreads, smem, s->stream>>>(
         c.miss, c.nmiss, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, log(2.0 * M_PI), c.ssq, c.xt, c.ld, c.y, c.ldy, pmin,
-        pmax, c.slabs, c.slab_doubles, imputed, ldi, maha, logpdf, counts);
+        pmax, c.slabs, c.slab_doubles, imputed, ldi, maha, logpdf, counts, so.sdo, so.draws, so.ldo, so.draw_stride, so.seed, so.row0,
+        so.n_draws);
     LAUNCHED(s);
     return 0;
 }
-}  // namespace
 
-extern "C" long long lcx_condition_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
-    if (n_rows <= 0 || n_vars <= 0 || n_factors <= 0) return -1;
-    return condition_carve(nullptr, n_rows, n_vars, n_factors).total;
-}
-
-extern "C" int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
-                                  double marker, const double* mean, const double* sd, const double* b, long long ldb, int n_factors,
-                                  const double* h, long long ldh, const double* dinv, const double* logdet, double* imputed,
-                                  long long ldi, double* maha, double* logpdf, long long* class_counts, double* scratch,
-                                  long long scratch_doubles) {
-    LCX_REQUIRE(s && x && mean && sd && b && h && dinv && logdet && scratch, "null argument");
-    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && n_vars > 0 && n_factors > 0 && ldx >= n_vars && ldb >= n_vars && ldb % 2 == 0 &&
-                    ldh >= n_factors,
-                "bad shape");
-    LCX_REQUIRE(imputed == nullptr || ldi >= n_vars, "bad shape (ldi must be >= n_vars)");
-    LCX_REQUIRE(scratch_doubles >= lcx_condition_scratch_doubles(n_rows, n_vars, n_factors),
-                "scratch too small (see lcx_condition_scratch_doubles)");
-    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+// the body of lcx_condition_rows / lcx_condition_sample_rows after the argument checks: the masked standardisation, the
+// projection c = X~° B^T and the three size classes
+template <int MODE>
+int condition_rows(lcx_session* s, const char* who, const void* x, int dtype, long long n_rows, int n, long long ldx, int has_marker,
+                   double marker, const double* mean, const double* sd, const double* b, long long ldb, int m, const double* h,
+                   long long ldh, const double* dinv, const double* logdet, double* imputed, long long ldi, double* maha,
+                   double* logpdf, const CondSampleOut& so, long long* class_counts, double* scratch) {
     LCX_CUDA(cudaSetDevice(s->device));
-    const int n = n_vars, m = n_factors;
-    const ConditionScratch c = condition_carve(scratch, n_rows, n, m);
+    const ConditionScratch c = condition_carve(scratch, n_rows, n, m, MODE == lowrank::kCondSample);
     const int nan_marker = marker != marker;
     LCX_CUDA(cudaMemsetAsync(c.counts, 0, lowrank::kCondCounts * sizeof(unsigned long long), s->stream));
 #define LCX_MASK_LAUNCH(T, V)                                                                                                  \
@@ -1348,20 +1345,20 @@ extern "C" int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long
     else if (dtype == LCX_F64)
         LCX_MASK_LAUNCH(double, false);
     else
-        return fail(LCX_ERR_ARG, "lcx_condition_rows", "unknown dtype");
+        return fail(LCX_ERR_ARG, who, "unknown dtype");
 #undef LCX_MASK_LAUNCH
     LAUNCHED(s);
     // c = X~° B^T: lcx_score_rows' projection, so a complete row gets the same c bit for bit
     LCX_TRY(lcx_project(s, c.xt, n_rows, n, c.ld, b, ldb, m, c.y, c.ldy, nullptr, nullptr, 0));
     // size classes by the order p of a row's system: [0, 64] and (64, 160] in shared memory, beyond in the slabs
-    LCX_TRY(launch_condition<true>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, 0, min(c.pmax, lowrank::kCondSmallMax),
-                                   imputed, ldi, maha, logpdf, c.counts));
+    LCX_TRY((launch_condition<true, MODE>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, 0,
+                                          min(c.pmax, lowrank::kCondSmallMax), imputed, ldi, maha, logpdf, c.counts, so)));
     if (c.pmax > lowrank::kCondSmallMax)
-        LCX_TRY(launch_condition<true>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, lowrank::kCondSmallMax + 1,
-                                       min(c.pmax, lowrank::kCondSmemMax), imputed, ldi, maha, logpdf, c.counts));
+        LCX_TRY((launch_condition<true, MODE>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, lowrank::kCondSmallMax + 1,
+                                              min(c.pmax, lowrank::kCondSmemMax), imputed, ldi, maha, logpdf, c.counts, so)));
     if (c.pmax > lowrank::kCondSmemMax)
-        LCX_TRY(launch_condition<false>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, lowrank::kCondSmemMax + 1, c.pmax,
-                                        imputed, ldi, maha, logpdf, c.counts));
+        LCX_TRY((launch_condition<false, MODE>(s, c, n_rows, n, m, b, ldb, h, ldh, dinv, mean, sd, logdet, lowrank::kCondSmemMax + 1,
+                                               c.pmax, imputed, ldi, maha, logpdf, c.counts, so)));
     LCX_CUDA(cudaGetLastError());
     if (class_counts) {
         unsigned long long hc[lowrank::kCondCounts];
@@ -1369,5 +1366,146 @@ extern "C" int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long
         LCX_CUDA(cudaStreamSynchronize(s->stream));
         for (int i = 0; i < lowrank::kCondCounts; ++i) class_counts[i] = (long long)hc[i];
     }
+    return 0;
+}
+}  // namespace
+
+extern "C" long long lcx_condition_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
+    if (n_rows <= 0 || n_vars <= 0 || n_factors <= 0) return -1;
+    return condition_carve(nullptr, n_rows, n_vars, n_factors).total;
+}
+
+extern "C" long long lcx_condition_sample_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
+    if (n_rows <= 0 || n_vars <= 0 || n_factors <= 0) return -1;
+    return condition_carve(nullptr, n_rows, n_vars, n_factors, true).total;
+}
+
+extern "C" int lcx_condition_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                                  double marker, const double* mean, const double* sd, const double* b, long long ldb, int n_factors,
+                                  const double* h, long long ldh, const double* dinv, const double* logdet, double* imputed,
+                                  long long ldi, double* maha, double* logpdf, long long* class_counts, double* scratch,
+                                  long long scratch_doubles) {
+    LCX_REQUIRE(s && x && mean && sd && b && h && dinv && logdet && scratch, "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && n_vars > 0 && n_factors > 0 && ldx >= n_vars && ldb >= n_vars && ldb % 2 == 0 &&
+                    ldh >= n_factors,
+                "bad shape");
+    LCX_REQUIRE(imputed == nullptr || ldi >= n_vars, "bad shape (ldi must be >= n_vars)");
+    LCX_REQUIRE(scratch_doubles >= lcx_condition_scratch_doubles(n_rows, n_vars, n_factors),
+                "scratch too small (see lcx_condition_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    const CondSampleOut none = {};
+    return condition_rows<lowrank::kCondMean>(s, "lcx_condition_rows", x, dtype, n_rows, n_vars, ldx, has_marker, marker, mean, sd, b,
+                                              ldb, n_factors, h, ldh, dinv, logdet, imputed, ldi, maha, logpdf, none, class_counts,
+                                              scratch);
+}
+
+extern "C" int lcx_condition_sample_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                                         int has_marker, double marker, const double* mean, const double* sd, const double* b,
+                                         long long ldb, int n_factors, const double* h, long long ldh, const double* dinv,
+                                         double* imputed, long long ldi, double* std_out, double* draws, long long ldo,
+                                         long long draw_stride, unsigned long long seed, long long row0, int n_draws,
+                                         long long* class_counts, double* scratch, long long scratch_doubles) {
+    LCX_REQUIRE(s && x && mean && sd && b && h && dinv && imputed && scratch, "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && n_vars > 0 && n_factors > 0 && ldx >= n_vars && ldb >= n_vars && ldb % 2 == 0 &&
+                    ldh >= n_factors && ldi >= n_vars,
+                "bad shape");
+    LCX_REQUIRE((std_out == nullptr && draws == nullptr) || ldo >= n_vars, "bad shape (ldo must be >= n_vars)");
+    LCX_REQUIRE(draws == nullptr || (n_draws > 0 && draw_stride >= n_rows * ldo), "bad draws (n_draws > 0, draw_stride >= n_rows ldo)");
+    LCX_REQUIRE(row0 >= 0, "row0 must be >= 0");
+    LCX_REQUIRE(scratch_doubles >= lcx_condition_sample_scratch_doubles(n_rows, n_vars, n_factors),
+                "scratch too small (see lcx_condition_sample_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    if (std_out) LCX_CUDA(cudaMemsetAsync(std_out, 0, (size_t)n_rows * ldo * sizeof(double), s->stream));  // observed entries: 0
+    const CondSampleOut so = {std_out, draws, ldo, draw_stride, seed, row0, draws ? n_draws : 0};
+    return condition_rows<lowrank::kCondSample>(s, "lcx_condition_sample_rows", x, dtype, n_rows, n_vars, ldx, has_marker, marker, mean,
+                                                sd, b, ldb, n_factors, h, ldh, dinv, nullptr, imputed, ldi, nullptr, nullptr, so,
+                                                class_counts, scratch);
+}
+
+// ---- sampling from the fitted Gaussian (lowrank_kernels.cuh: normal_fill_kernel, sample_prep_kernel, sample_finish_kernel) ----
+namespace {
+// scratch of lcx_sample_rows: Z (m x ldz) | sqrt(Delta) (n) | mailbox scalars (16) | U (rows x ldu)
+struct SampleScratch {
+    double *z, *sqd, *scalars, *u;
+    long long ldz, ldu, total;
+};
+SampleScratch sample_carve(double* base, long long rows, int n, int m) {
+    SampleScratch c;
+    c.ldz = round_up(n, 16);
+    c.ldu = round_up(m, 8);
+    long long cur = 0;
+    auto take = [&](long long count) {
+        double* p = base ? base + cur : nullptr;
+        cur = align16(cur + count);
+        return p;
+    };
+    c.z = take((long long)m * c.ldz);
+    c.sqd = take(n);
+    c.scalars = take(16);
+    c.u = take(rows * c.ldu);
+    c.total = cur;
+    return c;
+}
+int normal_fill(lcx_session* s, unsigned long long seed, int tag, long long row0, long long rows, long long draw, int cols,
+                double* out, long long ldo, uint32_t* words, long long ldw) {
+    const long long work = rows * ((cols + 1) / 2);
+    lowrank::normal_fill_kernel<<<(unsigned)min((long long)cdiv(work, 256), (long long)kSMs * 16), 256, 0, s->stream>>>(
+        seed, tag, row0, rows, draw, cols, out, ldo, words, ldw);
+    LAUNCHED(s);
+    return 0;
+}
+}  // namespace
+
+extern "C" int lcx_normal_fill(lcx_session* s, unsigned long long seed, int tag, long long row0, long long n_rows, long long draw,
+                               int n_cols, double* out, long long ldo, unsigned int* words, long long ldw) {
+    LCX_REQUIRE(s && out, "null argument");
+    LCX_REQUIRE(tag >= 0 && tag < 256 && row0 >= 0 && n_rows > 0 && row0 + n_rows <= (1LL << 56) && draw >= 0 && draw < (1LL << 32) &&
+                    n_cols > 0 && ldo >= n_cols && (words == nullptr || ldw >= 4LL * ((n_cols + 1) / 2)),
+                "bad argument");
+    LCX_CUDA(cudaSetDevice(s->device));
+    LCX_TRY(normal_fill(s, seed, tag, row0, n_rows, draw, n_cols, out, ldo, words, ldw));
+    LCX_CUDA(cudaGetLastError());
+    return 0;
+}
+
+extern "C" long long lcx_sample_scratch_doubles(long long n_rows, int n_vars, int n_factors) {
+    if (n_rows <= 0 || n_vars <= 0 || n_factors <= 0) return -1;
+    return sample_carve(nullptr, n_rows, n_vars, n_factors).total;
+}
+
+extern "C" int lcx_sample_rows(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
+                               double eps, const double* mean, const double* sd, unsigned long long seed, long long row0,
+                               long long n_rows, double* out, long long ldo, double* scratch, long long scratch_doubles) {
+    LCX_REQUIRE(s && rhoinvrho && si && mean && sd && out && scratch, "null argument");
+    const int m = n_factors, n = n_vars;
+    LCX_REQUIRE(m > 0 && n > 0 && ld >= n && n_rows > 0 && n_rows < (1LL << 31) && ldo >= n && ldo % 2 == 0, "bad shape (ldo must be even)");
+    LCX_REQUIRE(row0 >= 0 && row0 + n_rows <= (1LL << 56), "bad row0");
+    LCX_REQUIRE(eps >= 0.0 && eps < 1.0, "eps must lie in [0, 1)");
+    LCX_REQUIRE(scratch_doubles >= lcx_sample_scratch_doubles(n_rows, n, m), "scratch too small (see lcx_sample_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)out % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const SampleScratch c = sample_carve(scratch, n_rows, n, m);
+    LCX_CUDA(cudaMemsetAsync(c.scalars, 0, 16 * sizeof(double), s->stream));
+    lowrank::sample_prep_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(rhoinvrho, si, ld, c.ldz, m, n, 1.0 / sqrt(1.0 - eps * eps), c.z,
+                                                                     c.sqd, c.scalars);
+    LAUNCHED(s);
+    LCX_TRY(normal_fill(s, seed, 0, row0, n_rows, 0, m, c.u, c.ldu, nullptr, 0));
+    {   // Y = U Z into out: predict's layout (A row-major rows x m, B factor-major m x n), no split-K, so every entry sums its
+        // m products in the same order whatever the row blocking
+        GemmArgs a;
+        memset(&a, 0, sizeof(a));
+        a.A = c.u; a.B = c.z; a.C = out;
+        a.M = (int)n_rows; a.N = n; a.K = m;
+        a.lda = c.ldu; a.ldb = c.ldz; a.ldc = ldo;
+        LCX_TRY(run_gemm(s, kLayoutKN, plan_gemm((int)n_rows, n, m, kSMs, 1, false), a, nullptr, 0));
+    }
+    const long long work = n_rows * (((long long)(m + n - 1) >> 1) - (m >> 1) + 1);
+    lowrank::sample_finish_kernel<<<(unsigned)min((long long)cdiv(work, 256), (long long)kSMs * 16), 256, 0, s->stream>>>(
+        out, ldo, n_rows, m, n, c.sqd, mean, sd, seed, row0);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
+    LCX_TRY(read_mailbox(s, c.scalars));
+    if (s->mailbox[0] != 0.0) return fail(LCX_ERR_NOT_PD, "lcx_sample_rows", "Matrix is not positive definite");
     return 0;
 }

@@ -20,7 +20,11 @@
 //   precision_finish_kernel    (delta_ik / Delta_i - (B^T B)_ik) / (sd_i sd_k) of one row block
 //   eye_kernel            the identity that lu_solve_kernel turns into G^-1 (H = G^-1 G^-T, the m x m matrix conditioning needs)
 //   condition_rows_kernel conditional mean of the missing entries, q_O and log p(x_O) of a row, one CTA per row: the
-//                         order-p system of Path A or B in shared memory (p <= 160) or in a per-CTA global slab
+//                         order-p system of Path A or B in shared memory (p <= 160) or in a per-CTA global slab; in its
+//                         kCondSample mode also conditional standard deviations and draws from the same factor
+//   normal_fill_kernel    counter-based standard normals (Philox4x32-10 + Box-Muller), the U of sampling
+//   sample_prep_kernel    Z and sqrt(Delta) for sampling, Delta as factor_prep_kernel forms it
+//   sample_finish_kernel  theta0 + theta1 (U Z + sqrt(Delta) eps), eps generated in registers
 #pragma once
 #include "common.cuh"
 #include "lu_solve.cuh"
@@ -29,8 +33,24 @@
 namespace lcx {
 namespace lowrank {
 
-// One thread per variable i; the m factors are summed in index order.  rinv: ld ldr; zh, zd: ld ldz.  status[1] = 1 when some
-// Delta_i <= 0 (Sigma is then not treated as positive definite).
+// Z_ji and Delta_i (the m factors summed in index order) of column i, c = 1 + Si_i: the one definition that scoring,
+// conditioning and sampling share, so that all of them see the same Delta bit for bit.
+__device__ __forceinline__ double lowrank_z(const double* __restrict__ rinv, long long ldr, int j, int i, double c,
+                                            double inv_sqrt_scale) {
+    return rinv[(long long)j * ldr + i] / c * inv_sqrt_scale;
+}
+__device__ __forceinline__ double lowrank_delta(const double* __restrict__ rinv, long long ldr, int m, int i, double c,
+                                                double inv_sqrt_scale) {
+    double acc = 0.0;
+    for (int j = 0; j < m; ++j) {
+        const double z = lowrank_z(rinv, ldr, j, i, c, inv_sqrt_scale);
+        acc += z * z;
+    }
+    return 1.0 - acc;
+}
+
+// One thread per variable i.  rinv: ld ldr; zh, zd: ld ldz.  status[1] = 1 when some Delta_i <= 0 (Sigma is then not treated
+// as positive definite).
 __global__ void factor_prep_kernel(const double* __restrict__ rinv, const double* __restrict__ si, long long ldr, long long ldz,
                                    int m, int n, double inv_sqrt_scale, const double* __restrict__ sd, double* __restrict__ zh,
                                    double* __restrict__ zd, double* __restrict__ dinv, double* __restrict__ ldiag,
@@ -38,20 +58,107 @@ __global__ void factor_prep_kernel(const double* __restrict__ rinv, const double
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const double c = 1.0 + si[i];
-    double acc = 0.0;
-    for (int j = 0; j < m; ++j) {
-        const double z = rinv[(long long)j * ldr + i] / c * inv_sqrt_scale;
-        acc += z * z;
-    }
-    const double delta = 1.0 - acc;
+    const double delta = lowrank_delta(rinv, ldr, m, i, c, inv_sqrt_scale);
     if (!(delta > 0.0)) status[1] = 1;
     const double di = 1.0 / delta, rs = sqrt(di);
     dinv[i] = di;
     ldiag[i] = 2.0 * log(sd[i]) + log(delta);
     for (int j = 0; j < m; ++j) {
-        const double z = rinv[(long long)j * ldr + i] / c * inv_sqrt_scale;
+        const double z = lowrank_z(rinv, ldr, j, i, c, inv_sqrt_scale);
         zh[(long long)j * ldz + i] = z * rs;
         zd[(long long)j * ldz + i] = z * di;
+    }
+}
+
+// ---- counter-based standard normals (Corex.sample, sample_missing) ---------------------------------------------------------
+// Philox4x32-10 (Salmon et al., SC'11; Random123's constants).  Normal j of stream (seed, tag, row, draw) comes from the
+// counter (j / 2, draw, row mod 2^32, row / 2^32 + 2^24 tag) under the key (seed mod 2^32, seed / 2^32): two uniforms in
+// (0, 1] of 53 bits each, u1 from words 0/1 and u2 from words 2/3, then Box-Muller, z_2t = sqrt(-2 ln u1) cospi(2 u2) and
+// z_2t+1 = sqrt(-2 ln u1) sinpi(2 u2).  It depends on nothing else, so results are the same under any grid, row blocking or
+// split of the rows between calls.  Tag 0: sample (columns 0..m-1 are u, m..m+n-1 eps); tag 1: conditional draws.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    return c;
+}
+__device__ __forceinline__ uint4 philox_words(unsigned long long seed, int tag, long long row, long long draw, long long t) {
+    const unsigned long long ur = (unsigned long long)row;
+    return philox4x32_10(make_uint4((uint32_t)t, (uint32_t)draw, (uint32_t)ur, (uint32_t)(ur >> 32) + ((uint32_t)tag << 24)),
+                         (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+__device__ __forceinline__ double uniform53(uint32_t hi, uint32_t lo) {  // (0, 1], exact
+    return (double)((((unsigned long long)hi << 21) | (lo >> 11)) + 1ULL) * 0x1p-53;
+}
+__device__ __forceinline__ double2 normal_pair(unsigned long long seed, int tag, long long row, long long draw, long long t) {
+    const uint4 w = philox_words(seed, tag, row, draw, t);
+    const double r = sqrt(-2.0 * log(uniform53(w.x, w.y)));
+    double s, c;
+    sincospi(2.0 * uniform53(w.z, w.w), &s, &c);
+    return make_double2(r * c, r * s);
+}
+__device__ __forceinline__ double normal_at(unsigned long long seed, int tag, long long row, long long draw, long long j) {
+    const double2 z = normal_pair(seed, tag, row, draw, j >> 1);
+    return (j & 1) ? z.y : z.x;
+}
+
+// out (rows x ldo): out[r][j] = normal j of stream (seed, tag, row0 + r, draw) for j < cols; words (optional, rows x ldw) the
+// four Philox words behind normals 2t and 2t + 1 at words[r][4t .. 4t + 3].  One thread per counter.
+__global__ void __launch_bounds__(256) normal_fill_kernel(unsigned long long seed, int tag, long long row0, long long rows,
+                                                          long long draw, int cols, double* __restrict__ out, long long ldo,
+                                                          uint32_t* __restrict__ words, long long ldw) {
+    const long long pairs = (cols + 1) / 2;
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < rows * pairs; e += (long long)gridDim.x * 256) {
+        const long long r = e / pairs, t = e % pairs;
+        const double2 z = normal_pair(seed, tag, row0 + r, draw, t);
+        out[r * ldo + 2 * t] = z.x;
+        if (2 * t + 1 < cols) out[r * ldo + 2 * t + 1] = z.y;
+        if (words) {
+            const uint4 w = philox_words(seed, tag, row0 + r, draw, t);
+            uint32_t* o = words + r * ldw + 4 * t;
+            o[0] = w.x, o[1] = w.y, o[2] = w.z, o[3] = w.w;
+        }
+    }
+}
+
+// One thread per variable i: Z (m x ldz) and sqrt(Delta) of Sigma~ = Z^T Z + Delta, with factor_prep_kernel's Delta_i.
+// scalars[0] = 1 when some Delta_i <= 0 (the host reads it through the mailbox).
+__global__ void sample_prep_kernel(const double* __restrict__ rinv, const double* __restrict__ si, long long ldr, long long ldz,
+                                   int m, int n, double inv_sqrt_scale, double* __restrict__ z, double* __restrict__ sqd,
+                                   double* __restrict__ scalars) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double c = 1.0 + si[i];
+    const double delta = lowrank_delta(rinv, ldr, m, i, c, inv_sqrt_scale);
+    if (!(delta > 0.0)) scalars[0] = 1.0;
+    sqd[i] = sqrt(delta);
+    for (int j = 0; j < m; ++j) z[(long long)j * ldz + i] = lowrank_z(rinv, ldr, j, i, c, inv_sqrt_scale);
+}
+
+// out (rows x ldo) holds Y = U Z on entry and theta0 + theta1 (Y + sqrt(Delta) eps) on exit, eps_i = normal m + i of stream
+// (seed, 0, row0 + r, 0), generated here and never stored.  One thread per Philox counter (two normals).
+__global__ void __launch_bounds__(256) sample_finish_kernel(double* __restrict__ out, long long ldo, long long rows, int m, int n,
+                                                            const double* __restrict__ sqd, const double* __restrict__ mean,
+                                                            const double* __restrict__ sd, unsigned long long seed,
+                                                            long long row0) {
+    const long long t0 = m >> 1, pairs = ((long long)(m + n - 1) >> 1) - t0 + 1;
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < rows * pairs; e += (long long)gridDim.x * 256) {
+        const long long r = e / pairs, t = t0 + e % pairs;
+        const double2 z = normal_pair(seed, 0, row0 + r, 0, t);
+        const long long i0 = 2 * t - m;
+        if (i0 >= 0) {
+            double* o = out + r * ldo + i0;
+            *o = mean[i0] + sd[i0] * (*o + sqd[i0] * z.x);
+        }
+        if (i0 + 1 < n) {
+            double* o = out + r * ldo + i0 + 1;
+            *o = mean[i0 + 1] + sd[i0 + 1] * (*o + sqd[i0 + 1] * z.y);
+        }
     }
 }
 
@@ -259,20 +366,29 @@ __global__ void eye_kernel(double* __restrict__ out, long long ldo, int m) {
 // Path B (order m):  E = H + sum_O Delta_i b_i b_i^T  (= I - sum_M Delta_i b_i b_i^T, formed from PSD terms only),
 //   Lambda_MM^-1 g = Delta_M g + Delta_M B_M^T E^-1 B_M Delta_M g,  log det Lambda_MM = log det E - sum_M log Delta_i.
 // The path with the smaller cost estimate wins; its order decides the size class (cond_class).
+// kCondSample mode, with W = L D L^T the factor of the row's system (Lambda_MM for Path A, E for Path B):
+//   Path A  var_a = sum_r (L^-1 e_a)_r^2 / d_r                        draw x^ + L^-T D^-1/2 eps
+//   Path B  var_a = Delta_a + Delta_a^2 sum_r (L^-1 b_a)_r^2 / d_r     draw x^ + Delta_M^1/2 eps1 + Delta_M B_M^T L^-T D^-1/2 eps2
+// (Cov of the Path B draw: Delta_M + Delta_M B_M^T E^-1 B_M Delta_M = Lambda_MM^-1.)  A row with nothing observed solves E = H,
+// Path B with O empty: std 1 in standardised units, unconditional draws.  eps: tag-1 normals of stream (row, draw), columns
+// 0..k-1 over the missing columns in ascending order, then (Path B) k..k+m-1 for eps2.
 constexpr int kCondThreads = 256;
 constexpr int kCondChunk = 16;       // gathered vectors staged per pass of the matrix build
 constexpr int kCondSmallMax = 64;    // class 1: the order-p matrix in shared memory, several CTAs per SM
 constexpr int kCondSmemMax = 160;    // class 2: one CTA per SM, p (p|1) + kCondChunk p doubles <= 227 KB
 enum CondCount { kCountTrivial = 0, kCountSmall, kCountSmem, kCountGlobal, kCountPathA, kCountPathB, kCondCounts = 8 };
+enum CondMode { kCondMean = 0, kCondSample = 1 };  // mean (+ q_O, log p); mean + optional std and draws
 
 __host__ __device__ inline bool cond_path_a(long long k, long long n, long long m) {
     const double a = (double)k * k * m + (double)k * k * k / 3.0;
     const double b = (double)(n - k) * m * m + (double)m * m * m / 3.0;
     return a <= b;
 }
-// order of the system a row with k of n entries missing solves (0: nothing to solve)
-__host__ __device__ inline int cond_order(int k, int n, int m) {
-    if (k == 0 || k == n) return 0;
+// order of the system a row with k of n entries missing solves (0: nothing to solve); in kCondSample mode a row with nothing
+// observed solves E = H, of order m
+__host__ __device__ inline int cond_order(int k, int n, int m, bool sample = false) {
+    if (k == 0) return 0;
+    if (k == n) return sample ? m : 0;
     return cond_path_a(k, n, m) ? k : m;
 }
 __host__ __device__ inline int cond_class(int p) {
@@ -305,18 +421,55 @@ __device__ __forceinline__ double cond_ldl_solve(const double* W, int ldw, int p
     return quad;
 }
 
+// V[t] <- L^-1 V[t] for the kCondChunk right-hand sides V[t] = V + t p, L the unit lower factor in W; V[t]_r = 0 for r < c0.
+// The caller synchronises before.
+__device__ __forceinline__ void cond_fwd_chunk(const double* W, int ldw, int p, double* V, int c0) {
+    for (int c = c0; c < p - 1; ++c) {
+        double vc[kCondChunk];
+#pragma unroll
+        for (int t = 0; t < kCondChunk; ++t) vc[t] = V[(long long)t * p + c];
+        for (int r = c + 1 + threadIdx.x; r < p; r += kCondThreads) {
+            const double l = W[(long long)r * ldw + c];
+#pragma unroll
+            for (int t = 0; t < kCondChunk; ++t) V[(long long)t * p + r] -= l * vc[t];
+        }
+        __syncthreads();
+    }
+}
+
+// V[t] <- L^-T V[t] for the kCondChunk right-hand sides.  The caller synchronises before.
+__device__ __forceinline__ void cond_back_chunk(const double* W, int ldw, int p, double* V) {
+    for (int c = p - 1; c > 0; --c) {
+        double vc[kCondChunk];
+#pragma unroll
+        for (int t = 0; t < kCondChunk; ++t) vc[t] = V[(long long)t * p + c];
+        for (int r = threadIdx.x; r < c; r += kCondThreads) {
+            const double l = W[(long long)c * ldw + r];
+#pragma unroll
+            for (int t = 0; t < kCondChunk; ++t) V[(long long)t * p + r] -= l * vc[t];
+        }
+        __syncthreads();
+    }
+}
+
 // One CTA per row of the rows whose order lies in [pmin, pmax] (persistent grid, rows blockIdx.x + t gridDim.x).
 // IN_SMEM: the order-p matrix and the staged vectors in dynamic shared memory; otherwise in this CTA's slab of `slabs`
 // (slab_doubles each).  vec (ld ldv): the row of x~° on entry, g and then x^_M on exit; y (ld ldy): c on entry, Path B's
 // B_M Delta_M g and E^-1 of it on exit.  Outputs optional: xout (ld ldxo) receives mean + sd x^ at the missing columns,
 // maha / logpdf q_O and log p(x_O).  counts (kCondCounts) += rows per class and per path.
-template <bool IN_SMEM>
+// MODE == kCondSample (maha, logpdf and logdet unused; xout required): sdo (optional, ld ldo, zero on entry) receives sd sqrt(var)
+// at the missing columns; draws (optional) n_draws completed rows per row, draw d of row r at draws + d draw_stride + r ldo,
+// drawn from stream (seed, 1, row0 + r, d).
+template <bool IN_SMEM, int MODE = kCondMean>
 __global__ void __launch_bounds__(kCondThreads) condition_rows_kernel(
     const int* __restrict__ miss, const int* __restrict__ nmiss, long long N, int n, int m, const double* __restrict__ b,
     long long ldb, const double* __restrict__ h, long long ldh, const double* __restrict__ dinv, const double* __restrict__ mean,
     const double* __restrict__ sd, const double* __restrict__ logdet, double log_2pi, const double* __restrict__ ssq, double* vec,
     long long ldv, double* y, long long ldy, int pmin, int pmax, double* slabs, long long slab_doubles, double* __restrict__ xout,
-    long long ldxo, double* __restrict__ maha, double* __restrict__ logpdf, unsigned long long* __restrict__ counts) {
+    long long ldxo, double* __restrict__ maha, double* __restrict__ logpdf, unsigned long long* __restrict__ counts,
+    double* __restrict__ sdo, double* __restrict__ draws, long long ldo, long long draw_stride, unsigned long long seed,
+    long long row0, int n_draws) {
+    constexpr bool SAMPLE = MODE == kCondSample;
     extern __shared__ __align__(16) unsigned char cond_smem_raw[];
     __shared__ double red[8];
     __shared__ double wt[kCondChunk];
@@ -325,7 +478,7 @@ __global__ void __launch_bounds__(kCondThreads) condition_rows_kernel(
     double* work = IN_SMEM ? reinterpret_cast<double*>(cond_smem_raw) : slabs + (long long)blockIdx.x * slab_doubles;
     for (long long r = blockIdx.x; r < N; r += gridDim.x) {
         const int k = nmiss[r];
-        const int p = cond_order(k, n, m);
+        const int p = cond_order(k, n, m, SAMPLE);
         if (p < pmin || p > pmax) continue;
         const int* ml = miss + r * n;
         double* g = vec + r * ldv;
@@ -343,13 +496,16 @@ __global__ void __launch_bounds__(kCondThreads) condition_rows_kernel(
         const double c2 = s_c2;
         double q = 0.0, lp = 0.0;
         if (k == 0) {  // complete row: score_finish_kernel's arithmetic
-            q = ssq[r] - c2;
-            lp = -0.5 * (__dmul_rn((double)n, log_2pi) + logdet[0] + q);  // the host's n log 2 pi: no contraction into an fma
-        } else if (k == n) {  // nothing observed: x^ = 0, log p = 0
+            if constexpr (!SAMPLE) {
+                q = ssq[r] - c2;
+                lp = -0.5 * (__dmul_rn((double)n, log_2pi) + logdet[0] + q);  // the host's n log 2 pi: no contraction into an fma
+            }
+        } else if (k == n && !SAMPLE) {  // nothing observed: x^ = 0, log p = 0
             if (xout)
                 for (int i = tid; i < n; i += kCondThreads) xout[r * ldxo + i] = mean[i];
         } else {
-            const bool path_a = p == k;
+            bool path_a = p == k;
+            if constexpr (SAMPLE) path_a = path_a && k < n;  // nothing observed: Path B with O empty, even when m = n
             // g = B_M^T c, and the fixed-order sums of log sd_i and -log Delta_i over M
             double lsd = 0.0, ldel = 0.0;
             for (int a = tid; a < k; a += kCondThreads) {
@@ -449,13 +605,93 @@ __global__ void __launch_bounds__(kCondThreads) condition_rows_kernel(
                 ldet += ldel;
             }
             q = ssq[r] - c2 - gx;
-            lp = -0.5 * (__dmul_rn((double)(n - k), log_2pi) + (logdet[0] - 2.0 * lsd + ldet) + q);
+            if constexpr (!SAMPLE) lp = -0.5 * (__dmul_rn((double)(n - k), log_2pi) + (logdet[0] - 2.0 * lsd + ldet) + q);
             if (xout)
                 for (int a = tid; a < k; a += kCondThreads) {
                     const int i = ml[a];
                     xout[r * ldxo + i] = mean[i] + sd[i] * g[a];
                 }
+            if constexpr (SAMPLE) {
+                double* V = work + (long long)p * ldw;  // the staging area of the build: kCondChunk right-hand sides of length p
+                if (sdo)
+                    for (int a0 = 0; a0 < k; a0 += kCondChunk) {
+                        const int nb = min(kCondChunk, k - a0);
+                        __syncthreads();
+                        for (int e = tid; e < kCondChunk * p; e += kCondThreads) {
+                            double u = 0.0;
+                            if (path_a) {  // e_a
+                                const int t = e / p, rr = e % p;
+                                if (t < nb && rr == a0 + t) u = 1.0;
+                                V[(long long)t * p + rr] = u;
+                            } else {  // b_a: consecutive threads read consecutive missing columns of one factor row
+                                const int t = e % kCondChunk, j = e / kCondChunk;
+                                if (t < nb) u = b[(long long)j * ldb + ml[a0 + t]];
+                                V[(long long)t * p + j] = u;
+                            }
+                        }
+                        __syncthreads();
+                        cond_fwd_chunk(W, ldw, p, V, path_a ? a0 : 0);
+                        for (int t = warp; t < nb; t += kCondThreads / 32) {
+                            double acc = 0.0;
+                            for (int rr = lane; rr < p; rr += 32) {
+                                const double v = V[(long long)t * p + rr];
+                                acc += v * v / W[(long long)rr * ldw + rr];
+                            }
+                            acc = warp_sum(acc);
+                            if (lane == 0) {
+                                const int i = ml[a0 + t];
+                                double var = acc;
+                                if (!path_a) {
+                                    const double dl = 1.0 / dinv[i];
+                                    var = dl + dl * dl * acc;
+                                }
+                                sdo[r * ldo + i] = sd[i] * sqrt(var);
+                            }
+                        }
+                    }
+                if (draws) {
+                    const long long grow = row0 + r;
+                    const int j0 = path_a ? 0 : k;  // eps (Path A) or eps2 (Path B)
+                    for (int d0 = 0; d0 < n_draws; d0 += kCondChunk) {
+                        const int nd = min(kCondChunk, n_draws - d0);
+                        __syncthreads();
+                        for (int e = tid; e < kCondChunk * p; e += kCondThreads) {  // D^-1/2 eps of draw d0 + t
+                            const int t = e / p, rr = e % p;
+                            V[e] = t < nd ? normal_at(seed, 1, grow, d0 + t, j0 + rr) / sqrt(W[(long long)rr * ldw + rr]) : 0.0;
+                        }
+                        __syncthreads();
+                        cond_back_chunk(W, ldw, p, V);
+                        for (int a = tid; a < k; a += kCondThreads) {
+                            const int i = ml[a];
+                            double bv[kCondChunk];  // Path B: (B_M^T L^-T D^-1/2 eps2)_a, factors summed in index order
+#pragma unroll
+                            for (int t = 0; t < kCondChunk; ++t) bv[t] = 0.0;
+                            if (!path_a)
+                                for (int j = 0; j < m; ++j) {
+                                    const double bj = b[(long long)j * ldb + i];
+#pragma unroll
+                                    for (int t = 0; t < kCondChunk; ++t) bv[t] += bj * V[(long long)t * p + j];
+                                }
+                            const double dl = 1.0 / dinv[i];
+#pragma unroll
+                            for (int t = 0; t < kCondChunk; ++t) {
+                                if (t >= nd) break;
+                                const double v = path_a ? V[(long long)t * p + a]
+                                                        : sqrt(dl) * normal_at(seed, 1, grow, d0 + t, a) + dl * bv[t];
+                                draws[(d0 + t) * draw_stride + r * ldo + i] = mean[i] + sd[i] * (g[a] + v);
+                            }
+                        }
+                    }
+                }
+            }
             if (tid == 0 && counts) atomicAdd(counts + (path_a ? kCountPathA : kCountPathB), 1ULL);
+        }
+        if constexpr (SAMPLE) {  // observed entries of every draw: the input's binary64, as xout holds it
+            if (draws && k < n)
+                for (long long e = tid; e < (long long)n_draws * (n - k); e += kCondThreads) {
+                    const int d = (int)(e / (n - k)), i = ml[n - 1 - (int)(e % (n - k))];
+                    draws[d * draw_stride + r * ldo + i] = xout[r * ldxo + i];
+                }
         }
         if (tid == 0) {
             if (maha) maha[r] = q;
