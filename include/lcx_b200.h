@@ -42,6 +42,7 @@ extern "C" {
 #define LCX_ERR_STATE (-3)
 #define LCX_ERR_SINGULAR (-4) /* a pivot of the details-path solve was exactly zero: numpy raises LinAlgError there */
 #define LCX_ERR_NOT_PD (-5)   /* the covariance estimate is not (treated as) positive definite: lcx_lowrank_factor */
+#define LCX_ERR_MISSING (-6)  /* a row has a missing entry (NaN, or the marker) in a column it is conditioned on: lcx_conditional_rows */
 
 /* precision modes */
 #define LCX_PRECISION_FP64 0   /* DMMA (mma.sync m8n8k4 f64) contractions, everything in binary64 */
@@ -326,7 +327,8 @@ int lcx_condition_sample_rows(lcx_session* s, const void* x, int dtype, long lon
  *   53-bit uniforms in (0, 1], u1 from words 0/1 and u2 from words 2/3, ((w_hi 2^21 + w_lo / 2^11) + 1) 2^-53; Box-Muller
  *   z_2t = sqrt(-2 ln u1) cospi(2 u2), z_2t+1 = sqrt(-2 ln u1) sinpi(2 u2).  A normal depends on nothing else.  words
  *   (optional, n_rows x ldw uint32, ldw >= 4 ceil(n_cols / 2)) receives the Philox words of counter t at [4t, 4t + 4).
- *   Tags: 0 = lcx_sample_rows (columns 0..m-1 are u, m..m+n-1 eps), 1 = lcx_condition_sample_rows.
+ *   Tags: 0 = lcx_sample_rows (columns 0..m-1 are u, m..m+n-1 eps), 1 = lcx_condition_sample_rows, 2 =
+ *   lcx_conditional_sample_rows (columns 0..m-1 are u, m..m+n_tgt-1 eps in the order of the targets).
  * lcx_sample_rows: rows row0 .. row0 + n_rows - 1 of the stream of draws x = mean + sd (Z^T u + Delta^1/2 eps) from
  *   N(mean, Sigma), Sigma = S (Z^T Z + Delta) S as for lcx_lowrank_factor (same inputs, same Delta bit for bit), into out
  *   (n_rows x ldo, device, ldo even).  O(n m) per row: Z and sqrt(Delta) by one column kernel, U (n_rows x m) by
@@ -339,6 +341,50 @@ long long lcx_sample_scratch_doubles(long long n_rows, int n_vars, int n_factors
 int lcx_sample_rows(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars, double eps,
                     const double* mean, const double* sd, unsigned long long seed, long long row0, long long n_rows, double* out,
                     long long ldo, double* scratch, long long scratch_doubles);
+
+/* ---- conditioning on a fixed set of observed columns (ns variant) -----------------------------------------------------
+ * Every row observes the same columns O and asks for the same targets T (disjoint; device int arrays observed[n_obs],
+ * targets[n_tgt] of distinct indices in [0, n_vars)).  In standardised space, with Z and Delta as for lcx_lowrank_factor:
+ *   E_O = I + Z_O Delta_O^-1 Z_O^T = L L^T,  A = L^-1 Z_O Delta_O^-1 (m x n_obs),  P = L^-1 Z_T (m x n_tgt),  v = A x~_O,
+ *   E[x~_T | x~_O] = P^T v,  Cov[x~_T | x~_O] = Delta_T + P^T P,  q_O = sum_O x~_i^2 / Delta_i - |v|^2,
+ *   log det Sigma_OO = sum_O (2 log sd_i + log Delta_i) + 2 sum log L_kk,  log p(x_O) = -(n_obs log 2 pi + log det Sigma_OO + q_O) / 2.
+ * The system is the same for every row, so it is factored once; a row then costs two DMMA products of order m (n_obs + n_tgt).
+ * lcx_conditional_factor: the pattern factor, enqueued on the stream, then ONE mailbox read: rhoinvrho, si, ld, eps, mean
+ *   (theta0), sd (theta1) as for lcx_lowrank_factor (same Delta bit for bit) -> a (m x lda), p (m x ldp), ocols (3 rows of n_obs:
+ *   theta0_O, theta1_O, 1/Delta_O), tcols (5 rows of n_tgt: theta0_T, theta1_T, Delta_T, sqrt(Delta_T), theta1_T sqrt(Delta_T +
+ *   |p_t|^2)) and logdet (1 double) = log det Sigma_OO, all device.  E_O - I is the DMMA product with lcx_lowrank_factor's fixed-order
+ *   split-K combine and E_O is factored by its Cholesky kernel.  n_obs = 0 gives A empty, P = Z_T, logdet 0; n_tgt = 0 skips P.
+ *   LCX_ERR_NOT_PD when a selected Delta_i <= 0, LCX_ERR_ARG when an index lies outside [0, n_vars).  lda, ldp even.
+ *   scratch >= lcx_conditional_factor_scratch_doubles(m, n_obs, n_tgt).
+ * lcx_conditional_rows: raw fp32 / fp64 rows of the n_obs observed columns only (ld ldx, in the order of `observed`; x may be
+ *   NULL when n_obs = 0) -> optional device outputs: pred (n_rows x ldpred, ldpred even) = theta0_T + theta1_T E[x~_T | x~_O];
+ *   maha = q_O; logpdf = log p(x_O).  x~_O has lcx_score_rows' arithmetic, V = X~_O A^T is its projection and V P is a DMMA
+ *   product without split-K, so every per-row sum runs in an order fixed by n_obs and m and results do not depend on the row
+ *   blocking.  A missing entry (NaN, or the marker when has_marker) is not conditioned on: after the call's one mailbox read it
+ *   returns LCX_ERR_MISSING.  scratch >= lcx_conditional_scratch_doubles(n_rows, n_obs, n_factors).
+ * lcx_conditional_sample_rows: the same rows -> n_draws draws of x_T per row, draw d of row r at draws + d draw_stride + r ldo
+ *   (ldo, draw_stride even): theta0_T + theta1_T (P^T (v + u) + Delta_T^1/2 eps) with u, eps the normals 0..m-1 and m..m+n_tgt-1
+ *   of lcx_normal_fill's stream (seed, tag 2, row0 + r, d).  Row r depends only on (seed, row0 + r), so a split of the rows
+ *   between calls or ranks gives the same draws.  LCX_ERR_MISSING as for lcx_conditional_rows; same scratch.
+ * lcx_conditional_covariance_rows: rows [row0, row0 + rows) of the n_tgt x n_tgt covariance theta1_T (Delta_T + P^T P) theta1_T
+ *   into out (rows x ldc, device); row0 even, ldc even. */
+long long lcx_conditional_factor_scratch_doubles(int n_factors, int n_obs, int n_tgt);
+int lcx_conditional_factor(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors, int n_vars,
+                           double eps, const double* mean, const double* sd, const int* observed, int n_obs, const int* targets,
+                           int n_tgt, double* a, long long lda, double* p, long long ldp, double* ocols, double* tcols,
+                           double* logdet, double* scratch, long long scratch_doubles);
+long long lcx_conditional_scratch_doubles(long long n_rows, int n_obs, int n_factors);
+int lcx_conditional_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_obs, long long ldx, int has_marker,
+                         double marker, const double* a, long long lda, const double* ocols, const double* p, long long ldp,
+                         int n_tgt, const double* tcols, int n_factors, const double* logdet, double* pred, long long ldpred,
+                         double* maha, double* logpdf, double* scratch, long long scratch_doubles);
+int lcx_conditional_sample_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_obs, long long ldx,
+                                int has_marker, double marker, const double* a, long long lda, const double* ocols, const double* p,
+                                long long ldp, int n_tgt, const double* tcols, int n_factors, double* draws, long long ldo,
+                                long long draw_stride, unsigned long long seed, long long row0, int n_draws, double* scratch,
+                                long long scratch_doubles);
+int lcx_conditional_covariance_rows(lcx_session* s, const double* p, long long ldp, int n_factors, int n_tgt, const double* tcols,
+                                    int row0, int rows, double* out, long long ldc);
 
 /* ---- raw FP64 tensor-core GEMM (unit tests / building block) ----------------------------------- */
 /* layout: 0 = A[M][K], B[N][K];  1 = A[K][M], B[K][N];  2 = A[M][K], B[K][N].  C = A*B (+ cadd), optionally

@@ -9,7 +9,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "liblcx_b200.so")
 
 OK, QUICK_FAIL = 0, 1
-ERR_SINGULAR, ERR_NOT_PD = -4, -5
+ERR_SINGULAR, ERR_NOT_PD, ERR_MISSING = -4, -5, -6
 PRECISION_FP64, PRECISION_FAST, PRECISION_FP64_SPLIT, PRECISION_FP64_SPLIT5, PRECISION_FP64_SPLIT7 = 0, 1, 2, 3, 4
 PRECISIONS = {"fp64": PRECISION_FP64, "fast": PRECISION_FAST, "fp64_split": PRECISION_FP64_SPLIT,
               "fp64_split5": PRECISION_FP64_SPLIT5, "fp64_split7": PRECISION_FP64_SPLIT7}
@@ -96,6 +96,14 @@ SIGNATURES = {
     "lcx_normal_fill": (_i, [_p, _ull, _i, _ll, _ll, _ll, _i, _p, _ll, _p, _ll]),
     "lcx_sample_scratch_doubles": (_ll, [_ll, _i, _i]),
     "lcx_sample_rows": (_i, [_p, _p, _p, _ll, _i, _i, _d, _p, _p, _ull, _ll, _ll, _p, _ll, _p, _ll]),
+    "lcx_conditional_factor_scratch_doubles": (_ll, [_i, _i, _i]),
+    "lcx_conditional_factor": (_i, [_p, _p, _p, _ll, _i, _i, _d, _p, _p, _p, _i, _p, _i, _p, _ll, _p, _ll, _p, _p, _p, _p, _ll]),
+    "lcx_conditional_scratch_doubles": (_ll, [_ll, _i, _i]),
+    "lcx_conditional_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _ll, _p, _p, _ll, _i, _p, _i, _p, _p, _ll, _p, _p, _p,
+                                  _ll]),
+    "lcx_conditional_sample_rows": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _ll, _p, _p, _ll, _i, _p, _i, _p, _ll, _ll, _ull,
+                                         _ll, _i, _p, _ll]),
+    "lcx_conditional_covariance_rows": (_i, [_p, _p, _ll, _i, _i, _p, _i, _i, _p, _ll]),
     "lcx_gemm_f64": (_i, [_p, _i, _i, _i, _i, _p, _ll, _p, _ll, _p, _ll, _i, _p, _i, _p, _ll]),
     "lcx_solve_scratch_doubles": (_ll, [_i]),
     "lcx_solve": (_i, [_p, _p, _ll, _i, _p, _ll, _p, _ll, _i, _p, _ll]),

@@ -61,6 +61,8 @@ Methods beyond the reference (sklearn's covariance-estimator interface; discoura
                       standard deviations
   sample_missing(x)   multiple imputation: draws of the missing entries from their conditional distribution
   sample(n_samples)   draws from N(theta[0], get_covariance()), reproducible per (seed, row) and splittable by `first_row`
+  conditional(obs)    a ConditionalGaussian given a fixed set of observed columns: predict, std, get_covariance, sample and
+                      the marginal score of the observed columns, one factor per pattern and a scoring pass per row
 The estimate is low rank plus diagonal, S (Z^T Z + Delta) S, so none of these forms or factors an n x n matrix: a factor
 B = G^-1 Z Delta^-1 (m x n) is built from the moments on each call and a row costs O(n m), in binary64 on the DMMA engine
 (conditioning: one SPD system of order |M| or m per row).  Random draws come from counter-based Philox4x32-10 normals, so
@@ -1262,17 +1264,17 @@ class Corex(object):
                                                sd.data_ptr(), r0, rows, dst.data_ptr(), ldd), "lcx_covariance_rows")
         return self._n_by_n_rows(fill, block_rows, out, block_callback)
 
-    def _n_by_n_rows(self, fill, block_rows, out, block_callback):
+    def _n_by_n_rows(self, fill, block_rows, out, block_callback, n=None):
         """Output side of get_covariance / get_precision: fill(row0, rows, dst, ld_dst) writes a row block of the n x n matrix
-        into device memory; the blocks go to a new ndarray, to `out` (ndarray / memmap, or a CUDA tensor written in place) or
-        to `block_callback`."""
+        (n = nv unless given) into device memory; the blocks go to a new ndarray, to `out` (ndarray / memmap, or a CUDA tensor
+        written in place) or to `block_callback`."""
         torch = _torch()
         sess = self._session()
-        n = self.nv
+        n = self.nv if n is None else n
         on_device = isinstance(out, torch.Tensor) and out.is_cuda
         if on_device:
             assert tuple(out.shape) == (n, n) and out.dtype == torch.float64 and out.stride(1) == 1 and out.stride(0) % 2 == 0, \
-                "out must be an (n, n) float64 CUDA tensor with unit column stride and an even row stride"
+                "out must be an (%d, %d) float64 CUDA tensor with unit column stride and an even row stride" % (n, n)
         elif out is None and block_callback is None:
             out = np.empty((n, n), dtype=np.float64)
         ldc = sess.lib.lcx_ld(n)
@@ -1552,3 +1554,238 @@ class Corex(object):
             _lib.check(lib.lcx_precision_rows(self._sess.h, b.data_ptr(), ldb, self.m, n, dinv.data_ptr(), sd.data_ptr(), r0,
                                               rows, dst.data_ptr(), ldd), "lcx_precision_rows")
         return self._n_by_n_rows(fill, block_rows, out, block_callback)
+
+    def conditional(self, observed, targets=None):
+        """The fitted Gaussian N(theta[0], get_covariance()) conditioned on a fixed set of observed columns: a
+        ConditionalGaussian that predicts, scores and draws the `targets` (default: every column not in `observed`) for many
+        rows that all observe the columns `observed`, in that order.  Building it factors the order-m system of the pattern
+        once (about m^2 (|O| + |T|) + m^3 / 3 flops); a row then costs O(m (|O| + |T|)), as scoring does.  Indices out of
+        range, duplicated or in both lists raise ValueError; the preconditions and errors are those of score_samples."""
+        return ConditionalGaussian(self, observed, targets)
+
+
+class ConditionalGaussian(object):
+    """N(theta[0], get_covariance()) of a Corex model conditioned on the columns `observed` (Corex.conditional).
+
+    In standardised space x~ = (x - theta[0]) / theta[1], with Sigma~ = Z^T Z + Delta (DESIGN.md section 8) and
+    E_O = I + Z_O Delta_O^-1 Z_O^T = L L^T,  A = L^-1 Z_O Delta_O^-1,  P = L^-1 Z_T,  v = A x~_O:
+        E[x~_T | x~_O] = P^T v,   Cov[x~_T | x~_O] = Delta_T + P^T P   (the same for every row),
+        log p(x_O) = -(|O| log 2 pi + log det Sigma_OO + sum_O x~_i^2 / Delta_i - |v|^2) / 2.
+    The object holds its own device factor (A, P, the gathered theta and Delta, log det Sigma_OO), built once: refitting the
+    parent does not change it, and it pickles with host copies that give the same bits.
+
+    x_obs arguments hold the observed columns only, in the order of `observed`: a float32 / float64 ndarray, a CUDA tensor,
+    or a row provider with `.shape` and row slicing, blocked as transform blocks its input.  A missing entry (NaN, or the
+    parent's missing_values) raises ValueError: rows with their own missing patterns go to Corex.impute."""
+
+    _as_input = Corex._as_input
+    _upload = Corex._upload
+    _n_by_n_rows = Corex._n_by_n_rows
+    _DEVICE = ("_a", "_p", "_ocols", "_tcols", "_logdet")
+
+    def __init__(self, model, observed, targets=None):
+        torch = _torch()
+        n = int(model.nv)
+        observed = self._indices(observed, n, "observed")
+        if targets is None:
+            keep = np.ones(n, dtype=bool)
+            keep[observed] = False
+            targets = np.flatnonzero(keep)
+        else:
+            targets = self._indices(targets, n, "targets")
+            if np.intersect1d(observed, targets).size:
+                raise ValueError("observed and targets must be disjoint")
+        rinv, ld, si, sd = model._lowrank_moments()
+        self.observed, self.targets = observed, targets
+        self.m, self.nv = int(model.m), n
+        self.missing_values = model.missing_values
+        self.input_dtype = model.input_dtype
+        self.stream_rows = model.stream_rows
+        self._comm = model._comm
+        self._device = model._device
+        self._sess = None
+        sess = self._session()
+        lib = sess.lib
+        m, no, nt = self.m, len(observed), len(targets)
+        new = lambda *shape: torch.zeros(shape, dtype=torch.float64, device=sess.device)
+        self._a, self._p = new(m, lib.lcx_ld(no)), new(m, lib.lcx_ld(nt))
+        self._ocols, self._tcols, self._logdet = new(3 * no), new(5 * nt), new(1)
+        mean = torch.as_tensor(np.asarray(model.theta[0], dtype=np.float64), device=sess.device)
+        idx = lambda a: torch.as_tensor(a.astype(np.int32), device=sess.device) if len(a) else None
+        oi, ti = idx(observed), idx(targets)
+        nscr = lib.lcx_conditional_factor_scratch_doubles(m, no, nt)
+        scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+        ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None
+        _lib.check(lib.lcx_conditional_factor(sess.h, rinv.data_ptr(), si.data_ptr(), ld, m, n, float(model.eps), mean.data_ptr(),
+                                              sd.data_ptr(), ptr(oi), no, ptr(ti), nt, ptr(self._a), self._a.shape[1],
+                                              ptr(self._p), self._p.shape[1], ptr(self._ocols), ptr(self._tcols),
+                                              self._logdet.data_ptr(), scratch.data_ptr(), nscr), "lcx_conditional_factor")
+
+    @staticmethod
+    def _indices(v, n, what):
+        a = np.asarray(v)
+        if a.size == 0:
+            return np.zeros(0, dtype=np.int64)
+        if a.ndim != 1 or a.dtype.kind not in "iu":
+            raise ValueError("%s must be a 1-d sequence of column indices" % what)
+        a = a.astype(np.int64)
+        if np.any((a < 0) | (a >= n)):
+            raise ValueError("%s has a column index outside [0, %d)" % (what, n))
+        if np.unique(a).size != a.size:
+            raise ValueError("%s has a duplicate column index" % what)
+        return a
+
+    def __getstate__(self):
+        d = dict(self.__dict__)
+        d["_sess"] = d["_comm"] = None
+        for k in self._DEVICE:
+            d[k] = d[k].cpu().numpy() if not isinstance(d[k], np.ndarray) else d[k]
+        return d
+
+    def _session(self):
+        if self._sess is None:
+            self._sess = _DeviceSession(_lib.PRECISION_FP64, self._device)
+        return self._sess
+
+    def _factor(self):
+        """The device factor (A, P, ocols, tcols, log det), uploaded once after unpickling."""
+        torch = _torch()
+        dev = self._session().device
+        for k in self._DEVICE:
+            v = getattr(self, k)
+            if isinstance(v, np.ndarray):
+                setattr(self, k, torch.as_tensor(v, device=dev))
+        return tuple(getattr(self, k) for k in self._DEVICE)
+
+    def _check(self, rc, what):
+        if rc == _lib.ERR_MISSING:
+            raise ValueError("x_obs has a missing entry (NaN or missing_values) in an observed column; a ConditionalGaussian "
+                             "conditions every row on all of its observed columns -- use Corex.impute for rows with missing "
+                             "entries of their own")
+        return _lib.check(rc, what)
+
+    def _blocks(self, x, n_draws=1):
+        """(N, row-block size) of x_obs after its checks; blocks as transform's (whole arrays when they fit)."""
+        torch = _torch()
+        shape = tuple(np.shape(x))
+        if len(shape) != 2 or shape[1] != len(self.observed):
+            raise ValueError("x_obs must have shape (N, %d): the observed columns, in the order of `observed`"
+                             % len(self.observed))
+        N = int(shape[0])
+        if not isinstance(x, (np.ndarray, torch.Tensor, list, tuple)):
+            return N, int(self.stream_rows or 32768)
+        lib = self._session().lib
+        width = lib.lcx_ld(len(self.observed)) + n_draws * lib.lcx_ld(len(self.targets))
+        free, _total = torch.cuda.mem_get_info(self._session().device)
+        return N, (int(self.stream_rows or 32768) if N * width * 12 > 0.8 * free else max(N, 1))
+
+    def _rows(self, x, per_block, n_draws=1):
+        """per_block(lo, hi, x pointer, dtype, ldx) over the row blocks of x_obs, with the scratch of the block size."""
+        torch = _torch()
+        N, rows = self._blocks(x, n_draws)
+        if N == 0:
+            return N
+        sess = self._session()
+        nscr = sess.lib.lcx_conditional_scratch_doubles(min(rows, N), len(self.observed), self.m)
+        scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
+        for lo in range(0, N, rows):
+            hi = min(N, lo + rows)
+            if len(self.observed):
+                xd = self._as_input(x[lo:hi])
+                per_block(lo, hi, xd.data_ptr(), _lib.F32 if xd.dtype == torch.float32 else _lib.F64, xd.stride(0), scratch)
+            else:
+                per_block(lo, hi, None, _lib.F64, 0, scratch)
+        return N
+
+    def _conditioned(self, x, pred, scores):
+        torch = _torch()
+        sess = self._session()
+        lib = sess.lib
+        a, p, oc, tc, logdet = self._factor()
+        no, nt = len(self.observed), len(self.targets)
+        N = int(np.shape(x)[0]) if len(np.shape(x)) == 2 else 0
+        new = lambda *shape: torch.empty(shape, dtype=torch.float64, device=sess.device)
+        out = new(N, p.shape[1]) if pred else None
+        maha, logp = (new(N), new(N)) if scores else (None, None)
+        has_marker = self.missing_values is not None
+        marker = float(self.missing_values) if has_marker else 0.0
+        at = lambda t, lo: t[lo].data_ptr() if t is not None else None
+
+        def block(lo, hi, xp, dt, ldx, scratch):
+            self._check(lib.lcx_conditional_rows(sess.h, xp, dt, hi - lo, no, ldx, int(has_marker), marker, a.data_ptr(), a.shape[1],
+                                                 oc.data_ptr(), p.data_ptr(), p.shape[1], nt, tc.data_ptr(), self.m,
+                                                 logdet.data_ptr(), at(out, lo) if nt else None, p.shape[1], at(maha, lo),
+                                                 at(logp, lo), scratch.data_ptr(), scratch.numel()), "lcx_conditional_rows")
+        self._rows(x, block)
+        return out, maha, logp
+
+    def predict(self, x_obs, return_device=False):
+        """E[x_T | x_O] in the units of the input: an (N, |T|) float64 ndarray (a CUDA tensor view with return_device=True)."""
+        out = self._conditioned(x_obs, True, False)[0][:, :len(self.targets)]
+        return out if return_device else out.cpu().numpy()
+
+    @property
+    def std(self):
+        """(|T|,) conditional standard deviations theta1_T sqrt(Delta_T + |p_t|^2), the same for every row."""
+        nt = len(self.targets)
+        return self._factor()[3][4 * nt:5 * nt].cpu().numpy()
+
+    def get_covariance(self, block_rows=4096, out=None, block_callback=None):
+        """The |T| x |T| conditional covariance theta1_T (Delta_T + P^T P) theta1_T, in row blocks on the device, with
+        Corex.get_covariance's output options (`out` ndarray / memmap / CUDA tensor, `block_callback`)."""
+        lib = self._session().lib
+        _a, p, _oc, tc, _ld = self._factor()
+        nt = len(self.targets)
+
+        def fill(r0, rows, dst, ldd):
+            _lib.check(lib.lcx_conditional_covariance_rows(self._sess.h, p.data_ptr(), p.shape[1], self.m, nt, tc.data_ptr(), r0,
+                                                           rows, dst.data_ptr(), ldd), "lcx_conditional_covariance_rows")
+        return self._n_by_n_rows(fill, min(block_rows, 65534), out, block_callback, n=nt)
+
+    def sample(self, x_obs, n_draws=1, seed=None, first_row=0, return_device=False):
+        """n_draws draws of x_T from N(E[x_T | x_O], Cov[x_T | x_O]) for every row: an (n_draws, N, |T|) float64 ndarray (a
+        CUDA tensor view with return_device=True).  Draw d of row l depends only on (seed, first_row + l, d), so rows split
+        between calls or ranks get the same draws as one call.  seed=None takes a seed from numpy's global legacy RNG, as
+        Corex.sample does."""
+        torch = _torch()
+        n_draws = int(n_draws)
+        if n_draws < 1:
+            raise ValueError("n_draws must be >= 1")
+        seed = Corex._sample_seed(seed)
+        first_row = int(first_row)
+        if first_row < 0:
+            raise ValueError("first_row must be >= 0")
+        sess = self._session()
+        lib = sess.lib
+        a, p, oc, tc, _logdet = self._factor()
+        no, nt = len(self.observed), len(self.targets)
+        N = int(np.shape(x_obs)[0]) if len(np.shape(x_obs)) == 2 else 0
+        ldo = p.shape[1]
+        draws = torch.empty((n_draws, N, ldo), dtype=torch.float64, device=sess.device)
+        has_marker = self.missing_values is not None
+        marker = float(self.missing_values) if has_marker else 0.0
+
+        def block(lo, hi, xp, dt, ldx, scratch):
+            self._check(lib.lcx_conditional_sample_rows(sess.h, xp, dt, hi - lo, no, ldx, int(has_marker), marker, a.data_ptr(),
+                                                        a.shape[1], oc.data_ptr(), p.data_ptr(), ldo, nt, tc.data_ptr(), self.m,
+                                                        draws[0, lo].data_ptr() if nt else None, ldo, N * ldo, seed,
+                                                        first_row + lo, n_draws, scratch.data_ptr(), scratch.numel()),
+                        "lcx_conditional_sample_rows")
+        self._rows(x_obs, block, n_draws)
+        out = draws[:, :, :nt]
+        return out if return_device else out.cpu().numpy()
+
+    def score_samples(self, x_obs):
+        """log p(x_O) of every row under the marginal N(theta[0]_O, Sigma_OO): an (N,) float64 ndarray (0 when O is empty)."""
+        return self._conditioned(x_obs, False, True)[2].cpu().numpy()
+
+    def mahalanobis(self, x_obs):
+        """Squared Mahalanobis distances of the rows under Sigma_OO: an (N,) float64 ndarray."""
+        return self._conditioned(x_obs, False, True)[1].cpu().numpy()
+
+    def score(self, x_obs):
+        """Mean of score_samples(x_obs); with the parent's `comm`, x_obs is this rank's row block and the mean is over all
+        ranks' rows (every rank returns the same value)."""
+        logp = self.score_samples(x_obs)
+        red = Reducer(self._comm)
+        return float(red.sum_scalar(float(np.sum(logp)))) / float(red.sum_scalar(len(logp)))

@@ -1086,27 +1086,13 @@ extern "C" long long lcx_lowrank_h_scratch_doubles(int n_factors, int n_vars) {
     return lowrank_carve(nullptr, n_factors, n_vars, true).total;
 }
 
-// lcx_lowrank_factor, and with h != nullptr also H = G^-1 G^-T (m x ldh) before the one mailbox read
-static int lowrank_factor(lcx_session* s, const char* who, const double* rhoinvrho, const double* si, long long ld, int n_factors,
-                          int n_vars, double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* h,
-                          long long ldh, double* scratch, long long scratch_doubles) {
-    LCX_REQUIRE(s && rhoinvrho && si && sd && b && dinv && logdet && scratch, "null argument");
-    const int m = n_factors, n = n_vars;
-    LCX_REQUIRE(m > 0 && n > 0 && ld >= n && ldb >= n && ldb % 2 == 0, "bad shape (ldb must be even and >= n_vars)");
-    LCX_REQUIRE(eps >= 0.0 && eps < 1.0, "eps must lie in [0, 1)");
-    const bool with_h = h != nullptr;
-    LCX_REQUIRE(scratch_doubles >= lowrank_carve(nullptr, m, n, with_h).total,
-                with_h ? "scratch too small (see lcx_lowrank_h_scratch_doubles)" : "scratch too small (see lcx_lowrank_scratch_doubles)");
-    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
-    LCX_REQUIRE(!with_h || (ldh >= m && ldh % 2 == 0 && (uintptr_t)h % 16 == 0), "bad h (ldh must be even and >= n_factors)");
-    LCX_CUDA(cudaSetDevice(s->device));
-    const LowrankScratch c = lowrank_carve(scratch, m, n, with_h);
-    LCX_CUDA(cudaMemsetAsync(c.status, 0, 2 * sizeof(int), s->stream));
-    lowrank::factor_prep_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(rhoinvrho, si, ld, c.ldz, m, n, 1.0 / sqrt(1.0 - eps * eps), sd,
-                                                                     c.zh, c.zd, dinv, c.ldiag, c.status);
-    LAUNCHED(s);
-    {   // K - I = (Z Delta^-1/2)(Z Delta^-1/2)^T: both operands K-contiguous, split-K over the variables, fixed-order combine;
-        // the identity is added where the factorisation loads K
+// K - I = (Z Delta^-1/2)(Z Delta^-1/2)^T from the n columns of c.zh (zero when n = 0), then K = G G^T into c.lup / c.lpiv
+// (chol_factor_kernel: one CTA in shared memory for m <= 160, the cooperative grid beyond)
+static int gram_chol(lcx_session* s, const LowrankScratch& c, int m, int n) {
+    if (n == 0) {
+        LCX_CUDA(cudaMemsetAsync(c.kmat, 0, (size_t)m * c.ldk * sizeof(double), s->stream));
+    } else {  // both operands K-contiguous, split-K over the variables, fixed-order combine; the identity is added where the
+              // factorisation loads K
         GemmArgs a;
         memset(&a, 0, sizeof(a));
         a.A = c.zh; a.B = c.zh; a.C = c.kmat;
@@ -1138,6 +1124,29 @@ static int lowrank_factor(lcx_session* s, const char* who, const double* rhoinvr
                                              s->stream));
     }
     LAUNCHED(s);
+    return 0;
+}
+
+// lcx_lowrank_factor, and with h != nullptr also H = G^-1 G^-T (m x ldh) before the one mailbox read
+static int lowrank_factor(lcx_session* s, const char* who, const double* rhoinvrho, const double* si, long long ld, int n_factors,
+                          int n_vars, double eps, const double* sd, double* b, long long ldb, double* dinv, double* logdet, double* h,
+                          long long ldh, double* scratch, long long scratch_doubles) {
+    LCX_REQUIRE(s && rhoinvrho && si && sd && b && dinv && logdet && scratch, "null argument");
+    const int m = n_factors, n = n_vars;
+    LCX_REQUIRE(m > 0 && n > 0 && ld >= n && ldb >= n && ldb % 2 == 0, "bad shape (ldb must be even and >= n_vars)");
+    LCX_REQUIRE(eps >= 0.0 && eps < 1.0, "eps must lie in [0, 1)");
+    const bool with_h = h != nullptr;
+    LCX_REQUIRE(scratch_doubles >= lowrank_carve(nullptr, m, n, with_h).total,
+                with_h ? "scratch too small (see lcx_lowrank_h_scratch_doubles)" : "scratch too small (see lcx_lowrank_scratch_doubles)");
+    LCX_REQUIRE(((uintptr_t)scratch % 16 == 0) && ((uintptr_t)b % 16 == 0), "misaligned device pointer");
+    LCX_REQUIRE(!with_h || (ldh >= m && ldh % 2 == 0 && (uintptr_t)h % 16 == 0), "bad h (ldh must be even and >= n_factors)");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const LowrankScratch c = lowrank_carve(scratch, m, n, with_h);
+    LCX_CUDA(cudaMemsetAsync(c.status, 0, 2 * sizeof(int), s->stream));
+    lowrank::factor_prep_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(rhoinvrho, si, ld, c.ldz, m, n, 1.0 / sqrt(1.0 - eps * eps), sd,
+                                                                     c.zh, c.zd, dinv, c.ldiag, c.status);
+    LAUNCHED(s);
+    LCX_TRY(gram_chol(s, c, m, n));
     // B = G^-1 (Z Delta^-1) = diag(G)^-1 L^-1 (Z Delta^-1): the details path's triangular sweeps, identity permutation
     LCX_TRY(lu::launch_solve(c.lup, m, c.perm, m, c.zd, c.ldz, b, ldb, n, c.status, nullptr, s->stream, &s->launches));
     if (with_h) {  // G^-1 = the same sweeps on the identity (held in h until the product overwrites it), H = G^-1 (G^-1)^T
@@ -1448,10 +1457,10 @@ SampleScratch sample_carve(double* base, long long rows, int n, int m) {
     return c;
 }
 int normal_fill(lcx_session* s, unsigned long long seed, int tag, long long row0, long long rows, long long draw, int cols,
-                double* out, long long ldo, uint32_t* words, long long ldw) {
+                double* out, long long ldo, uint32_t* words, long long ldw, const double* base = nullptr) {
     const long long work = rows * ((cols + 1) / 2);
     lowrank::normal_fill_kernel<<<(unsigned)min((long long)cdiv(work, 256), (long long)kSMs * 16), 256, 0, s->stream>>>(
-        seed, tag, row0, rows, draw, cols, out, ldo, words, ldw);
+        seed, tag, row0, rows, draw, cols, base, out, ldo, words, ldw);
     LAUNCHED(s);
     return 0;
 }
@@ -1502,10 +1511,244 @@ extern "C" int lcx_sample_rows(lcx_session* s, const double* rhoinvrho, const do
     }
     const long long work = n_rows * (((long long)(m + n - 1) >> 1) - (m >> 1) + 1);
     lowrank::sample_finish_kernel<<<(unsigned)min((long long)cdiv(work, 256), (long long)kSMs * 16), 256, 0, s->stream>>>(
-        out, ldo, n_rows, m, n, c.sqd, mean, sd, seed, row0);
+        out, ldo, n_rows, m, n, c.sqd, mean, sd, seed, row0, 0, 0);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     LCX_TRY(read_mailbox(s, c.scalars));
     if (s->mailbox[0] != 0.0) return fail(LCX_ERR_NOT_PD, "lcx_sample_rows", "Matrix is not positive definite");
+    return 0;
+}
+
+// ---- conditioning on a fixed column set (lowrank_kernels.cuh: given_*_kernel and the pieces of lcx_lowrank_factor) -------
+namespace {
+// scratch of lcx_conditional_factor: lcx_lowrank_factor's for the |O| observed columns (zh, zd, K - I, ..., log terms of O) |
+// Z_T (m x ldt)
+struct GivenFactorScratch {
+    LowrankScratch f;
+    double* zt;
+    long long ldt, total;
+};
+GivenFactorScratch given_factor_carve(double* base, int m, int no, int nt) {
+    GivenFactorScratch c;
+    c.f = lowrank_carve(base, m, max(no, 1), false);
+    c.ldt = round_up(max(nt, 1), 16);
+    c.zt = base ? base + c.f.total : nullptr;
+    c.total = c.f.total + align16((long long)m * c.ldt);
+    return c;
+}
+
+// scratch of lcx_conditional_rows / lcx_conditional_sample_rows: x~_O (rows x ldx) | s (rows) | V (rows x ldv) | q, log p when
+// the caller wants neither (rows each) | mailbox scalars (16) | V + U of a draw (rows x ldv)
+struct GivenRowsScratch {
+    double *xt, *ssq, *v, *maha, *logpdf, *scalars, *u;
+    long long ldx, ldv, total;
+};
+GivenRowsScratch given_rows_carve(double* base, long long rows, int no, int m) {
+    GivenRowsScratch c;
+    c.ldx = round_up(max(no, 1), 16);
+    c.ldv = round_up(m, 8);
+    long long cur = 0;
+    auto take = [&](long long count) {
+        double* p = base ? base + cur : nullptr;
+        cur = align16(cur + count);
+        return p;
+    };
+    c.xt = take(rows * c.ldx);
+    c.ssq = take(rows);
+    c.v = take(rows * c.ldv);
+    c.maha = take(rows);
+    c.logpdf = take(rows);
+    c.scalars = take(16);
+    c.u = take(rows * c.ldv);
+    c.total = cur;
+    return c;
+}
+
+// x~_O and s = sum_O x~_i^2 / Delta_i (score_standardize_kernel, FLAG mode: a missing entry raises scalars[0]), then V = X~_O A^T
+// by lcx_score_rows' projection (no split-K: every row's sums run in an order fixed by |O|).  |O| = 0: V = 0, s = 0.
+int given_project(lcx_session* s, const char* who, const GivenRowsScratch& c, const void* x, int dtype, long long n_rows, int no,
+                  long long ldx, int has_marker, double marker, const double* a, long long lda, const double* ocols, int m) {
+    LCX_CUDA(cudaMemsetAsync(c.scalars, 0, 16 * sizeof(double), s->stream));
+    if (no == 0) {
+        LCX_CUDA(cudaMemsetAsync(c.ssq, 0, n_rows * sizeof(double), s->stream));
+        LCX_CUDA(cudaMemsetAsync(c.v, 0, n_rows * c.ldv * sizeof(double), s->stream));
+        return 0;
+    }
+    const int nan_marker = marker != marker;
+#define LCX_FLAG_LAUNCH(T, V)                                                                                                    \
+    lowrank::score_standardize_kernel<T, V, false, true><<<(unsigned)n_rows, 256, 0, s->stream>>>(                               \
+        (const T*)x, n_rows, no, ldx, has_marker, marker, nan_marker, nullptr, ocols, ocols + no, ocols + 2 * no, c.xt, c.ldx, c.ssq, \
+        nullptr, nullptr, c.scalars, 0)
+    if (dtype == LCX_F32 && vec4_ok((const float*)x, ldx))
+        LCX_FLAG_LAUNCH(float, true);
+    else if (dtype == LCX_F32)
+        LCX_FLAG_LAUNCH(float, false);
+    else if (dtype == LCX_F64 && vec4_ok((const double*)x, ldx))
+        LCX_FLAG_LAUNCH(double, true);
+    else if (dtype == LCX_F64)
+        LCX_FLAG_LAUNCH(double, false);
+    else
+        return fail(LCX_ERR_ARG, who, "unknown dtype");
+#undef LCX_FLAG_LAUNCH
+    LAUNCHED(s);
+    return lcx_project(s, c.xt, n_rows, no, c.ldx, a, lda, m, c.v, c.ldv, nullptr, nullptr, 0);
+}
+
+// out (rows x ldo) = left (rows x ldv) P on the DMMA engine: sample's layout, no split-K, so every entry sums its m products in
+// the same order whatever the row blocking
+int given_times_p(lcx_session* s, const double* left, long long ldv, long long rows, const double* p, long long ldp, int m, int nt,
+                  double* out, long long ldo) {
+    GemmArgs g;
+    memset(&g, 0, sizeof(g));
+    g.A = left; g.B = p; g.C = out;
+    g.M = (int)rows; g.N = nt; g.K = m;
+    g.lda = ldv; g.ldb = ldp; g.ldc = ldo;
+    return run_gemm(s, kLayoutKN, plan_gemm((int)rows, nt, m, kSMs, 1, false), g, nullptr, 0);
+}
+
+int given_status(lcx_session* s, const char* who, const GivenRowsScratch& c) {
+    LCX_CUDA(cudaGetLastError());
+    LCX_TRY(read_mailbox(s, c.scalars));
+    if (s->mailbox[0] != 0.0) return fail(LCX_ERR_MISSING, who, "a row has a missing entry in an observed column");
+    return 0;
+}
+}  // namespace
+
+extern "C" long long lcx_conditional_factor_scratch_doubles(int n_factors, int n_obs, int n_tgt) {
+    if (n_factors <= 0 || n_obs < 0 || n_tgt < 0) return -1;
+    return given_factor_carve(nullptr, n_factors, n_obs, n_tgt).total;
+}
+
+extern "C" int lcx_conditional_factor(lcx_session* s, const double* rhoinvrho, const double* si, long long ld, int n_factors,
+                                      int n_vars, double eps, const double* mean, const double* sd, const int* observed, int n_obs,
+                                      const int* targets, int n_tgt, double* a, long long lda, double* p, long long ldp,
+                                      double* ocols, double* tcols, double* logdet, double* scratch, long long scratch_doubles) {
+    LCX_REQUIRE(s && rhoinvrho && si && mean && sd && logdet && scratch, "null argument");
+    LCX_REQUIRE(n_obs == 0 || (observed && a && ocols), "null argument (observed, a, ocols)");
+    LCX_REQUIRE(n_tgt == 0 || (targets && p && tcols), "null argument (targets, p, tcols)");
+    const int m = n_factors, n = n_vars, no = n_obs, nt = n_tgt;
+    LCX_REQUIRE(m > 0 && n > 0 && ld >= n && no >= 0 && nt >= 0 && (long long)no + nt <= n, "bad shape");
+    LCX_REQUIRE(no == 0 || (lda >= no && lda % 2 == 0 && (uintptr_t)a % 16 == 0), "bad a (lda must be even and >= n_obs)");
+    LCX_REQUIRE(nt == 0 || (ldp >= nt && ldp % 2 == 0 && (uintptr_t)p % 16 == 0), "bad p (ldp must be even and >= n_tgt)");
+    LCX_REQUIRE(eps >= 0.0 && eps < 1.0, "eps must lie in [0, 1)");
+    LCX_REQUIRE(scratch_doubles >= lcx_conditional_factor_scratch_doubles(m, no, nt),
+                "scratch too small (see lcx_conditional_factor_scratch_doubles)");
+    LCX_REQUIRE((uintptr_t)scratch % 16 == 0, "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const GivenFactorScratch c = given_factor_carve(scratch, m, no, nt);
+    LCX_CUDA(cudaMemsetAsync(c.f.status, 0, 2 * sizeof(int), s->stream));
+    LCX_CUDA(cudaMemsetAsync(c.f.scalars, 0, 16 * sizeof(double), s->stream));
+    if (no + nt > 0) {
+        lowrank::given_prep_kernel<<<cdiv(no + nt, 256), 256, 0, s->stream>>>(
+            rhoinvrho, si, ld, m, n, 1.0 / sqrt(1.0 - eps * eps), mean, sd, observed, no, targets, nt, c.f.zh, c.f.zd, c.f.ldz, ocols,
+            c.f.ldiag, c.zt, c.ldt, tcols, c.f.status, c.f.scalars);
+        LAUNCHED(s);
+    }
+    // E_O - I and E_O = L L^T exactly as lcx_lowrank_factor forms K on all columns; then A and P by the same sweeps as B
+    LCX_TRY(gram_chol(s, c.f, m, no));
+    if (no > 0) LCX_TRY(lu::launch_solve(c.f.lup, m, c.f.perm, m, c.f.zd, c.f.ldz, a, lda, no, c.f.status, nullptr, s->stream, &s->launches));
+    if (nt > 0) {
+        LCX_TRY(lu::launch_solve(c.f.lup, m, c.f.perm, m, c.zt, c.ldt, p, ldp, nt, c.f.status, nullptr, s->stream, &s->launches));
+        lowrank::given_std_kernel<<<cdiv(nt, 256), 256, 0, s->stream>>>(p, ldp, m, nt, tcols);
+        LAUNCHED(s);
+    }
+    lowrank::logdet_kernel<<<1, 256, 0, s->stream>>>(c.f.ldiag, no, c.f.lpiv, m, c.f.status, logdet, c.f.scalars);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
+    LCX_TRY(read_mailbox(s, c.f.scalars));
+    if (s->mailbox[2] != 0.0) return fail(LCX_ERR_ARG, "lcx_conditional_factor", "column index out of range");
+    if (s->mailbox[0] != 0.0) return fail(LCX_ERR_NOT_PD, "lcx_conditional_factor", "Matrix is not positive definite");
+    return 0;
+}
+
+extern "C" long long lcx_conditional_scratch_doubles(long long n_rows, int n_obs, int n_factors) {
+    if (n_rows <= 0 || n_obs < 0 || n_factors <= 0) return -1;
+    return given_rows_carve(nullptr, n_rows, n_obs, n_factors).total;
+}
+
+extern "C" int lcx_conditional_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_obs, long long ldx, int has_marker,
+                                    double marker, const double* a, long long lda, const double* ocols, const double* p, long long ldp,
+                                    int n_tgt, const double* tcols, int n_factors, const double* logdet, double* pred, long long ldpred,
+                                    double* maha, double* logpdf, double* scratch, long long scratch_doubles) {
+    const int m = n_factors, no = n_obs, nt = n_tgt;
+    LCX_REQUIRE(s && logdet && scratch && (no == 0 || (x && a && ocols)) && (nt == 0 || (p && tcols)), "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && no >= 0 && nt >= 0 && m > 0 && ldx >= no && (no == 0 || lda >= no) &&
+                    (nt == 0 || ldp >= nt),
+                "bad shape");
+    LCX_REQUIRE(pred == nullptr || nt == 0 || (ldpred >= nt && ldpred % 2 == 0 && (uintptr_t)pred % 16 == 0),
+                "bad pred (ldpred must be even and >= n_tgt)");
+    LCX_REQUIRE(scratch_doubles >= lcx_conditional_scratch_doubles(n_rows, no, m), "scratch too small (see lcx_conditional_scratch_doubles)");
+    LCX_REQUIRE((uintptr_t)scratch % 16 == 0 && (no == 0 || (uintptr_t)a % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const GivenRowsScratch c = given_rows_carve(scratch, n_rows, no, m);
+    LCX_TRY(given_project(s, "lcx_conditional_rows", c, x, dtype, n_rows, no, ldx, has_marker, marker, a, lda, ocols, m));
+    if (pred && nt > 0) {
+        LCX_TRY(given_times_p(s, c.v, c.ldv, n_rows, p, ldp, m, nt, pred, ldpred));
+        const long long work = n_rows * nt;
+        lowrank::given_mean_finish_kernel<<<(unsigned)min((long long)cdiv(work, 256), (long long)kSMs * 16), 256, 0, s->stream>>>(
+            pred, ldpred, n_rows, nt, tcols);
+        LAUNCHED(s);
+    }
+    if (maha || logpdf) {  // q = s - |V_r|^2 and log p with |O| and log det Sigma_OO: score_finish_kernel's arithmetic
+        lowrank::score_finish_kernel<<<cdiv(n_rows, 8), 256, 0, s->stream>>>(c.v, c.ldv, c.ssq, n_rows, m, logdet,
+                                                                             (double)no * log(2.0 * M_PI), maha ? maha : c.maha,
+                                                                             logpdf ? logpdf : c.logpdf);
+        LAUNCHED(s);
+    }
+    return given_status(s, "lcx_conditional_rows", c);
+}
+
+extern "C" int lcx_conditional_sample_rows(lcx_session* s, const void* x, int dtype, long long n_rows, int n_obs, long long ldx,
+                                           int has_marker, double marker, const double* a, long long lda, const double* ocols,
+                                           const double* p, long long ldp, int n_tgt, const double* tcols, int n_factors,
+                                           double* draws, long long ldo, long long draw_stride, unsigned long long seed,
+                                           long long row0, int n_draws, double* scratch, long long scratch_doubles) {
+    const int m = n_factors, no = n_obs, nt = n_tgt;
+    LCX_REQUIRE(s && scratch && (no == 0 || (x && a && ocols)) && (nt == 0 || (p && tcols && draws)), "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && no >= 0 && nt >= 0 && m > 0 && ldx >= no && (no == 0 || lda >= no) &&
+                    (nt == 0 || ldp >= nt),
+                "bad shape");
+    LCX_REQUIRE(nt == 0 || (ldo >= nt && ldo % 2 == 0 && (uintptr_t)draws % 16 == 0), "bad draws (ldo must be even and >= n_tgt)");
+    LCX_REQUIRE(n_draws > 0 && (nt == 0 || n_draws == 1 || (draw_stride >= n_rows * ldo && draw_stride % 2 == 0)),
+                "bad draws (n_draws > 0, draw_stride even and >= n_rows ldo)");
+    LCX_REQUIRE(row0 >= 0 && row0 + n_rows <= (1LL << 56), "bad row0");
+    LCX_REQUIRE(scratch_doubles >= lcx_conditional_scratch_doubles(n_rows, no, m), "scratch too small (see lcx_conditional_scratch_doubles)");
+    LCX_REQUIRE((uintptr_t)scratch % 16 == 0 && (no == 0 || (uintptr_t)a % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    const GivenRowsScratch c = given_rows_carve(scratch, n_rows, no, m);
+    LCX_TRY(given_project(s, "lcx_conditional_sample_rows", c, x, dtype, n_rows, no, ldx, has_marker, marker, a, lda, ocols, m));
+    if (nt > 0)
+        for (int d = 0; d < n_draws; ++d) {  // V + u (tag-2 normals 0..m-1), (V + u) P, then + Delta_T^1/2 eps (normals m..m+|T|-1)
+            double* out = draws + (long long)d * draw_stride;
+            LCX_TRY(normal_fill(s, seed, 2, row0, n_rows, d, m, c.u, c.ldv, nullptr, 0, c.v));
+            LCX_TRY(given_times_p(s, c.u, c.ldv, n_rows, p, ldp, m, nt, out, ldo));
+            const long long work = n_rows * (((long long)(m + nt - 1) >> 1) - (m >> 1) + 1);
+            lowrank::sample_finish_kernel<<<(unsigned)min((long long)cdiv(work, 256), (long long)kSMs * 16), 256, 0, s->stream>>>(
+                out, ldo, n_rows, m, nt, tcols + 3 * (long long)nt, tcols, tcols + nt, seed, row0, 2, d);
+            LAUNCHED(s);
+        }
+    return given_status(s, "lcx_conditional_sample_rows", c);
+}
+
+// rows [row0, row0 + rows) of theta1_T (Delta_T + P^T P) theta1_T: P^T P on the DMMA engine in lcx_precision_rows' layout, then the
+// diagonal and the scales
+extern "C" int lcx_conditional_covariance_rows(lcx_session* s, const double* p, long long ldp, int n_factors, int n_tgt,
+                                               const double* tcols, int row0, int rows, double* out, long long ldc) {
+    LCX_REQUIRE(s && p && tcols && out, "null argument");
+    LCX_REQUIRE(n_factors > 0 && n_tgt > 0 && ldp >= n_tgt && ldp % 2 == 0, "bad shape (ldp must be even and >= n_tgt)");
+    LCX_REQUIRE(row0 >= 0 && rows > 0 && row0 + rows <= n_tgt && row0 % 2 == 0 && rows < 65536, "bad row block (row0 must be even)");
+    LCX_REQUIRE(ldc >= n_tgt && ldc % 2 == 0, "ldc must be even and >= n_tgt");
+    LCX_REQUIRE(((uintptr_t)p % 16 == 0) && ((uintptr_t)out % 16 == 0), "misaligned device pointer");
+    LCX_CUDA(cudaSetDevice(s->device));
+    GemmArgs g;
+    memset(&g, 0, sizeof(g));
+    g.A = p + row0; g.B = p; g.C = out;
+    g.M = rows; g.N = n_tgt; g.K = n_factors;
+    g.lda = ldp; g.ldb = ldp; g.ldc = ldc;
+    LCX_TRY(launch_gemm(kLayoutMN, plan_gemm(rows, n_tgt, n_factors, kSMs, 1, false), g, s->stream));
+    LAUNCHED(s);
+    lowrank::given_cov_finish_kernel<<<dim3(cdiv(n_tgt, 256), rows), 256, 0, s->stream>>>(out, ldc, row0, rows, n_tgt, tcols);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
     return 0;
 }

@@ -25,6 +25,11 @@
 //   normal_fill_kernel    counter-based standard normals (Philox4x32-10 + Box-Muller), the U of sampling
 //   sample_prep_kernel    Z and sqrt(Delta) for sampling, Delta as factor_prep_kernel forms it
 //   sample_finish_kernel  theta0 + theta1 (U Z + sqrt(Delta) eps), eps generated in registers
+//   given_prep_kernel     conditioning on a fixed column set O: Z_O Delta_O^-1/2, Z_O Delta_O^-1, the gathered theta and
+//                         1/Delta of O, Z_T and Delta_T of the targets T, with factor_prep_kernel's Delta_i
+//   given_std_kernel      theta1_t sqrt(Delta_t + |p_t|^2), the conditional standard deviation of target t
+//   given_mean_finish_kernel   theta0_T + theta1_T (V P) of a row block (the conditional means)
+//   given_cov_finish_kernel    theta1_T (Delta_T + P^T P) theta1_T of a row block (the conditional covariance)
 #pragma once
 #include "common.cuh"
 #include "lu_solve.cuh"
@@ -75,7 +80,9 @@ __global__ void factor_prep_kernel(const double* __restrict__ rinv, const double
 // counter (j / 2, draw, row mod 2^32, row / 2^32 + 2^24 tag) under the key (seed mod 2^32, seed / 2^32): two uniforms in
 // (0, 1] of 53 bits each, u1 from words 0/1 and u2 from words 2/3, then Box-Muller, z_2t = sqrt(-2 ln u1) cospi(2 u2) and
 // z_2t+1 = sqrt(-2 ln u1) sinpi(2 u2).  It depends on nothing else, so results are the same under any grid, row blocking or
-// split of the rows between calls.  Tag 0: sample (columns 0..m-1 are u, m..m+n-1 eps); tag 1: conditional draws.
+// split of the rows between calls.  Tag 0: sample (columns 0..m-1 are u, m..m+n-1 eps); tag 1: conditional draws of the
+// missing entries (sample_missing); tag 2: draws given a fixed column set (ConditionalGaussian.sample: columns 0..m-1 are u,
+// m..m+|T|-1 eps in the order of the targets).
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
 #pragma unroll
     for (int r = 0; r < 10; ++r) {
@@ -107,17 +114,19 @@ __device__ __forceinline__ double normal_at(unsigned long long seed, int tag, lo
     return (j & 1) ? z.y : z.x;
 }
 
-// out (rows x ldo): out[r][j] = normal j of stream (seed, tag, row0 + r, draw) for j < cols; words (optional, rows x ldw) the
-// four Philox words behind normals 2t and 2t + 1 at words[r][4t .. 4t + 3].  One thread per counter.
+// out (rows x ldo): out[r][j] = normal j of stream (seed, tag, row0 + r, draw) for j < cols, plus base[r][j] when base (ld
+// ldo) is given; words (optional, rows x ldw) the four Philox words behind normals 2t and 2t + 1 at words[r][4t .. 4t + 3].
+// One thread per counter.
 __global__ void __launch_bounds__(256) normal_fill_kernel(unsigned long long seed, int tag, long long row0, long long rows,
-                                                          long long draw, int cols, double* __restrict__ out, long long ldo,
+                                                          long long draw, int cols, const double* __restrict__ base,
+                                                          double* __restrict__ out, long long ldo,
                                                           uint32_t* __restrict__ words, long long ldw) {
     const long long pairs = (cols + 1) / 2;
     for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < rows * pairs; e += (long long)gridDim.x * 256) {
         const long long r = e / pairs, t = e % pairs;
         const double2 z = normal_pair(seed, tag, row0 + r, draw, t);
-        out[r * ldo + 2 * t] = z.x;
-        if (2 * t + 1 < cols) out[r * ldo + 2 * t + 1] = z.y;
+        out[r * ldo + 2 * t] = base ? base[r * ldo + 2 * t] + z.x : z.x;
+        if (2 * t + 1 < cols) out[r * ldo + 2 * t + 1] = base ? base[r * ldo + 2 * t + 1] + z.y : z.y;
         if (words) {
             const uint4 w = philox_words(seed, tag, row0 + r, draw, t);
             uint32_t* o = words + r * ldw + 4 * t;
@@ -141,15 +150,16 @@ __global__ void sample_prep_kernel(const double* __restrict__ rinv, const double
 }
 
 // out (rows x ldo) holds Y = U Z on entry and theta0 + theta1 (Y + sqrt(Delta) eps) on exit, eps_i = normal m + i of stream
-// (seed, 0, row0 + r, 0), generated here and never stored.  One thread per Philox counter (two normals).
+// (seed, tag, row0 + r, draw), generated here and never stored.  One thread per Philox counter (two normals).  sample: tag 0,
+// draw 0; ConditionalGaussian.sample: tag 2, n = |T|, the gathered theta and sqrt(Delta) of the targets.
 __global__ void __launch_bounds__(256) sample_finish_kernel(double* __restrict__ out, long long ldo, long long rows, int m, int n,
                                                             const double* __restrict__ sqd, const double* __restrict__ mean,
                                                             const double* __restrict__ sd, unsigned long long seed,
-                                                            long long row0) {
+                                                            long long row0, int tag, long long draw) {
     const long long t0 = m >> 1, pairs = ((long long)(m + n - 1) >> 1) - t0 + 1;
     for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < rows * pairs; e += (long long)gridDim.x * 256) {
         const long long r = e / pairs, t = t0 + e % pairs;
-        const double2 z = normal_pair(seed, 0, row0 + r, 0, t);
+        const double2 z = normal_pair(seed, tag, row0 + r, draw, t);
         const long long i0 = 2 * t - m;
         if (i0 >= 0) {
             double* o = out + r * ldo + i0;
@@ -244,7 +254,9 @@ __global__ void __launch_bounds__(256) logdet_kernel(const double* __restrict__ 
 // out of ssq; miss[r * n + 0 .. nmiss[r]) lists the missing columns in ascending order and miss[r * n + n - 1 - j] the j-th
 // observed one; raw (optional, ld ldr) receives the observed entries as binary64.  An observed entry goes through exactly
 // the arithmetic of MASK = false, so a complete row gives the same out and ssq bit for bit.
-template <typename T, bool VEC, bool MASK>
+// FLAG (conditioning on a fixed column set, where no entry may be missing): a missing entry is zeroed and left out of ssq as
+// with MASK, no lists are written, and raw[0] (one double) is set to 1.0.
+template <typename T, bool VEC, bool MASK, bool FLAG = false>
 __global__ void __launch_bounds__(256) score_standardize_kernel(const T* __restrict__ x, long long N, int n, long long ldx,
                                                                 int has_marker, double marker, int marker_is_nan,
                                                                 const double* __restrict__ impute, const double* __restrict__ mean,
@@ -275,7 +287,8 @@ __global__ void __launch_bounds__(256) score_standardize_kernel(const T* __restr
             for (int j = 0; j < 4; ++j) {
                 const int i = i0 + j;
                 o[j] = 0.0;
-                if (MASK && i < n) mis[j] = (v[j] != v[j]) || (has_marker && !marker_is_nan && v[j] == marker);
+                if ((MASK || FLAG) && i < n) mis[j] = (v[j] != v[j]) || (has_marker && !marker_is_nan && v[j] == marker);
+                if (FLAG && mis[j]) raw[0] = 1.0;
                 if (i < n && !mis[j]) {
                     o[j] = standardize_value(v[j], i, has_marker, marker, marker_is_nan, 0, impute, mean, sd);
                     acc += o[j] * o[j] * dinv[i];
@@ -699,6 +712,90 @@ __global__ void __launch_bounds__(kCondThreads) condition_rows_kernel(
             if (counts) atomicAdd(counts + cond_class(p), 1ULL);
         }
         __syncthreads();
+    }
+}
+
+// ---- conditioning on a fixed column set (ConditionalGaussian) -----------------------------------------------------------
+// Observed columns O, targets T (disjoint), standardised space, Sigma~ = Z^T Z + Delta:
+//   E_O = I + Z_O Delta_O^-1 Z_O^T = L L^T,   A = L^-1 Z_O Delta_O^-1 (m x |O|),   P = L^-1 Z_T (m x |T|)
+//   v = A x~_O,  E[x~_T | x~_O] = P^T v,  Cov[x~_T | x~_O] = Delta_T + P^T P,  q_O = sum_O x~_i^2 / Delta_i - |v|^2,
+//   log det Sigma_OO = sum_O (2 log sd_i + log Delta_i) + 2 sum_k log L_kk,   draw x~_T = P^T (v + u) + Delta_T^1/2 eps.
+// E_O - I, its factor, the sweeps for A and P and log det are lcx_lowrank_factor's pieces run on the gathered columns.
+
+// One thread per selected column: t < no is observed column obs[t], t >= no target column tgt[t - no].  Observed: zh, zd (m x
+// ldo) = Z_O Delta_O^-1/2, Z_O Delta_O^-1 (factor_prep_kernel's arithmetic), ocols = [theta0_O | theta1_O | 1/Delta_O] (rows of
+// no), ldiag = 2 log sd + log Delta.  Targets: zt (m x ldt) = Z_T, tcols rows 0..3 of nt = [theta0_T | theta1_T | Delta_T |
+// sqrt(Delta_T)].  status[1] = 1 when a selected Delta_i <= 0; scalars[2] = 1 when an index lies outside [0, n).
+__global__ void given_prep_kernel(const double* __restrict__ rinv, const double* __restrict__ si, long long ldr, int m, int n,
+                                  double inv_sqrt_scale, const double* __restrict__ mean, const double* __restrict__ sd,
+                                  const int* __restrict__ obs, int no, const int* __restrict__ tgt, int nt, double* __restrict__ zh,
+                                  double* __restrict__ zd, long long ldo, double* __restrict__ ocols, double* __restrict__ ldiag,
+                                  double* __restrict__ zt, long long ldt, double* __restrict__ tcols, int* __restrict__ status,
+                                  double* __restrict__ scalars) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= no + nt) return;
+    const bool is_obs = t < no;
+    const int a = is_obs ? t : t - no;
+    const int i = is_obs ? obs[a] : tgt[a];
+    if (i < 0 || i >= n) {
+        scalars[2] = 1.0;
+        return;
+    }
+    const double c = 1.0 + si[i];
+    const double delta = lowrank_delta(rinv, ldr, m, i, c, inv_sqrt_scale);
+    if (!(delta > 0.0)) status[1] = 1;
+    if (is_obs) {
+        const double di = 1.0 / delta, rs = sqrt(di);
+        ocols[a] = mean[i];
+        ocols[no + a] = sd[i];
+        ocols[2 * no + a] = di;
+        ldiag[a] = 2.0 * log(sd[i]) + log(delta);
+        for (int j = 0; j < m; ++j) {
+            const double z = lowrank_z(rinv, ldr, j, i, c, inv_sqrt_scale);
+            zh[(long long)j * ldo + a] = z * rs;
+            zd[(long long)j * ldo + a] = z * di;
+        }
+    } else {
+        tcols[a] = mean[i];
+        tcols[nt + a] = sd[i];
+        tcols[2 * nt + a] = delta;
+        tcols[3 * nt + a] = sqrt(delta);
+        for (int j = 0; j < m; ++j) zt[(long long)j * ldt + a] = lowrank_z(rinv, ldr, j, i, c, inv_sqrt_scale);
+    }
+}
+
+// tcols row 4 = theta1_t sqrt(Delta_t + sum_k P_kt^2) (k ascending), one thread per target
+__global__ void given_std_kernel(const double* __restrict__ p, long long ldp, int m, int nt, double* __restrict__ tcols) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nt) return;
+    double acc = 0.0;
+    for (int k = 0; k < m; ++k) {
+        const double v = p[(long long)k * ldp + t];
+        acc += v * v;
+    }
+    tcols[4 * nt + t] = tcols[nt + t] * sqrt(tcols[2 * nt + t] + acc);
+}
+
+// out (rows x ldo) holds V P on entry and theta0_T + theta1_T (V P) on exit
+__global__ void __launch_bounds__(256) given_mean_finish_kernel(double* __restrict__ out, long long ldo, long long rows, int nt,
+                                                                const double* __restrict__ tcols) {
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < rows * nt; e += (long long)gridDim.x * 256) {
+        const long long r = e / nt;
+        const int t = (int)(e % nt);
+        double* o = out + r * ldo + t;
+        *o = tcols[t] + tcols[nt + t] * *o;
+    }
+}
+
+// out (rows x ldc) holds rows [row0, row0 + rows) of P^T P; turned into the same rows of theta1_T (Delta_T + P^T P) theta1_T
+__global__ void given_cov_finish_kernel(double* __restrict__ out, long long ldc, int row0, int rows, int nt,
+                                        const double* __restrict__ tcols) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    const int r = blockIdx.y;
+    if (k < nt && r < rows) {
+        const int i = row0 + r;
+        const double v = (i == k ? tcols[2 * nt + i] : 0.0) + out[(long long)r * ldc + k];
+        out[(long long)r * ldc + k] = v * (tcols[nt + i] * tcols[nt + k]);
     }
 }
 
