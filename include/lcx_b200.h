@@ -198,6 +198,33 @@ int lcx_standardize(lcx_session* s, const void* x, int dtype, long long n_rows, 
                     int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
                     const double* sd, double* out, long long ldo);
 long long lcx_colstats_scratch_doubles(long long n_rows, int n_vars);
+/* ---- per-row sample weights (Corex.fit(x, sample_weight=w)) ------------------------------------------------------
+ * Every data-dependent quantity of the fit is an average over rows of a product of two linear functions of one row, so
+ * scaling row l of X~ by r_l = sqrt(n_rows_total * w_l / w_total) (w_total = sum of w over all ranks) turns each into its
+ * weighted average with n_rows_total kept as the divisor; nothing after the pass that writes X~ changes.  All pointers are
+ * device pointers, every call is enqueued on the session stream.  With every w_l equal, every r_l is exactly 1 and each
+ * call below returns bit for bit what its unweighted sibling returns.  A row with w_l = 0 is left out of the statistics
+ * and its row of X~ is zero.
+ * lcx_row_scale: r[l] = sqrt(n_rows_total * w[l] / w_total), l < n_rows.
+ * lcx_colstats_sum_w: lcx_colstats_sum with sum[i] = sum_l w_l x_li and cnt[i] = sum_l w_l over observed entries.
+ * lcx_colstats_sqdev_w: lcx_colstats_sqdev with sq[i] = sum_l w_l (x_li - mean_i)^2; maxdev (optional) bounds
+ *   r_l |x_li - mean_i| over the rows with w_l > 0.  Then lcx_colstats_mean / lcx_colstats_std as before, with
+ *   w_total in place of n_rows_total and the weighted cnt.
+ * lcx_standardize_w / lcx_standardize_slice_w: row l of X~ (of the digit planes) is r_l times lcx_standardize's; for the
+ *   slice variant r[0] is the scale of row row0. */
+int lcx_row_scale(lcx_session* s, const double* w, long long n_rows, double n_rows_total, double w_total, double* r);
+int lcx_colstats_sum_w(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                       int has_marker, double marker, double* sum, double* cnt, double* scratch, long long scratch_doubles,
+                       const double* w);
+int lcx_colstats_sqdev_w(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                         int has_marker, double marker, const double* mean, double* sq, double* maxdev, double* scratch,
+                         long long scratch_doubles, const double* w, const double* r);
+int lcx_standardize_w(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                      int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                      const double* sd, double* out, long long ldo, const double* r);
+int lcx_standardize_slice_w(lcx_session* s, const void* x, int dtype, long long row0, long long n_rows, long long ldx,
+                            int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                            const double* sd, const double* r);
 
 /* ---- the two X contractions ----------------------------------------------------------------- */
 /* Y = X~ A^T  (:247, :210, :226, :394) and optionally colsq[j] = sum_l Y_lj^2 (:248, :227).

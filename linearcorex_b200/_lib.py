@@ -60,6 +60,11 @@ SIGNATURES = {
     "lcx_colstats_std": (_i, [_p, _p, _p, _d, _i, _p, _i]),
     "lcx_standardize": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _i, _p, _p, _p, _p, _ll]),
     "lcx_colstats_scratch_doubles": (_ll, [_ll, _i]),
+    "lcx_row_scale": (_i, [_p, _p, _ll, _d, _d, _p]),
+    "lcx_colstats_sum_w": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _ll, _p]),
+    "lcx_colstats_sqdev_w": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _p, _p, _p, _p, _ll, _p, _p]),
+    "lcx_standardize_w": (_i, [_p, _p, _i, _ll, _i, _ll, _i, _d, _i, _p, _p, _p, _p, _ll, _p]),
+    "lcx_standardize_slice_w": (_i, [_p, _p, _i, _ll, _ll, _ll, _i, _d, _i, _p, _p, _p, _p]),
     "lcx_project": (_i, [_p, _p, _ll, _i, _ll, _p, _ll, _i, _p, _ll, _p, _p, _ll]),
     "lcx_project_scratch_doubles": (_ll, [_ll, _i]),
     "lcx_sig": (_i, [_p, _p, _d, _p]),

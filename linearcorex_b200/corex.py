@@ -54,7 +54,7 @@ behaviour):
 Methods beyond the reference (sklearn's covariance-estimator interface; discourage_overlap=True models with theta):
   score_samples(x)    log N(x_l; theta[0], get_covariance()) per row, in the units of the input (g() of 'outliers' is not
                       applied: it is the density of the covariance estimate itself)
-  score(x)            their mean (over all ranks' rows with `comm`)
+  score(x)            their mean (over all ranks' rows with `comm`); with sample_weight, the weighted mean
   mahalanobis(x)      squared Mahalanobis distances under the same Gaussian
   get_precision()     the inverse of get_covariance(), in row blocks, with get_covariance's output options
   impute(x)           conditional means E[x_M | x_O] of the missing entries; return_std=True adds their conditional
@@ -68,6 +68,10 @@ B = G^-1 Z Delta^-1 (m x n) is built from the moments on each call and a row cos
 (conditioning: one SPD system of order |M| or m per row).  Random draws come from counter-based Philox4x32-10 normals, so
 they do not depend on how rows are blocked.
 Inputs are handled as by transform (containers, row providers, imputation of missing entries with the new data's means).
+
+Per-row sample weights: `fit(x, sample_weight=w)` (also fit_transform, hierarchy.fit_layers) estimates everything from the
+w-weighted averages over rows -- theta, the moments and the fit itself -- so for integer weights the fit is the fit of the
+data with row l repeated w_l times (only `n_samples` stays the row count).  DESIGN.md section 12.
 """
 import ctypes as C
 import os
@@ -513,8 +517,11 @@ class Corex(object):
             return self._upload(x)  # float32 values are exact in float64: keep the narrow upload
         return self._upload(np.asarray(x, dtype=want))
 
-    def preprocess(self, x, fit=False):
-        """Device preprocessing (:397-429).  Returns the fp64 X~ tensor (N x ld)."""
+    def preprocess(self, x, fit=False, _weights=None):
+        """Device preprocessing (:397-429).  Returns the fp64 X~ tensor (N x ld).
+
+        `_weights` (fit only): (w, w_total) from `_sample_weights` -- weighted column statistics, and row l of X~ scaled by
+        r_l = sqrt(N w_l / w_total) (DESIGN.md section 12)."""
         torch = _torch()
         sess = self._session()
         lib = sess.lib
@@ -534,26 +541,44 @@ class Corex(object):
         scratch = torch.empty(nscr, dtype=torch.float64, device=sess.device)
         impute = mean = sd = None
         n_total = red.sum_scalar(N)
+        wd = rs = None
+        if _weights is not None and fit:
+            w_total = _weights[1]
+            wd = torch.as_tensor(_weights[0], dtype=torch.float64).to(sess.device)
+            rs = self._row_scale(wd, w_total, n_total)
         if has_marker or (fit and mode != _lib.GAUSS['none']):
             ssum, cnt = vec(), vec()
-            _lib.check(lib.lcx_colstats_sum(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker,
-                                            ssum.data_ptr(), cnt.data_ptr(), scratch.data_ptr(), nscr), "lcx_colstats_sum")
+            if wd is None:
+                _lib.check(lib.lcx_colstats_sum(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker,
+                                                ssum.data_ptr(), cnt.data_ptr(), scratch.data_ptr(), nscr), "lcx_colstats_sum")
+            else:
+                _lib.check(lib.lcx_colstats_sum_w(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker,
+                                                  ssum.data_ptr(), cnt.data_ptr(), scratch.data_ptr(), nscr, wd.data_ptr()),
+                           "lcx_colstats_sum_w")
             red.sum_(ssum)
             red.sum_(cnt)
             impute = vec()
             _lib.check(lib.lcx_colstats_mean(sess.h, ssum.data_ptr(), cnt.data_ptr(), impute.data_ptr(), n))
-            self.n_obs = cnt.cpu().numpy().astype(np.int64) if has_marker else int(n_total)
+            if wd is None:
+                self.n_obs = cnt.cpu().numpy().astype(np.int64) if has_marker else int(n_total)
+            else:
+                self.n_obs = cnt.cpu().numpy() if has_marker else float(w_total)
         else:
-            self.n_obs = int(n_total)
+            self.n_obs = int(n_total) if wd is None else float(w_total)
         if mode != _lib.GAUSS['none']:
             if fit:
                 mean = impute
                 sq, sd = vec(), vec()
-                _lib.check(lib.lcx_colstats_sqdev(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker,
-                                                  mean.data_ptr(), sq.data_ptr(), None, scratch.data_ptr(), nscr),
-                           "lcx_colstats_sqdev")
+                if wd is None:
+                    _lib.check(lib.lcx_colstats_sqdev(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker,
+                                                      mean.data_ptr(), sq.data_ptr(), None, scratch.data_ptr(), nscr),
+                               "lcx_colstats_sqdev")
+                else:
+                    _lib.check(lib.lcx_colstats_sqdev_w(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker,
+                                                        mean.data_ptr(), sq.data_ptr(), None, scratch.data_ptr(), nscr,
+                                                        wd.data_ptr(), rs.data_ptr()), "lcx_colstats_sqdev_w")
                 red.sum_(sq)
-                _lib.check(lib.lcx_colstats_std(sess.h, sq.data_ptr(), cnt.data_ptr(), float(n_total),
+                _lib.check(lib.lcx_colstats_std(sess.h, sq.data_ptr(), cnt.data_ptr(), float(n_total if wd is None else w_total),
                                                 int(self.gaussianize == 'standard'), sd.data_ptr(), n))
                 self._theta_dev = (mean, sd)
                 self.theta = (mean.cpu().numpy().copy(), sd.cpu().numpy().copy())
@@ -563,15 +588,71 @@ class Corex(object):
                                             for t in self.theta)
                 mean, sd = self._theta_dev
         p = lambda t: t.data_ptr() if t is not None else None
-        _lib.check(lib.lcx_standardize(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker, mode,
-                                       p(impute), p(mean), p(sd), out.data_ptr(), ldo), "lcx_standardize")
+        if rs is None:
+            _lib.check(lib.lcx_standardize(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker, mode,
+                                           p(impute), p(mean), p(sd), out.data_ptr(), ldo), "lcx_standardize")
+        else:
+            _lib.check(lib.lcx_standardize_w(sess.h, xd.data_ptr(), dt, N, n, xd.stride(0), int(has_marker), marker, mode,
+                                             p(impute), p(mean), p(sd), out.data_ptr(), ldo, rs.data_ptr()), "lcx_standardize_w")
         return out
+
+    def _sample_weights(self, sample_weight, n_rows, red):
+        """Validate per-row weights before any device work: (w as a host float64 array, their sum over all ranks).
+        Raises ValueError (on every rank when one rank's weights are bad) unless w is 1-D with one finite, non-negative
+        value per local row and the total over all ranks is positive."""
+        torch = _torch()
+        err = None
+        try:
+            if isinstance(sample_weight, torch.Tensor):
+                w = sample_weight.detach().to(device="cpu", dtype=torch.float64).numpy()
+            else:
+                w = np.asarray(sample_weight, dtype=np.float64)
+        except (TypeError, ValueError) as e:
+            w, err = None, "sample_weight must be numeric: %s" % e
+        if err is None:
+            if w.ndim != 1:
+                err = "sample_weight must be 1-D, got shape %s" % (w.shape,)
+            elif w.shape[0] != n_rows:
+                err = "sample_weight has %d entries for %d rows" % (w.shape[0], n_rows)
+            elif not np.isfinite(w).all():
+                err = "sample_weight must be finite"
+            elif (w < 0).any():
+                err = "sample_weight must be non-negative"
+        bad = 1 if err else 0
+        if red.world > 1:
+            bad = red.max_scalar(bad)
+        if err or bad:
+            raise ValueError(err or "sample_weight is invalid on another rank")
+        w_total = float(red.sum_scalar(float(np.sum(w))))
+        if not (0.0 < w_total < np.inf):
+            raise ValueError("sample_weight must have a positive, finite sum over all rows (got %r)" % w_total)
+        return np.ascontiguousarray(w), w_total
+
+    def _row_scale(self, wd, w_total, n_total):
+        """The row scales r_l = sqrt(N_total w_l / W_total) of X~ (lcx_row_scale) from the device weights wd."""
+        sess = self._session()
+        rs = _torch().empty(wd.shape[0], dtype=_torch().float64, device=sess.device)
+        _lib.check(sess.lib.lcx_row_scale(sess.h, wd.data_ptr(), wd.shape[0], float(n_total), float(w_total), rs.data_ptr()),
+                   "lcx_row_scale")
+        return rs
 
     # ------------------------------------------------------------------------------------------
     # fit (:107-164)
     # ------------------------------------------------------------------------------------------
-    def fit(self, x):
-        schedule = self._prepare(x)
+    def fit(self, x, sample_weight=None):
+        """Fit the model to the rows of x (:107-164).
+
+        sample_weight: None, or one non-negative weight per row (ndarray, list, host or CUDA tensor; used as float64).  Every
+        statistic of the fit becomes its weighted average -- the column means (also the imputation means of missing entries)
+        and stds in theta, n_obs (the weighted observed count), the moments -- and for integer weights the fit equals the fit
+        of the data with row l repeated w_l times; n_samples stays the row count.  With `comm`, each rank passes the weights
+        of its own rows.  The weights are validated before any device work (ValueError) and not stored.  The split precisions
+        keep one exponent for all of X~, whose row l is scaled by sqrt(N w_l / sum w): very uneven weights raise it by
+        log2 of the largest such scale, and every other row loses those bits (DESIGN.md section 12)."""
+        weights = None
+        if sample_weight is not None:
+            weights = self._sample_weights(sample_weight, int(np.shape(x)[0]), self._reducer())
+        schedule = self._prepare(x, weights)
         for i_eps, eps in enumerate(schedule):
             self._begin_stage(eps, rescale=i_eps > 0)
             if self.discourage_overlap and not self.verbose:
@@ -638,8 +719,9 @@ class Corex(object):
             left -= k
         return True
 
-    def _prepare(self, x):
-        """Preprocess, bind the device problem and initialise W (:108-122).  Returns the anneal schedule."""
+    def _prepare(self, x, weights=None):
+        """Preprocess, bind the device problem and initialise W (:108-122).  Returns the anneal schedule.
+        `weights`: None or (w, w_total) from `_sample_weights`."""
         if self.m is None:
             raise ValueError("n_hidden=None (pick_n_hidden) is not supported: the reference helper is broken (:458-480)")
         red = self._reducer()
@@ -658,10 +740,10 @@ class Corex(object):
         self._fitted_in_session = False
         rows = self._stream_rows_for(x, red)
         if rows:
-            self._prepare_streamed(x, rows, red)
+            self._prepare_streamed(x, rows, red, weights)
         else:
             t0 = time.perf_counter()
-            xt = self.preprocess(x, fit=True)
+            xt = self.preprocess(x, fit=True, _weights=weights)
             _torch().cuda.synchronize()
             self.timings["preprocess_s"] = time.perf_counter() - t0
             n_local, self.nv = xt.shape[0], int(np.shape(x)[1])
@@ -796,10 +878,11 @@ class Corex(object):
             stream = int(red.max_scalar(stream))
         return 32768 if stream else max(n_rows, 1)
 
-    def _prepare_streamed(self, x, rows, red):
+    def _prepare_streamed(self, x, rows, red, weights=None):
         """preprocess(fit=True) + bind without ever holding all of X~ in fp64 (SURVEY.md hard part 4): three passes over
         row blocks of the raw input -- column sums/counts; squared deviations and max |x - mean|; standardise + digit
-        slicing.  `x` only needs `.shape` and row slicing (ndarray, memmap, tensor, or a generator-backed object)."""
+        slicing.  `x` only needs `.shape` and row slicing (ndarray, memmap, tensor, or a generator-backed object).
+        `weights` (w, w_total): the weighted passes, w and the row scales taken in the same row blocks as the rows."""
         torch = _torch()
         sess = self._session()
         lib = sess.lib
@@ -824,34 +907,57 @@ class Corex(object):
             xd = resident[lo:hi] if resident is not None else self._as_input(x[lo:hi])
             return xd, (_lib.F32 if xd.dtype == torch.float32 else _lib.F64)
 
+        wd = rs = None
+        if weights is not None:
+            w_total = weights[1]
+            wd = torch.as_tensor(weights[0], dtype=torch.float64).to(sess.device)
         ssum, cnt, t1, t2 = vec(), vec(), vec(), vec()
         for lo, hi in blocks:  # pass 1
             xd, dt = block(lo, hi)
-            _lib.check(lib.lcx_colstats_sum(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker,
-                                            t1.data_ptr(), t2.data_ptr(), scratch.data_ptr(), nscr), "lcx_colstats_sum")
+            if wd is None:
+                _lib.check(lib.lcx_colstats_sum(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker,
+                                                t1.data_ptr(), t2.data_ptr(), scratch.data_ptr(), nscr), "lcx_colstats_sum")
+            else:
+                _lib.check(lib.lcx_colstats_sum_w(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker,
+                                                  t1.data_ptr(), t2.data_ptr(), scratch.data_ptr(), nscr, wd[lo:hi].data_ptr()),
+                           "lcx_colstats_sum_w")
             ssum += t1
             cnt += t2
         red.sum_(ssum)
         red.sum_(cnt)
         n_total = red.sum_scalar(N)
+        if wd is not None:
+            rs = self._row_scale(wd, w_total, n_total)
         mean, sq, maxdev, sd = vec(), vec(), vec(), vec()
         _lib.check(lib.lcx_colstats_mean(sess.h, ssum.data_ptr(), cnt.data_ptr(), mean.data_ptr(), n))
         for lo, hi in blocks:  # pass 2
             xd, dt = block(lo, hi)
-            _lib.check(lib.lcx_colstats_sqdev(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker,
-                                              mean.data_ptr(), t1.data_ptr(), t2.data_ptr(), scratch.data_ptr(), nscr),
-                       "lcx_colstats_sqdev")
+            if wd is None:
+                _lib.check(lib.lcx_colstats_sqdev(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker,
+                                                  mean.data_ptr(), t1.data_ptr(), t2.data_ptr(), scratch.data_ptr(), nscr),
+                           "lcx_colstats_sqdev")
+            else:
+                _lib.check(lib.lcx_colstats_sqdev_w(sess.h, xd.data_ptr(), dt, hi - lo, n, xd.stride(0), int(has_marker), marker,
+                                                    mean.data_ptr(), t1.data_ptr(), t2.data_ptr(), scratch.data_ptr(), nscr,
+                                                    wd[lo:hi].data_ptr(), rs[lo:hi].data_ptr()), "lcx_colstats_sqdev_w")
             sq += t1
             maxdev = torch.maximum(maxdev, t2)
         red.sum_(sq)
-        _lib.check(lib.lcx_colstats_std(sess.h, sq.data_ptr(), cnt.data_ptr(), float(n_total),
+        _lib.check(lib.lcx_colstats_std(sess.h, sq.data_ptr(), cnt.data_ptr(), float(n_total if wd is None else w_total),
                                         int(self.gaussianize == 'standard'), sd.data_ptr(), n))
         self._theta_dev = (mean, sd)
         self.theta = (mean.cpu().numpy().copy(), sd.cpu().numpy().copy())
-        self.n_obs = cnt.cpu().numpy().astype(np.int64) if has_marker else int(n_total)
-        zmax = float((maxdev / sd).max().item())
+        if wd is None:
+            self.n_obs = cnt.cpu().numpy().astype(np.int64) if has_marker else int(n_total)
+        else:
+            self.n_obs = cnt.cpu().numpy() if has_marker else float(w_total)
+        zmax = float((maxdev / sd).max().item())  # weighted: maxdev bounds r_l |x - mean| (r_l the row scale)
         if self.gaussianize == 'outliers' and np.isfinite(zmax):
             zmax = min(zmax, 4.0) + float(np.tanh(max(zmax - 4.0, 0.0)))  # g() is monotone (:483-487)
+            if rs is not None:
+                # |r_l g(z_l)| <= max(1, max r) g(zmax): g is concave with g(0) = 0, so r g(z) <= g(r z) for r <= 1, and
+                # z <= r z <= zmax for r > 1.  All weights equal: max r = 1 and the bound is the unweighted one.
+                zmax *= max(1.0, float(rs.max().item()))
         self.n_samples = int(n_total)
         self.timings["preprocess_s"] = time.perf_counter() - t0
         t0 = time.perf_counter()
@@ -859,9 +965,14 @@ class Corex(object):
         _lib.check(lib.lcx_set_x_scale(sess.h, zmax), "lcx_set_x_scale")
         for lo, hi in blocks:  # pass 3: raw rows -> int8 digit planes, X~ never exists in binary64
             xd, dt = block(lo, hi)
-            _lib.check(lib.lcx_standardize_slice(sess.h, xd.data_ptr(), dt, lo, hi - lo, xd.stride(0), int(has_marker), marker, mode,
-                                                 mean.data_ptr(), mean.data_ptr(), sd.data_ptr()), "lcx_standardize_slice")
-        del resident
+            if rs is None:
+                _lib.check(lib.lcx_standardize_slice(sess.h, xd.data_ptr(), dt, lo, hi - lo, xd.stride(0), int(has_marker), marker,
+                                                     mode, mean.data_ptr(), mean.data_ptr(), sd.data_ptr()), "lcx_standardize_slice")
+            else:
+                _lib.check(lib.lcx_standardize_slice_w(sess.h, xd.data_ptr(), dt, lo, hi - lo, xd.stride(0), int(has_marker),
+                                                       marker, mode, mean.data_ptr(), mean.data_ptr(), sd.data_ptr(),
+                                                       rs[lo:hi].data_ptr()), "lcx_standardize_slice_w")
+        del resident, wd, rs
         torch.cuda.synchronize()
         self.timings["bind_s"] = time.perf_counter() - t0
 
@@ -925,8 +1036,9 @@ class Corex(object):
         self.timings["finish_s"] = time.perf_counter() - t0
         return self
 
-    def fit_transform(self, x):
-        self.fit(x)
+    def fit_transform(self, x, sample_weight=None):
+        """fit(x, sample_weight), then transform(x) (unweighted: the representation of every row)."""
+        self.fit(x, sample_weight=sample_weight)
         return self.transform(x)
 
     def _set_w(self, w):
@@ -1536,12 +1648,19 @@ class Corex(object):
         missing='marginalize' gives the distance of the observed part under Sigma_OO (see score_samples)."""
         return self._scores_for(x, missing)[0].cpu().numpy()
 
-    def score(self, x, missing='impute'):
+    def score(self, x, missing='impute', sample_weight=None):
         """Mean log-likelihood of the rows of x (the mean of score_samples(x, missing)).  With `comm` set, x is this rank's row
-        block and the mean is over all ranks' rows; every rank returns the same value."""
-        logp = self._scores_for(x, missing)[1].cpu().numpy()
+        block and the mean is over all ranks' rows; every rank returns the same value.  sample_weight (one non-negative weight
+        per row, as for fit): the weighted mean sum w log p / sum w over all ranks."""
         red = self._reducer()
-        return float(red.sum_scalar(float(np.sum(logp)))) / float(red.sum_scalar(len(logp)))
+        weights = None
+        if sample_weight is not None:
+            weights = self._sample_weights(sample_weight, int(np.shape(x)[0]), red)
+        logp = self._scores_for(x, missing)[1].cpu().numpy()
+        if weights is None:
+            return float(red.sum_scalar(float(np.sum(logp)))) / float(red.sum_scalar(len(logp)))
+        w, w_total = weights
+        return float(red.sum_scalar(float(np.sum(w * logp)))) / w_total
 
     def get_precision(self, block_rows=4096, out=None, block_callback=None):
         """n x n precision matrix Sigma^-1 = S^-1 (Delta^-1 - B^T B) S^-1 of the covariance estimate, in row blocks on the

@@ -356,20 +356,20 @@ extern "C" long long lcx_colstats_scratch_doubles(long long n_rows, int n_vars) 
 template <typename T>
 static bool vec4_ok(const T* x, long long ldx) { return ((uintptr_t)x % 16 == 0) && (ldx % 4 == 0); }
 
-template <typename T>
+template <typename T, bool W>
 static int colstats_sum_t(lcx_session* s, const T* x, long long N, int n, long long ldx, int has_marker, double marker,
-                          double* sum, double* cnt, double* scratch) {
+                          double* sum, double* cnt, double* scratch, const double* w) {
     const int slabs = cdiv(N, kSlabRows);
     const long long ldp = round_up(n, 16);
     double* ps = scratch;
     double* pc = scratch + (long long)slabs * ldp;
     const dim3 block(32, 8);
     if (vec4_ok(x, ldx))
-        colstats_sum_kernel<T, 4><<<dim3(cdiv(n, 128), slabs), block, 0, s->stream>>>(x, N, n, ldx, kSlabRows, has_marker, marker,
-                                                                                    marker != marker, ps, pc, ldp);
+        colstats_sum_kernel<T, 4, W><<<dim3(cdiv(n, 128), slabs), block, 0, s->stream>>>(x, N, n, ldx, kSlabRows, has_marker,
+                                                                                       marker, marker != marker, ps, pc, ldp, w);
     else
-        colstats_sum_kernel<T, 1><<<dim3(cdiv(n, 32), slabs), block, 0, s->stream>>>(x, N, n, ldx, kSlabRows, has_marker, marker,
-                                                                                   marker != marker, ps, pc, ldp);
+        colstats_sum_kernel<T, 1, W><<<dim3(cdiv(n, 32), slabs), block, 0, s->stream>>>(x, N, n, ldx, kSlabRows, has_marker,
+                                                                                      marker, marker != marker, ps, pc, ldp, w);
     LAUNCHED(s);
     combine_slabs_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(ps, slabs, ldp, sum, n);
     LAUNCHED(s);
@@ -386,9 +386,36 @@ extern "C" int lcx_colstats_sum(lcx_session* s, const void* x, int dtype, long l
     LCX_REQUIRE(n_rows > 0 && n_vars > 0 && ldx >= n_vars, "bad shape");
     LCX_REQUIRE(scratch_doubles >= lcx_colstats_scratch_doubles(n_rows, n_vars), "scratch too small");
     LCX_CUDA(cudaSetDevice(s->device));
-    if (dtype == LCX_F32) return colstats_sum_t<float>(s, (const float*)x, n_rows, n_vars, ldx, has_marker, marker, sum, cnt, scratch);
-    if (dtype == LCX_F64) return colstats_sum_t<double>(s, (const double*)x, n_rows, n_vars, ldx, has_marker, marker, sum, cnt, scratch);
+    if (dtype == LCX_F32)
+        return colstats_sum_t<float, false>(s, (const float*)x, n_rows, n_vars, ldx, has_marker, marker, sum, cnt, scratch, nullptr);
+    if (dtype == LCX_F64)
+        return colstats_sum_t<double, false>(s, (const double*)x, n_rows, n_vars, ldx, has_marker, marker, sum, cnt, scratch, nullptr);
     return fail(LCX_ERR_ARG, "lcx_colstats_sum", "unknown dtype");
+}
+
+extern "C" int lcx_row_scale(lcx_session* s, const double* w, long long n_rows, double n_rows_total, double w_total,
+                             double* r) {
+    LCX_REQUIRE(s && w && r, "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_rows_total > 0.0 && w_total > 0.0 && w_total <= DBL_MAX, "bad row count or weight total");
+    LCX_CUDA(cudaSetDevice(s->device));
+    row_scale_kernel<<<(unsigned)cdiv(n_rows, 256), 256, 0, s->stream>>>(w, n_rows, n_rows_total, w_total, r);
+    LAUNCHED(s);
+    LCX_CUDA(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int lcx_colstats_sum_w(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                                  int has_marker, double marker, double* sum, double* cnt, double* scratch,
+                                  long long scratch_doubles, const double* w) {
+    LCX_REQUIRE(s && x && sum && cnt && scratch && w, "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_vars > 0 && ldx >= n_vars, "bad shape");
+    LCX_REQUIRE(scratch_doubles >= lcx_colstats_scratch_doubles(n_rows, n_vars), "scratch too small");
+    LCX_CUDA(cudaSetDevice(s->device));
+    if (dtype == LCX_F32)
+        return colstats_sum_t<float, true>(s, (const float*)x, n_rows, n_vars, ldx, has_marker, marker, sum, cnt, scratch, w);
+    if (dtype == LCX_F64)
+        return colstats_sum_t<double, true>(s, (const double*)x, n_rows, n_vars, ldx, has_marker, marker, sum, cnt, scratch, w);
+    return fail(LCX_ERR_ARG, "lcx_colstats_sum_w", "unknown dtype");
 }
 
 extern "C" int lcx_colstats_mean(lcx_session* s, const double* sum, const double* cnt, double* mean, int n_vars) {
@@ -400,19 +427,19 @@ extern "C" int lcx_colstats_mean(lcx_session* s, const double* sum, const double
     return 0;
 }
 
-template <typename T>
+template <typename T, bool W>
 static int colstats_sqdev_t(lcx_session* s, const T* x, long long N, int n, long long ldx, int has_marker, double marker,
-                            const double* mean, double* sq, double* maxdev, double* scratch) {
+                            const double* mean, double* sq, double* maxdev, double* scratch, const double* w, const double* r) {
     const int slabs = cdiv(N, kSlabRows);
     const long long ldp = round_up(n, 16);
     double* pmax = maxdev ? scratch + (long long)slabs * ldp : nullptr;
     const dim3 block(32, 8);
     if (vec4_ok(x, ldx))
-        colstats_sqdev_kernel<T, 4><<<dim3(cdiv(n, 128), slabs), block, 0, s->stream>>>(x, N, n, ldx, kSlabRows, has_marker, marker,
-                                                                                      marker != marker, mean, scratch, pmax, ldp);
+        colstats_sqdev_kernel<T, 4, W><<<dim3(cdiv(n, 128), slabs), block, 0, s->stream>>>(
+            x, N, n, ldx, kSlabRows, has_marker, marker, marker != marker, mean, scratch, pmax, ldp, w, r);
     else
-        colstats_sqdev_kernel<T, 1><<<dim3(cdiv(n, 32), slabs), block, 0, s->stream>>>(x, N, n, ldx, kSlabRows, has_marker, marker,
-                                                                                     marker != marker, mean, scratch, pmax, ldp);
+        colstats_sqdev_kernel<T, 1, W><<<dim3(cdiv(n, 32), slabs), block, 0, s->stream>>>(
+            x, N, n, ldx, kSlabRows, has_marker, marker, marker != marker, mean, scratch, pmax, ldp, w, r);
     LAUNCHED(s);
     combine_slabs_kernel<<<cdiv(n, 256), 256, 0, s->stream>>>(scratch, slabs, ldp, sq, n);
     LAUNCHED(s);
@@ -431,9 +458,29 @@ extern "C" int lcx_colstats_sqdev(lcx_session* s, const void* x, int dtype, long
     LCX_REQUIRE(n_rows > 0 && n_vars > 0 && ldx >= n_vars, "bad shape");
     LCX_REQUIRE(scratch_doubles >= lcx_colstats_scratch_doubles(n_rows, n_vars), "scratch too small");
     LCX_CUDA(cudaSetDevice(s->device));
-    if (dtype == LCX_F32) return colstats_sqdev_t<float>(s, (const float*)x, n_rows, n_vars, ldx, has_marker, marker, mean, sq, maxdev, scratch);
-    if (dtype == LCX_F64) return colstats_sqdev_t<double>(s, (const double*)x, n_rows, n_vars, ldx, has_marker, marker, mean, sq, maxdev, scratch);
+    if (dtype == LCX_F32)
+        return colstats_sqdev_t<float, false>(s, (const float*)x, n_rows, n_vars, ldx, has_marker, marker, mean, sq, maxdev, scratch,
+                                              nullptr, nullptr);
+    if (dtype == LCX_F64)
+        return colstats_sqdev_t<double, false>(s, (const double*)x, n_rows, n_vars, ldx, has_marker, marker, mean, sq, maxdev,
+                                               scratch, nullptr, nullptr);
     return fail(LCX_ERR_ARG, "lcx_colstats_sqdev", "unknown dtype");
+}
+
+extern "C" int lcx_colstats_sqdev_w(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                                    int has_marker, double marker, const double* mean, double* sq, double* maxdev,
+                                    double* scratch, long long scratch_doubles, const double* w, const double* r) {
+    LCX_REQUIRE(s && x && mean && sq && scratch && w && r, "null argument");
+    LCX_REQUIRE(n_rows > 0 && n_vars > 0 && ldx >= n_vars, "bad shape");
+    LCX_REQUIRE(scratch_doubles >= lcx_colstats_scratch_doubles(n_rows, n_vars), "scratch too small");
+    LCX_CUDA(cudaSetDevice(s->device));
+    if (dtype == LCX_F32)
+        return colstats_sqdev_t<float, true>(s, (const float*)x, n_rows, n_vars, ldx, has_marker, marker, mean, sq, maxdev, scratch,
+                                             w, r);
+    if (dtype == LCX_F64)
+        return colstats_sqdev_t<double, true>(s, (const double*)x, n_rows, n_vars, ldx, has_marker, marker, mean, sq, maxdev,
+                                              scratch, w, r);
+    return fail(LCX_ERR_ARG, "lcx_colstats_sqdev_w", "unknown dtype");
 }
 
 extern "C" int lcx_colstats_std(lcx_session* s, const double* sq, const double* cnt, double n_rows_total, int use_nobs,
@@ -446,9 +493,10 @@ extern "C" int lcx_colstats_std(lcx_session* s, const double* sq, const double* 
     return 0;
 }
 
-extern "C" int lcx_standardize(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
-                               int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
-                               const double* sd, double* out, long long ldo) {
+template <bool W>
+static int standardize_d(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx, int has_marker,
+                         double marker, int gauss_mode, const double* impute, const double* mean, const double* sd, double* out,
+                         long long ldo, const double* r) {
     LCX_REQUIRE(s && x && out, "null argument");
     LCX_REQUIRE(gauss_mode == LCX_GAUSS_NONE || (mean && sd), "mean/std required");
     LCX_REQUIRE(has_marker == 0 || impute != nullptr, "imputation means required when a missing marker is set");
@@ -459,17 +507,17 @@ extern "C" int lcx_standardize(lcx_session* s, const void* x, int dtype, long lo
                     (dtype == LCX_F32 ? vec4_ok((const float*)x, ldx) : vec4_ok((const double*)x, ldx));
     const dim3 grid((unsigned)n_rows, cdiv(ldo, v4 ? 1024 : 256));
     if (dtype == LCX_F32 && v4)
-        standardize_kernel<float, 4><<<grid, 256, 0, s->stream>>>((const float*)x, n_rows, n_vars, ldx, has_marker, marker,
-                                                                nan_marker, gauss_mode, impute, mean, sd, out, ldo);
+        standardize_kernel<float, 4, W><<<grid, 256, 0, s->stream>>>((const float*)x, n_rows, n_vars, ldx, has_marker, marker,
+                                                                nan_marker, gauss_mode, impute, mean, sd, out, ldo, r);
     else if (dtype == LCX_F32)
-        standardize_kernel<float, 1><<<grid, 256, 0, s->stream>>>((const float*)x, n_rows, n_vars, ldx, has_marker, marker,
-                                                                nan_marker, gauss_mode, impute, mean, sd, out, ldo);
+        standardize_kernel<float, 1, W><<<grid, 256, 0, s->stream>>>((const float*)x, n_rows, n_vars, ldx, has_marker, marker,
+                                                                nan_marker, gauss_mode, impute, mean, sd, out, ldo, r);
     else if (dtype == LCX_F64 && v4)
-        standardize_kernel<double, 4><<<grid, 256, 0, s->stream>>>((const double*)x, n_rows, n_vars, ldx, has_marker, marker,
-                                                                 nan_marker, gauss_mode, impute, mean, sd, out, ldo);
+        standardize_kernel<double, 4, W><<<grid, 256, 0, s->stream>>>((const double*)x, n_rows, n_vars, ldx, has_marker, marker,
+                                                                 nan_marker, gauss_mode, impute, mean, sd, out, ldo, r);
     else if (dtype == LCX_F64)
-        standardize_kernel<double, 1><<<grid, 256, 0, s->stream>>>((const double*)x, n_rows, n_vars, ldx, has_marker, marker,
-                                                                 nan_marker, gauss_mode, impute, mean, sd, out, ldo);
+        standardize_kernel<double, 1, W><<<grid, 256, 0, s->stream>>>((const double*)x, n_rows, n_vars, ldx, has_marker, marker,
+                                                                 nan_marker, gauss_mode, impute, mean, sd, out, ldo, r);
     else
         return fail(LCX_ERR_ARG, "lcx_standardize", "unknown dtype");
     LAUNCHED(s);
@@ -477,53 +525,86 @@ extern "C" int lcx_standardize(lcx_session* s, const void* x, int dtype, long lo
     return 0;
 }
 
-template <typename T, int S>
+extern "C" int lcx_standardize(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                               int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                               const double* sd, double* out, long long ldo) {
+    return standardize_d<false>(s, x, dtype, n_rows, n_vars, ldx, has_marker, marker, gauss_mode, impute, mean, sd, out, ldo,
+                                nullptr);
+}
+
+extern "C" int lcx_standardize_w(lcx_session* s, const void* x, int dtype, long long n_rows, int n_vars, long long ldx,
+                                 int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                                 const double* sd, double* out, long long ldo, const double* r) {
+    LCX_REQUIRE(r != nullptr, "null argument");
+    return standardize_d<true>(s, x, dtype, n_rows, n_vars, ldx, has_marker, marker, gauss_mode, impute, mean, sd, out, ldo, r);
+}
+
+template <typename T, int S, bool W>
 static int standardize_slice_t(lcx_session* s, const T* x, long long row0, long long rows, long long ldx, int has_marker,
-                               double marker, int mode, const double* impute, const double* mean, const double* sd) {
+                               double marker, int mode, const double* impute, const double* mean, const double* sd,
+                               const double* r) {
     const Layout& L = s->L;
     const dim3 grid((unsigned)rows, cdiv(L.ld8, 4 * 128));
     int8_t* out = s->xs() + row0 * L.ld8;
     const int nan_marker = marker != marker;
     if (vec4_ok(x, ldx))
-        standardize_slice_kernel<T, S, 4><<<grid, 128, 0, s->stream>>>(x, rows, s->n, ldx, has_marker, marker, nan_marker, mode,
+        standardize_slice_kernel<T, S, 4, W><<<grid, 128, 0, s->stream>>>(x, rows, s->n, ldx, has_marker, marker, nan_marker, mode,
                                                                      impute, mean, sd, s->oz_xscale(), out, L.ld8,
-                                                                     s->Nl * L.ld8, (double)oz::kRadix);
+                                                                     s->Nl * L.ld8, (double)oz::kRadix, r);
     else
-        standardize_slice_kernel<T, S, 1><<<grid, 128, 0, s->stream>>>(x, rows, s->n, ldx, has_marker, marker, nan_marker, mode,
+        standardize_slice_kernel<T, S, 1, W><<<grid, 128, 0, s->stream>>>(x, rows, s->n, ldx, has_marker, marker, nan_marker, mode,
                                                                      impute, mean, sd, s->oz_xscale(), out, L.ld8,
-                                                                     s->Nl * L.ld8, (double)oz::kRadix);
+                                                                     s->Nl * L.ld8, (double)oz::kRadix, r);
     LAUNCHED(s);
     LCX_CUDA(cudaGetLastError());
     return 0;
 }
 
-template <typename T>
+template <typename T, bool W>
 static int standardize_slice_d(lcx_session* s, const T* x, long long row0, long long rows, long long ldx, int has_marker,
-                               double marker, int mode, const double* impute, const double* mean, const double* sd) {
+                               double marker, int mode, const double* impute, const double* mean, const double* sd,
+                               const double* r) {
     switch (s->L.S) {
-        case 3: return standardize_slice_t<T, 3>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd);
-        case 4: return standardize_slice_t<T, 4>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd);
-        case 5: return standardize_slice_t<T, 5>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd);
-        case 6: return standardize_slice_t<T, 6>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd);
-        case 7: return standardize_slice_t<T, 7>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd);
+        case 3: return standardize_slice_t<T, 3, W>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd, r);
+        case 4: return standardize_slice_t<T, 4, W>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd, r);
+        case 5: return standardize_slice_t<T, 5, W>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd, r);
+        case 6: return standardize_slice_t<T, 6, W>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd, r);
+        case 7: return standardize_slice_t<T, 7, W>(s, x, row0, rows, ldx, has_marker, marker, mode, impute, mean, sd, r);
     }
     return fail(LCX_ERR_STATE, "lcx_standardize_slice", "bad digit count");
 }
 
 // lcx_standardize + lcx_slice_block in one pass over the raw rows (split modes, after lcx_bind(xt = NULL) + lcx_set_x_scale)
-extern "C" int lcx_standardize_slice(lcx_session* s, const void* x, int dtype, long long row0, long long n_rows, long long ldx,
-                                     int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
-                                     const double* sd) {
+template <bool W>
+static int standardize_slice_any(lcx_session* s, const void* x, int dtype, long long row0, long long n_rows, long long ldx,
+                                 int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                                 const double* sd, const double* r) {
     S_REQUIRE_BOUND(s);
     LCX_REQUIRE(s->L.S > 0 && !s->gram, "only meaningful in the split modes, on a session bound to X~");
     LCX_REQUIRE(x != nullptr && row0 >= 0 && n_rows > 0 && row0 + n_rows <= s->Nl && ldx >= s->n, "bad row block");
     LCX_REQUIRE(gauss_mode == LCX_GAUSS_NONE || (mean && sd), "mean/std required");
     LCX_REQUIRE(has_marker == 0 || impute != nullptr, "imputation means required when a missing marker is set");
     if (dtype == LCX_F32)
-        return standardize_slice_d<float>(s, (const float*)x, row0, n_rows, ldx, has_marker, marker, gauss_mode, impute, mean, sd);
+        return standardize_slice_d<float, W>(s, (const float*)x, row0, n_rows, ldx, has_marker, marker, gauss_mode, impute, mean,
+                                             sd, r);
     if (dtype == LCX_F64)
-        return standardize_slice_d<double>(s, (const double*)x, row0, n_rows, ldx, has_marker, marker, gauss_mode, impute, mean, sd);
+        return standardize_slice_d<double, W>(s, (const double*)x, row0, n_rows, ldx, has_marker, marker, gauss_mode, impute, mean,
+                                              sd, r);
     return fail(LCX_ERR_ARG, "lcx_standardize_slice", "unknown dtype");
+}
+
+extern "C" int lcx_standardize_slice(lcx_session* s, const void* x, int dtype, long long row0, long long n_rows, long long ldx,
+                                     int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                                     const double* sd) {
+    return standardize_slice_any<false>(s, x, dtype, row0, n_rows, ldx, has_marker, marker, gauss_mode, impute, mean, sd, nullptr);
+}
+
+// r: the row scales of rows [row0, row0 + n_rows) (r[0] belongs to row row0)
+extern "C" int lcx_standardize_slice_w(lcx_session* s, const void* x, int dtype, long long row0, long long n_rows, long long ldx,
+                                       int has_marker, double marker, int gauss_mode, const double* impute, const double* mean,
+                                       const double* sd, const double* r) {
+    LCX_REQUIRE(r != nullptr, "null argument");
+    return standardize_slice_any<true>(s, x, dtype, row0, n_rows, ldx, has_marker, marker, gauss_mode, impute, mean, sd, r);
 }
 
 // ---- exported steps ----------------------------------------------------------------------------

@@ -33,11 +33,14 @@ __device__ __forceinline__ bool is_missing_d(double d, int has_marker, double ma
 // pass 1: part_sum[slab][i] = sum of observed x, part_cnt[slab][i] = number observed (finite, not missing)
 // Each thread owns V adjacent columns (V = 4: 16-byte loads) and every eighth row of the slab; a column's rows are
 // summed in the same order whatever V is, so the result does not depend on the vector width.
-template <typename T, int V>
+// WEIGHTED: sum of w_l x and of w_l over the observed entries, rows with w_l = 0 skipped, in the same order -- with every
+// w_l = 1 both sums are the unweighted ones bit for bit.
+template <typename T, int V, bool WEIGHTED = false>
 __global__ void __launch_bounds__(256) colstats_sum_kernel(const T* __restrict__ x, long long N, int n, long long ldx,
                                                            int rows_per_slab, int has_marker, double marker,
                                                            int marker_is_nan, double* __restrict__ part_sum,
-                                                           double* __restrict__ part_cnt, long long ldp) {
+                                                           double* __restrict__ part_cnt, long long ldp,
+                                                           const double* __restrict__ w = nullptr) {
     __shared__ double rs[8][32 * V], rc[8][32 * V];
     const int i0 = (blockIdx.x * 32 + threadIdx.x) * V;
     const long long r0 = (long long)blockIdx.y * rows_per_slab;
@@ -48,12 +51,21 @@ __global__ void __launch_bounds__(256) colstats_sum_kernel(const T* __restrict__
     if (i0 < n) {
 #pragma unroll 2
         for (long long r = r0 + threadIdx.y; r < r1; r += 8) {
+            double wl = 1.0;
+            if constexpr (WEIGHTED) {
+                wl = w[r];
+                if (wl == 0.0) continue;
+            }
             double v[V];
             load_row_vec<T, V>(x + r * ldx + i0, v);
 #pragma unroll
             for (int j = 0; j < V; ++j) {
                 const bool obs = has_marker ? (!is_missing_d(v[j], has_marker, marker, marker_is_nan) && isfinite(v[j])) : true;
-                if (obs) { s[j] += v[j]; c[j] += 1.0; }
+                if constexpr (WEIGHTED) {
+                    if (obs) { s[j] += wl * v[j]; c[j] += wl; }
+                } else {
+                    if (obs) { s[j] += v[j]; c[j] += 1.0; }
+                }
             }
         }
     }
@@ -76,12 +88,15 @@ __global__ void __launch_bounds__(256) colstats_sum_kernel(const T* __restrict__
 }
 
 // pass 2: part[slab][i] = sum over observed rows of (x - mean_i)^2   (imputed entries contribute 0)
-template <typename T, int V>
+// WEIGHTED: sum of w_l (x - mean_i)^2, and part_max bounds r_l |x - mean_i| (the row scale of X~, lcx_row_scale) over the
+// rows with w_l > 0, so a zero-weight outlier stays out of X~'s exponent.  Same order as the unweighted pass.
+template <typename T, int V, bool WEIGHTED = false>
 __global__ void __launch_bounds__(256) colstats_sqdev_kernel(const T* __restrict__ x, long long N, int n, long long ldx,
                                                              int rows_per_slab, int has_marker, double marker,
                                                              int marker_is_nan, const double* __restrict__ mean,
                                                              double* __restrict__ part, double* __restrict__ part_max,
-                                                             long long ldp) {
+                                                             long long ldp, const double* __restrict__ w = nullptr,
+                                                             const double* __restrict__ rsc = nullptr) {
     // part_max (optional): per-slab max |x - mean| -- bounds |X~| before X~ exists (streamed digit slicing)
     __shared__ double rs[8][32 * V], rm[8][32 * V];
     const int i0 = (blockIdx.x * 32 + threadIdx.x) * V;
@@ -96,14 +111,26 @@ __global__ void __launch_bounds__(256) colstats_sqdev_kernel(const T* __restrict
     if (i0 < n) {
 #pragma unroll 2
         for (long long r = r0 + threadIdx.y; r < r1; r += 8) {
+            double wl = 1.0, rl = 1.0;
+            if constexpr (WEIGHTED) {
+                wl = w[r];
+                if (wl == 0.0) continue;
+                rl = rsc[r];
+            }
             double v[V];
             load_row_vec<T, V>(x + r * ldx + i0, v);
 #pragma unroll
             for (int j = 0; j < V; ++j) {
                 if (!is_missing_d(v[j], has_marker, marker, marker_is_nan)) {
                     const double d = v[j] - mu[j];
-                    s[j] += d * d;
-                    mx[j] = amax_acc(mx[j], d);
+                    if constexpr (WEIGHTED) {
+                        const double wd = wl * d;
+                        s[j] += wd * d;
+                        mx[j] = amax_acc(mx[j], rl * d);
+                    } else {
+                        s[j] += d * d;
+                        mx[j] = amax_acc(mx[j], d);
+                    }
                 }
             }
         }
@@ -165,6 +192,18 @@ __global__ void finish_std_kernel(const double* __restrict__ sq, const double* _
     if (i < n) sd[i] = fmax(sqrt(sq[i] / (use_nobs ? cnt[i] : n_total)), 1e-10);
 }
 
+// r_l = sqrt(N_total w_l / W_total): scaling row l of X~ by r_l turns every average over rows of a product of two linear
+// functions of a row (X~^T Y / N, sum_l Y_lj^2 / N, X~^T X~ / N) into its w-weighted average, with N_total kept as the divisor.
+// All weights equal: every r_l is exactly 1.
+__global__ void row_scale_kernel(const double* __restrict__ w, long long N, double n_total, double w_total,
+                                 double* __restrict__ r) {
+    const long long l = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (l < N) r[l] = sqrt((n_total * w[l]) / w_total);
+}
+
+// o scaled by the row's r_l; a zero-weight row is exactly zero whatever it holds (an inf there poisons nothing).
+__device__ __forceinline__ double row_scaled(double rl, double o) { return rl == 0.0 ? 0.0 : rl * o; }
+
 __device__ __forceinline__ double squash_tails(double z) {  // g(), :483-487
     const double core = fmin(fmax(z, -4.0), 4.0);
     return core + tanh(z - core);
@@ -183,11 +222,12 @@ __device__ __forceinline__ double standardize_value(double d, int i, int has_mar
 
 // X~ = (x - mean)/std  [+ g()];  missing entries take the column mean first (:404, :415, :423).
 // mode: 0 = 'standard', 1 = 'outliers', 2 = 'none' (cast only).  Output fp64, ld = ldo, columns >= n zeroed.
-template <typename T, int V>
+// WEIGHTED: row r is scaled by rsc[r] (row_scale_kernel).
+template <typename T, int V, bool WEIGHTED = false>
 __global__ void standardize_kernel(const T* __restrict__ x, long long N, int n, long long ldx, int has_marker,
                                    double marker, int marker_is_nan, int mode, const double* __restrict__ impute,
                                    const double* __restrict__ mean, const double* __restrict__ sd,
-                                   double* __restrict__ out, long long ldo) {
+                                   double* __restrict__ out, long long ldo, const double* __restrict__ rsc = nullptr) {
     const int i0 = (blockIdx.y * blockDim.x + threadIdx.x) * V;  // rows on grid.x (up to 2^31-1), column blocks on grid.y
     const long long r = blockIdx.x;
     if (i0 >= ldo || r >= N) return;
@@ -199,6 +239,7 @@ __global__ void standardize_kernel(const T* __restrict__ x, long long N, int n, 
     for (int j = 0; j < V; ++j) {
         const int i = i0 + j;
         o[j] = i < n ? standardize_value(v[j], i, has_marker, marker, marker_is_nan, mode, impute, mean, sd) : 0.0;
+        if constexpr (WEIGHTED) o[j] = row_scaled(rsc[r], o[j]);
     }
     if constexpr (V == 1) {
         out[r * ldo + i0] = o[0];
@@ -213,13 +254,15 @@ __global__ void standardize_kernel(const T* __restrict__ x, long long N, int n, 
 // element instead of 12 + 8 + S + 8 through standardize_kernel, absmax and slice_rows.  The exponent of X~ must be known
 // beforehand (lcx_set_x_scale: max |x - mean| / std per column comes out of the squared-deviation pass).  The arithmetic of
 // each element is standardize_kernel's followed by split_digits's, operation for operation: the planes are bit-identical.
-template <typename T, int S, int V>
+// WEIGHTED: row r is scaled by rsc[r] before slicing, as in standardize_kernel.
+template <typename T, int S, int V, bool WEIGHTED = false>
 __global__ void __launch_bounds__(128) standardize_slice_kernel(const T* __restrict__ x, long long N, int n, long long ldx,
                                                                 int has_marker, double marker, int marker_is_nan, int mode,
                                                                 const double* __restrict__ impute, const double* __restrict__ mean,
                                                                 const double* __restrict__ sd, double* x_scale,
                                                                 int8_t* __restrict__ out, long long ld_out,
-                                                                long long slice_stride, double radix) {
+                                                                long long slice_stride, double radix,
+                                                                const double* __restrict__ rsc = nullptr) {
     const int c4 = (blockIdx.y * blockDim.x + threadIdx.x) * 4;   // four columns per thread: one char4 store per plane
     const long long r = blockIdx.x;
     if (c4 >= ld_out || r >= N) return;
@@ -244,6 +287,7 @@ __global__ void __launch_bounds__(128) standardize_slice_kernel(const T* __restr
         double o = 0.0;
         if (i < n) {
             o = standardize_value(v[j], i, has_marker, marker, marker_is_nan, mode, impute, mean, sd);
+            if constexpr (WEIGHTED) o = row_scaled(rsc[r], o);
             poison = poison || !(fabs(o) <= 1.7976931348623157e308);
         }
         oz::split_digits<S>(o, inv, radix, d[j]);

@@ -9,11 +9,12 @@ from .corex import Corex
 
 
 def fit_layers(x, layers, missing_values=None, gaussianize='standard', discourage_overlap=True, max_iter=10000,
-               tol=1e-5, seed=None, verbose=False, **corex_kwargs):
+               tol=1e-5, seed=None, verbose=False, sample_weight=None, **corex_kwargs):
     """Fit a stack of Corex layers.  Returns the list of fitted models (layer 0 first).
 
     `seed` is passed to every layer (the reference CLI never seeds, vis_corex.py:535-545); `corex_kwargs`
-    forwards the B200 extensions (`precision`, `exact_trials`, `comm`, `device`, ...)."""
+    forwards the B200 extensions (`precision`, `exact_trials`, `comm`, `device`, ...).  `sample_weight` (one
+    per row of x) is passed to every layer's fit: the rows of layer k's input are the rows of x."""
     layers = [int(v) for v in layers]
     if layers[-1] != 1:
         layers.append(1)  # last layer has one unit so the graph is fully connected
@@ -25,7 +26,7 @@ def fit_layers(x, layers, missing_values=None, gaussianize='standard', discourag
             kw["missing_values"] = missing_values
         else:
             x_prev = models[-1].transform(x_prev, return_device=True)
-        models.append(Corex(**kw).fit(x_prev))
+        models.append(Corex(**kw).fit(x_prev, sample_weight=sample_weight))
     return models
 
 
