@@ -204,16 +204,20 @@ struct GemmParams {
 // KMAJOR = true : A tile = [128 rows][64 B of K]   (SW64),  tensor map (K, rows, slice),      coordinates (k0, m0, s);
 // KMAJOR = false: A tile = [64 K rows][128 B of M] (SW128), tensor map (M, K rows, slice),    coordinates (m0, k0, s).
 // All MMAs of one 64-deep K block for a tile of compile-time width BN (multiple of 16, <= bn_max(S)).
-// BN % 16 == 8 (equal-width tiles such as 56): N = BN c is a legal UMMA N only for even c, so an odd plane count issues its
-// last plane as one instruction of N = BN + 8.  That plane always lands in the LAST group (g = S - 1): the 8 extra columns
-// fall into unused TMEM above the accumulators, and the 8 extra B rows it reads are whatever follows that plane in the stage.
+// BN % 16 == 8 (equal-width tiles such as 56): N = BN c is a legal UMMA N only for even c.  An odd count is legal as N = BN c + 8
+// in the instruction that closes a row of A: its last plane lands in the LAST group (g = S - 1), so the 8 extra columns fall
+// into unused TMEM above the accumulators, and the 8 extra B rows it reads are whatever follows that plane in the stage.  A row
+// therefore opens with the smallest even count that lets one instruction close it: bn = 56 issues 5 planes as 2 + 3 (N = 112,
+// 176) and 3 planes as one N = 176, not 4 + 1 and 2 + 1 -- an N = 64 instruction occupies the tensor pipe for ~55 cycles while
+// doing 28 cycles of work (profiles/r02_mma_mix_probe.txt), and S = 6 now needs 8 instructions per K step instead of 9.
 template <int S, bool KMAJOR, int BN>
 __device__ __forceinline__ void issue_kblock(uint32_t sa, uint32_t sb, uint32_t tmem_base, bool first_block) {
     constexpr int A_BYTES = kBM * kBK;
     constexpr int B_BYTES = BN * kBK;        // digit planes of B are packed at the tile's own width
     constexpr bool ODD8 = (BN % 16) != 0;
     constexpr int CMAX = ODD8 ? ((256 / BN) & ~1) : (256 / BN);  // digit planes of B per instruction (N <= 256)
-    static_assert(BN % 8 == 0 && BN >= 16 && CMAX >= 1, "tile width");
+    constexpr int CLAST = ODD8 ? (248 / BN) : CMAX;                // ... per row-closing instruction (N = BN c + 8 <= 256)
+    static_assert(BN % 8 == 0 && BN >= 16 && CMAX >= 1 && CLAST >= 1, "tile width");
 #pragma unroll
     for (int kk = 0; kk < kBK / 32; ++kk) {
 #pragma unroll
@@ -224,12 +228,11 @@ __device__ __forceinline__ void issue_kblock(uint32_t sa, uint32_t sb, uint32_t 
             for (int it = 0; it < kMaxInstr; ++it) {
                 const int left = S - ka - q0;
                 if (left <= 0) break;
-                int cnt = left < CMAX ? left : CMAX;
-                int n = BN * cnt;
-                if (ODD8) {
-                    if (cnt >= 2) { cnt &= ~1; n = BN * cnt; }
-                    else n = BN + 8;         // the row's last plane: spills 8 columns above group S - 1
-                }
+                int cnt;
+                if (left <= CLAST) cnt = left;                       // closes the row
+                else if (ODD8) cnt = min(CMAX, max(2, (left - CLAST + 1) & ~1));
+                else cnt = CMAX;
+                const int n = BN * cnt + ((ODD8 && (cnt & 1)) ? 8 : 0);  // (odd: spills 8 columns above group S - 1)
                 const uint32_t idesc = make_idesc_i8(kBM, n, KMAJOR ? 0 : 1, 0);
                 // K-major: rows at 64 B pitch, 8-row swizzle atoms of 512 B (SBO); a K step is +32 B inside the span; the
                 // next B plane starts BN/8 atoms further, i.e. N simply continues.
